@@ -400,27 +400,6 @@ SKM_API int skm_coo_merge_runs_packed(const uint64_t *d_packed_in, const int64_t
                               int count_bits, uint64_t *d_keys_out, int64_t *d_vals_out, int64_t *d_n_out,
                               void *workspace, size_t workspace_bytes, skm_stream_t stream);
 
-/* (a12) learn for the light annotations, on chip: one CTA sorts one TASK in shared memory (skm_annsort.cu; learn.smk:306-326,
- * 385-408).  The batch holds the sequences of the task annotations gathered in annotation order.  A task = the sequences
- * [seq_lo, seq_hi) of one annotation restricted to the codes [code_lo, code_hi), with at most skm_ann_sort_cap() windows;
- * tasks are listed in (annotation, code_lo) order and together produce ONE sorted COO list: task t writes its entries
- * (ann * S + code, count) from d_out_base[t] + (entries of the tasks in front, d_task_prefix[t]) on — out_base lets the
- * caller leave room for entries other paths produce (the dense rows of heavy annotations).  *d_total_out = entries of all
- * tasks; d_totals (NULL or int64 [S]) += the counts per code; *d_overflow != 0: a task had more windows than the capacity
- * (its output is then missing; the caller must recompute with smaller tasks).
- * skm_ann_hist: d_hist[r][code / bin_width] (uint32 [n_rows, n_bins]) = windows of the sequences [seq_lo[r], seq_hi[r]) per
- * code bin — what the caller cuts an annotation with more than the capacity into tasks with. */
-SKM_API int skm_ann_sort_cap(void);
-SKM_API int skm_ann_hist(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq, const uint8_t *d_lut, int nsym, int k,
-                 const int32_t *d_seq_lo, const int32_t *d_seq_hi, int64_t n_rows, uint32_t bin_width, int n_bins, uint32_t *d_hist,
-                 skm_stream_t stream);
-SKM_API size_t skm_ann_sort_workspace(int64_t n_tasks);
-SKM_API int skm_ann_sort(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq, const uint8_t *d_lut, int nsym, int k,
-                 const int32_t *d_seq_lo, const int32_t *d_seq_hi, const uint32_t *d_code_lo, const uint32_t *d_code_hi, const int64_t *d_ann,
-                 const int64_t *d_out_base, int64_t n_tasks, uint64_t *d_keys_out, int64_t *d_vals_out, int64_t capacity,
-                 int64_t *d_task_prefix, int64_t *d_totals, int64_t *d_total_out, int *d_overflow, void *workspace, size_t workspace_bytes,
-                 skm_stream_t stream);
-
 /* Multi-GPU fan-in over NVLink peer memory (one process per GPU; Merge.merge_dataframes across ranks, learn.smk:467-494).
  * The ONE exception to "the library never allocates": CUDA IPC exports whole allocations, so receive buffers are
  * cudaMalloc'ed here.  skm_peer_alloc returns the buffer and its 64-byte IPC handle (send it to the peers through the
@@ -447,10 +426,7 @@ SKM_API int skm_coo_pack_push(const uint64_t *d_keys, const int64_t *d_vals, con
  * skm_rows_emit: the non-zeros of block (r, b), in code order, as (ann_of_row[r] * S + code, count) from
  *   d_keys_out[d_row_dst[r] + d_block_offsets[r * nblk + b]] on — the caller's exclusive prefix sums of the block
  *   counts inside a row and the place of the row's annotation in the merged sorted list.
- * skm_rows_colsum: d_totals[c] += sum over rows (the Totals row of learn.smk:380; not atomic: one launch at a time).
- * skm_coo_shift_copy: out[i + shift(i)] = in[i] for a sorted COO list, shift(i) = d_insert_cum[h] for the largest h
- *   with d_insert_pos[h] <= i (0 below d_insert_pos[0]): makes room for blocks inserted at list positions
- *   d_insert_pos (ascending), d_insert_cum = inclusive prefix sums of the blocks' sizes. */
+ * skm_rows_colsum: d_totals[c] += sum over rows (the Totals row of learn.smk:380; not atomic: one launch at a time). */
 SKM_API int skm_rows_accumulate(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq,
                         const uint8_t *d_lut, int nsym, int k, const int32_t *d_row_of_seq, int64_t S,
                         uint32_t *d_rows, skm_stream_t stream);
@@ -460,9 +436,6 @@ SKM_API int skm_rows_emit(const uint32_t *d_rows, int64_t n_rows, int64_t S, con
                   const int64_t *d_row_dst, const int64_t *d_ann_of_row, uint64_t *d_keys_out, int64_t *d_vals_out,
                   int64_t out_capacity, skm_stream_t stream);
 SKM_API int skm_rows_colsum(const uint32_t *d_rows, int64_t n_rows, int64_t S, int64_t *d_totals, skm_stream_t stream);
-SKM_API int skm_coo_shift_copy(const uint64_t *d_keys, const int64_t *d_vals, int64_t n, const int64_t *d_insert_pos,
-                       const int64_t *d_insert_cum, int64_t n_insert, uint64_t *d_keys_out, int64_t *d_vals_out,
-                       skm_stream_t stream);
 
 /* Measurement helper (not on the product path): a kernel of `blocks` x 256 threads, each running 16 independent
  * chains of `iters` fp32 FMAs; *flops_out (host) = the flops it executes.  Timed with CUDA events by

@@ -96,10 +96,6 @@ SIGNATURES = {
     "skm_coo_pack": (_int, [_p, _p, _i64, _int, _p, _p, _p]),
     "skm_coo_merge_runs_packed_workspace": (_sz, [_i64, _int]),
     "skm_coo_merge_runs_packed": (_int, [_p, _p, _int, _int, _p, _p, _p, _p, _sz, _p]),
-    "skm_ann_sort_cap": (_int, []),
-    "skm_ann_hist": (_int, [_p, _i64, _p, _i64, _p, _int, _int, _p, _p, _i64, C.c_uint32, _int, _p, _p]),
-    "skm_ann_sort_workspace": (_sz, [_i64]),
-    "skm_ann_sort": (_int, [_p, _i64, _p, _i64, _p, _int, _int, _p, _p, _p, _p, _p, _p, _i64, _p, _p, _i64, _p, _p, _p, _p, _p, _sz, _p]),
     "skm_peer_alloc": (_int, [_sz, C.POINTER(C.c_void_p), _p]),
     "skm_peer_open": (_int, [_p, C.POINTER(C.c_void_p)]),
     "skm_peer_close": (_int, [_p]),
@@ -110,7 +106,6 @@ SIGNATURES = {
     "skm_rows_block_counts": (_int, [_p, _i64, _i64, _p, _p]),
     "skm_rows_emit": (_int, [_p, _i64, _i64, _p, _p, _p, _p, _p, _i64, _p]),
     "skm_rows_colsum": (_int, [_p, _i64, _i64, _p, _p]),
-    "skm_coo_shift_copy": (_int, [_p, _p, _i64, _p, _p, _i64, _p, _p, _p]),
     "skm_scatter_add_i64": (_int, [_p, _i64, _i64, _p, _p, _p, _i64, _i64, _p]),
 }
 

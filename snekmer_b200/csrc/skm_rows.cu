@@ -11,7 +11,6 @@
 //   skm_rows_block_counts  non-zeros per (row, 4096-code block): the caller's prefix sums give every block its place
 //   skm_rows_emit          (annotation * S + code, count) of every non-zero, in order, at the block's place
 //   skm_rows_colsum        totals[c] += sum over rows of rows[r][c]
-//   skm_coo_shift_copy     the sorted COO list of the light annotations moved to its places between the heavy ones
 // Integer adds only: results are order-independent, hence bit-reproducible and equal to the sorted path's.
 #include "skm_common.cuh"
 #include "skm_tile.cuh"
@@ -109,23 +108,6 @@ __global__ void __launch_bounds__(256) rows_colsum_kernel(const uint32_t *__rest
     }
 }
 
-// out[i + shift(i)] = in[i], shift(i) = cum[h] for the largest h with pos[h] <= i (cum[0] = 0 for i below pos[0]):
-// pos[h] = index in the light list where heavy annotation h's block is inserted, cum[h] = entries of heavy 0..h
-__global__ void __launch_bounds__(256) coo_shift_copy_kernel(const uint64_t *__restrict__ keys, const int64_t *__restrict__ vals,
-                                                             int64_t n, const int64_t *__restrict__ pos, const int64_t *__restrict__ cum,
-                                                             int n_heavy, uint64_t *__restrict__ keys_out, int64_t *__restrict__ vals_out) {
-    for (int64_t i = int64_t(blockIdx.x) * blockDim.x + threadIdx.x; i < n; i += int64_t(gridDim.x) * blockDim.x) {
-        int lo = 0, hi = n_heavy;                           // number of heavy blocks inserted at or before i
-        while (lo < hi) {
-            const int mid = (lo + hi) >> 1;
-            if (__ldg(pos + mid) <= i) lo = mid + 1; else hi = mid;
-        }
-        const int64_t shift = lo ? __ldg(cum + lo - 1) : 0;
-        keys_out[i + shift] = keys[i];
-        vals_out[i + shift] = vals[i];
-    }
-}
-
 }  // namespace skm
 
 extern "C" {
@@ -187,18 +169,6 @@ int skm_rows_colsum(const uint32_t *d_rows, int64_t n_rows, int64_t S, int64_t *
     const int grid = (int)std::min<int64_t>((S + 255) / 256, int64_t(sm_count()) * 16);
     rows_colsum_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_rows, S, (int)n_rows, reinterpret_cast<unsigned long long *>(d_totals));
     SKM_LAUNCH_CHECK("rows_colsum_kernel");
-    return SKM_OK;
-}
-
-int skm_coo_shift_copy(const uint64_t *d_keys, const int64_t *d_vals, int64_t n, const int64_t *d_insert_pos, const int64_t *d_insert_cum,
-                       int64_t n_insert, uint64_t *d_keys_out, int64_t *d_vals_out, skm_stream_t stream) {
-    using namespace skm;
-    if (n < 0 || n_insert < 0 || n_insert > (1 << 30)) { set_error("skm_coo_shift_copy: bad sizes"); return SKM_ERR_INVALID; }
-    if (n == 0) return SKM_OK;
-    if (!d_keys || !d_vals || !d_keys_out || !d_vals_out || (n_insert > 0 && (!d_insert_pos || !d_insert_cum))) { set_error("skm_coo_shift_copy: NULL argument"); return SKM_ERR_INVALID; }
-    const int grid = (int)std::min<int64_t>((n + 255) / 256, int64_t(sm_count()) * 16);
-    coo_shift_copy_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_keys, d_vals, n, d_insert_pos, d_insert_cum, (int)n_insert, d_keys_out, d_vals_out);
-    SKM_LAUNCH_CHECK("coo_shift_copy_kernel");
     return SKM_OK;
 }
 

@@ -872,8 +872,76 @@ def coo_pack(keys: torch.Tensor, vals: torch.Tensor, count_bits: int) -> Tuple[t
     return out, bool(flag.item())
 
 
+GROUP_MAX_RES = (1 << 31) - 64      # residues per skm_learn_sparse_group call (its 32-bit window keys need < 2^31)
+
+
+@dataclass
+class _Placement:
+    """Room for H foreign blocks (the dense rows of learn_sparse_hybrid's heavy annotations) inside the grouped list:
+    skm_learn_sparse_group_place writes every entry straight to its place in the larger list."""
+    ins_ann: torch.Tensor               # int64 [H] ascending annotation ids of the blocks
+    ins_cum: Optional[torch.Tensor]     # int64 [H] inclusive prefix of the block sizes (None when H = 0)
+    ins_pos: torch.Tensor               # int64 [H] INT64_MAX on entry; skm_learn_sparse_group_place's candidates per block
+    totals: Optional[torch.Tensor]      # int64 [S] += counts per code, or None
+    extra: int                          # entries of all blocks
+
+
+def _learn_grouped(batch: SequenceBatch, tab: AlphabetTables, k: int, ann_id: torch.Tensor, n_ann: int,
+                   place: Optional[_Placement] = None):
+    """The grouped path of learn_sparse: the annotated sequences are gathered in annotation order and sorted one
+    annotation slice at a time with 32-bit keys (skm_learn_sparse_group; with `place`, skm_learn_sparse_group_place).
+    ann_id: int32 on the device.  Returns (keys buffer, vals buffer, entries of the grouped list) without slicing — with
+    `place` the buffers also have room for its blocks — or None when the path does not apply (no sequences, no
+    annotations, a code space beyond 32-bit slice keys, or a slice of GROUP_MAX_RES residues or more)."""
+    dev = batch.device
+    S = code_space(tab.nsym, k)
+    per_group = ((1 << 32) - 2) // S
+    if per_group < 1 or batch.n == 0 or n_ann == 0:
+        return None
+    extra = place.extra if place is not None else 0
+    key = torch.where((ann_id >= 0) & (ann_id < n_ann), ann_id, torch.full_like(ann_id, n_ann))
+    sk, order = torch.sort(key, stable=True)
+    starts = list(range(0, n_ann, per_group)) + [n_ann]
+    bounds = torch.searchsorted(sk, torch.tensor(starts, dtype=torch.int32, device=dev)).tolist()     # one sync
+    n_sel = bounds[-1]
+    if n_sel == 0:
+        cap = max(extra, 1)
+        return torch.empty(cap, dtype=torch.int64, device=dev), torch.empty(cap, dtype=torch.int64, device=dev), 0
+    g_res, g_off = gather_sequences(batch, order[:n_sel])
+    g_ann = sk[:n_sel].contiguous()
+    edge = g_off[torch.tensor(bounds, dtype=torch.int64, device=dev)].tolist()
+    if max(edge[i + 1] - (edge[i] & ~15) for i in range(len(starts) - 1)) >= GROUP_MAX_RES:
+        return None
+    total = edge[-1] + extra
+    keys = torch.empty(max(total, 1), dtype=torch.int64, device=dev)
+    vals = torch.empty(max(total, 1), dtype=torch.int64, device=dev)
+    dn = torch.zeros(1, dtype=torch.int64, device=dev)
+    ws = None
+    for gi in range(len(starts) - 1):
+        s0, s1 = bounds[gi], bounds[gi + 1]
+        if s1 == s0:
+            continue
+        base = edge[gi] & ~15
+        nres = edge[gi + 1] - base
+        ws_bytes = lib().skm_learn_sparse_group_workspace(nres)
+        if ws is None or ws.numel() < ws_bytes:
+            ws = None
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        offs = (g_off[s0:s1 + 1] - base).contiguous()
+        args = (_ptr(g_res[base:]), nres, _ptr(offs), s1 - s0, _ptr(tab.lut), tab.nsym, int(k), _ptr(g_ann[s0:s1]), starts[gi],
+                starts[gi + 1] - starts[gi], _ptr(keys), _ptr(vals), total, _ptr(dn))
+        if place is not None:
+            check(lib().skm_learn_sparse_group_place(*args, _ptr(place.ins_ann), _ptr(place.ins_cum), int(place.ins_pos.numel()),
+                                                     _ptr(place.ins_pos), _ptr(place.totals), _ptr(ws), ws.numel(), _stream()))
+        else:
+            check(lib().skm_learn_sparse_group(*args, _ptr(ws), ws.numel(), _stream()))
+    m = int(dn.item())
+    assert m <= total
+    return keys, vals, m
+
+
 def learn_sparse(batch: SequenceBatch, alphabet, k: int, ann_id: torch.Tensor, n_ann: int,
-                 max_chunk_res: int = 1 << 28, method: str = "grouped", place: Optional[dict] = None):
+                 max_chunk_res: int = 1 << 28, method: str = "grouped") -> Tuple[torch.Tensor, torch.Tensor]:
     """Annotation x k-mer count matrix as a COO list sorted by key = ann * S + code
     (keys int64 holding the uint64 pattern, vals int64).  Sequences with ann_id < 0 do not
     contribute (Totals come from the basis tables).
@@ -881,66 +949,18 @@ def learn_sparse(batch: SequenceBatch, alphabet, k: int, ann_id: torch.Tensor, n
     method "grouped" (default): the annotated sequences are gathered in annotation order and sorted one annotation
     slice at a time with 32-bit keys (skm_learn_sparse_group); "global": one 64-bit radix sort over all window keys of
     the shard (skm_learn_sparse, the first implementation, kept as a cross-check and for slices whose keys need more
-    than 32 bits).
-    place (grouped path only; learn_sparse_hybrid): dict(ins_ann, ins_cum, ins_pos int64 [H], totals int64 [S] or None,
-    extra int) — the list is written straight into a larger list with room for H foreign blocks
-    (skm_learn_sparse_group_place); returns (keys buffer, vals buffer, entries of THIS list) without slicing, or None when
-    the grouped path does not apply (the caller then places the list itself)."""
+    than 32 bits)."""
+    if method not in ("grouped", "global"):
+        raise ValueError(f"learn_sparse: method must be 'grouped' or 'global', not {method!r}")
     tab = alphabet_tables(alphabet, batch.device)
     dev = batch.device
     ann_id = ann_id.to(device=dev, dtype=torch.int32).contiguous()
     assert ann_id.numel() == batch.n
     S = code_space(tab.nsym, k)
-    per_group = ((1 << 32) - 2) // S
-    if method == "grouped" and per_group >= 1 and batch.n > 0 and n_ann > 0:
-        key = torch.where((ann_id >= 0) & (ann_id < n_ann), ann_id, torch.full_like(ann_id, n_ann))
-        sk, order = torch.sort(key, stable=True)
-        starts = list(range(0, n_ann, per_group)) + [n_ann]
-        bounds = torch.searchsorted(sk, torch.tensor(starts, dtype=torch.int32, device=dev)).tolist()     # one sync
-        n_sel = bounds[-1]
-        if n_sel == 0:
-            if place:
-                cap = max(int(place["extra"]), 1)
-                return torch.empty(cap, dtype=torch.int64, device=dev), torch.empty(cap, dtype=torch.int64, device=dev), 0
-            z = torch.zeros(0, dtype=torch.int64, device=dev)
-            return z, z.clone()
-        g_res, g_off = gather_sequences(batch, order[:n_sel])
-        g_ann = sk[:n_sel].contiguous()
-        edge = g_off[torch.tensor(bounds, dtype=torch.int64, device=dev)].tolist()
-        if max(edge[i + 1] - (edge[i] & ~15) for i in range(len(starts) - 1)) < (1 << 31) - 64:
-            total = edge[-1] + (int(place["extra"]) if place else 0)
-            keys = torch.empty(max(total, 1), dtype=torch.int64, device=dev)
-            vals = torch.empty(max(total, 1), dtype=torch.int64, device=dev)
-            dn = torch.zeros(1, dtype=torch.int64, device=dev)
-            ws = None
-            for gi in range(len(starts) - 1):
-                s0, s1 = bounds[gi], bounds[gi + 1]
-                if s1 == s0:
-                    continue
-                base = edge[gi] & ~15
-                nres = edge[gi + 1] - base
-                ws_bytes = lib().skm_learn_sparse_group_workspace(nres)
-                if ws is None or ws.numel() < ws_bytes:
-                    ws = None
-                    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-                offs = (g_off[s0:s1 + 1] - base).contiguous()
-                if place:
-                    check(lib().skm_learn_sparse_group_place(_ptr(g_res[base:]), nres, _ptr(offs), s1 - s0, _ptr(tab.lut), tab.nsym, int(k),
-                                                             _ptr(g_ann[s0:s1]), starts[gi], starts[gi + 1] - starts[gi], _ptr(keys), _ptr(vals),
-                                                             total, _ptr(dn), _ptr(place["ins_ann"]), _ptr(place["ins_cum"]),
-                                                             int(place["ins_ann"].numel()), _ptr(place["ins_pos"]), _ptr(place.get("totals")),
-                                                             _ptr(ws), ws.numel(), _stream()))
-                else:
-                    check(lib().skm_learn_sparse_group(_ptr(g_res[base:]), nres, _ptr(offs), s1 - s0, _ptr(tab.lut), tab.nsym, int(k),
-                                                       _ptr(g_ann[s0:s1]), starts[gi], starts[gi + 1] - starts[gi], _ptr(keys), _ptr(vals),
-                                                       total, _ptr(dn), _ptr(ws), ws.numel(), _stream()))
-            m = int(dn.item())
-            assert m <= total
-            if place:
-                return keys, vals, m
-            return keys[:m].clone(), vals[:m].clone()
-    if place:
-        return None
+    grouped = _learn_grouped(batch, tab, k, ann_id, n_ann) if method == "grouped" else None
+    if grouped is not None:
+        keys, vals, m = grouped
+        return keys[:m].clone(), vals[:m].clone()
     parts_k, parts_v = [], []
     for lo, hi in _chunks_by_residues(batch.offsets_host, max_chunk_res):
         sub = _sub_batch(batch, lo, hi)
@@ -964,35 +984,49 @@ def learn_sparse(batch: SequenceBatch, alphabet, k: int, ann_id: torch.Tensor, n
     return coo_merge(torch.cat(parts_k), torch.cat(parts_v), key_bound=n_ann * S)
 
 
-HEAVY_ROW_DIV = int(os.environ.get("SKM_HEAVY_ROW_DIV", "4"))   # an annotation is "heavy" when it has more residues than S / HEAVY_ROW_DIV ...
-HEAVY_ROWS_MAX_BYTES = 8 << 30   # ... as long as the dense rows of all heavy annotations stay below this
-ROWS_L2_BYTES = int(os.environ.get("SKM_ROWS_L2_MB", "100")) << 20   # rows counted by one skm_rows_accumulate launch (L2-resident counters): ~0.8 of the 126 MB L2, from a sweep (profiles/R2al_*)
+def _learn_sorted(batch: SequenceBatch, tab: AlphabetTables, k: int, ann_id: torch.Tensor, n_ann: int, want_totals: bool):
+    """The all-sorted path (the reference of the hybrid one): learn_sparse, and with want_totals the Totals row — the
+    annotated share is the column sums of the matrix (one atomic per entry instead of one per window), the unannotated
+    sequences are counted window by window.  ann_id: int32 on the device."""
+    keys, vals = learn_sparse(batch, tab, k, ann_id, n_ann)
+    if not want_totals:
+        return keys, vals
+    dev = batch.device
+    S = code_space(tab.nsym, k)
+    totals = torch.zeros(S, dtype=torch.int64, device=dev)
+    check(lib().skm_coo_colsum(_ptr(keys), _ptr(vals), keys.numel(), S, _ptr(totals), _stream()))
+    rest = torch.nonzero((ann_id < 0) | (ann_id >= n_ann)).reshape(-1)
+    if rest.numel():
+        g_res, g_off = gather_sequences(batch, rest)
+        basis_accumulate(SequenceBatch(g_res, g_off, g_off.cpu().numpy()), tab, k, totals, None, 0)
+    return keys, vals, totals
+
+
+HEAVY_ROW_DIV = 4                   # an annotation is "heavy" when it has more residues than S / HEAVY_ROW_DIV ...
+HEAVY_ROWS_MAX_BYTES = 8 << 30      # ... as long as the dense rows of all heavy annotations stay below this
+ROWS_L2_BYTES = 100 << 20           # rows counted by one skm_rows_accumulate launch (L2-resident counters): ~0.8 of the 126 MB L2, from a sweep (profiles/R2al_*)
 
 
 def _learn_rows(batch: SequenceBatch, tab: AlphabetTables, k: int, ann_id: torch.Tensor, n_ann: int, S: int,
-                want_totals: bool, heavy_div: int, min_res: int = 0, heavy_ids: Optional[torch.Tensor] = None):
-    """Dense-row part of learn_sparse_hybrid: returns (rows uint32 [R, S], heavy annotation ids int64 [H] ascending,
-    rest_row index or -1).  Rows 0..H-1 are the heavy annotations, row H (when want_totals) the unannotated sequences."""
+                want_totals: bool, heavy_div: int):
+    """Dense-row part of learn_sparse_hybrid: returns (rows uint32 [R, S] or None when R = 0, heavy annotation ids
+    int64 [H] ascending).  Rows 0..H-1 are the heavy annotations, row H (when want_totals) the unannotated sequences."""
     dev = batch.device
     lens = (batch.offsets[1:] - batch.offsets[:-1])
     valid = (ann_id >= 0) & (ann_id < n_ann)
     per_ann = torch.zeros(n_ann + 1, dtype=torch.int64, device=dev)
     per_ann.index_add_(0, torch.where(valid, ann_id, torch.full_like(ann_id, n_ann)).to(torch.int64), lens)
-    if heavy_ids is not None:                            # the caller chose the rows (ascending ids)
-        heavy = heavy_ids.to(device=dev, dtype=torch.int64)
-    else:
-        thr = max(S // max(int(heavy_div), 1), 1, int(min_res))
-        heavy_mask = per_ann[:n_ann] > thr
-        max_rows = max(int(HEAVY_ROWS_MAX_BYTES // (4 * S)) - 1, 0)
-        heavy = torch.nonzero(heavy_mask).reshape(-1)
-        if heavy.numel() > max_rows:                         # keep the largest ones
-            order = torch.argsort(per_ann[heavy], descending=True)[:max_rows]
-            heavy = torch.sort(heavy[order]).values
+    thr = max(S // max(int(heavy_div), 1), 1)
+    max_rows = max(int(HEAVY_ROWS_MAX_BYTES // (4 * S)) - 1, 0)
+    heavy = torch.nonzero(per_ann[:n_ann] > thr).reshape(-1)
+    if heavy.numel() > max_rows:                         # keep the largest ones
+        order = torch.argsort(per_ann[heavy], descending=True)[:max_rows]
+        heavy = torch.sort(heavy[order]).values
     H = int(heavy.numel())                               # one sync
     rest_row = H if want_totals else -1
     R = H + (1 if want_totals else 0)
     if R == 0:
-        return None, heavy, -1
+        return None, heavy
     row_of_ann = torch.full((n_ann + 1,), -1, dtype=torch.int32, device=dev)
     row_of_ann[heavy] = torch.arange(H, dtype=torch.int32, device=dev)
     row_of_ann[n_ann] = rest_row
@@ -1032,24 +1066,32 @@ def _learn_rows(batch: SequenceBatch, tab: AlphabetTables, k: int, ann_id: torch
             offs = (g_off[lo:hi + 1] - base).contiguous()
             check(lib().skm_rows_accumulate(_ptr(g_res[base:]), e1 - base, _ptr(offs), hi - lo, _ptr(tab.lut), tab.nsym, int(k),
                                             _ptr(g_row[lo:hi]), int(S), _ptr(rows), _stream()))
-    return rows, heavy, rest_row
+    return rows, heavy
 
 
-def learn_sparse_hybrid(batch: SequenceBatch, alphabet, k: int, ann_id: torch.Tensor, n_ann: int, want_totals: bool = False,
-                        heavy_div: int = HEAVY_ROW_DIV):
-    """learn_sparse for heavy-tailed family sizes: annotations with more residues than S / heavy_div are COUNTED into
-    dense L2-resident rows (skm_rows_accumulate; their sequences gathered together), the others are sorted
-    (skm_learn_sparse_group); the two sorted lists are interleaved by annotation.  Same result as learn_sparse, bit for
-    bit.  want_totals: also return the Totals row (int64 [S], occurrences over ALL sequences, learn.smk:380) — the
-    unannotated sequences are then counted into a row of their own and the totals are column sums."""
-    tab = alphabet_tables(alphabet, batch.device)
+def _row_blocks(rows: Optional[torch.Tensor], H: int, S: int):
+    """Layout of the heavy rows' entries in the COO list: (blk_off int64 [H, nblk] exclusive non-zeros in front of each
+    block inside its row, row_nnz int64 [H], cum int64 [H] inclusive prefix of row_nnz, heavy_total); all None / 0 when
+    H == 0."""
+    if H == 0:
+        return None, None, None, 0
+    blk = lib().skm_rows_block()
+    counts = torch.empty((H, (S + blk - 1) // blk), dtype=torch.int32, device=rows.device)
+    check(lib().skm_rows_block_counts(_ptr(rows), H, S, _ptr(counts), _stream()))
+    c64 = counts.to(torch.int64)
+    incl = torch.cumsum(c64, dim=1)
+    blk_off = (incl - c64).contiguous()
+    row_nnz = incl[:, -1].contiguous()
+    cum = torch.cumsum(row_nnz, 0).contiguous()
+    return blk_off, row_nnz, cum, int(cum[-1].item())    # one sync
+
+
+def _learn_hybrid(batch: SequenceBatch, tab: AlphabetTables, k: int, ann_id: torch.Tensor, n_ann: int, S: int,
+                  want_totals: bool, heavy_div: int):
     dev = batch.device
-    S = code_space(tab.nsym, k)
-    ann_id = ann_id.to(device=dev, dtype=torch.int32).contiguous()
-    assert ann_id.numel() == batch.n
-    if S > _native.SKM_DENSE_MAX_SPACE:
-        raise SkmError(-3, f"code space {tab.nsym}^{k} exceeds the table limit 2^27")
-    rows, heavy, rest_row = _learn_rows(batch, tab, k, ann_id, n_ann, S, want_totals, heavy_div) if batch.n and n_ann else (None, torch.zeros(0, dtype=torch.int64, device=dev), -1)
+    if batch.n == 0 or n_ann == 0:
+        return _learn_sorted(batch, tab, k, ann_id, n_ann, want_totals)
+    rows, heavy = _learn_rows(batch, tab, k, ann_id, n_ann, S, want_totals, heavy_div)
     H = int(heavy.numel())
     totals = torch.zeros(S, dtype=torch.int64, device=dev) if want_totals else None
     # light part: the heavy annotations (and, with totals, nothing else) leave the sorted path
@@ -1060,250 +1102,63 @@ def learn_sparse_hybrid(batch: SequenceBatch, alphabet, k: int, ann_id: torch.Te
         ann_light = torch.where(is_heavy[safe], torch.full_like(ann_id, -1), ann_id)
     else:
         ann_light = ann_id
-    if H and os.environ.get("SKM_LEARN_PLACE", "1") != "0":
-        # The heavy blocks' sizes first (the rows are counted already), then the light list is sorted slice by slice and
-        # written STRAIGHT to its final places between the heavy blocks, adding its counts to the Totals on the way
-        # (skm_learn_sparse_group_place): no separate column-sum pass over the light list and no shift copy of it.
-        blk = lib().skm_rows_block()
-        nblk = (S + blk - 1) // blk
-        counts = torch.empty((H, nblk), dtype=torch.int32, device=dev)
-        check(lib().skm_rows_block_counts(_ptr(rows), H, S, _ptr(counts), _stream()))
-        c64 = counts.to(torch.int64)
-        incl = torch.cumsum(c64, dim=1)
-        blk_off = (incl - c64).contiguous()
-        row_nnz = incl[:, -1].contiguous()
-        cum = torch.cumsum(row_nnz, 0).contiguous()          # inclusive
-        heavy_total = int(cum[-1].item())                    # one sync
-        ins_pos = torch.full((H,), INT64_MAX, dtype=torch.int64, device=dev)
-        placed = learn_sparse(batch, alphabet, k, ann_light, n_ann,
-                              place=dict(ins_ann=heavy.contiguous(), ins_cum=cum, ins_pos=ins_pos, totals=totals, extra=heavy_total))
-        if placed is not None:
-            keys, vals, m_light = placed
-            if want_totals:
-                check(lib().skm_rows_colsum(_ptr(rows), rows.shape[0], S, _ptr(totals), _stream()))
-            # light entries in front of block h = the smallest recorded index over the blocks from h on (none: all of them)
-            tail = torch.cat([ins_pos, torch.tensor([m_light], dtype=torch.int64, device=dev)])
-            before = torch.flip(torch.cummin(torch.flip(tail, [0]), 0).values, [0])[:H]
-            row_dst = (before + cum - row_nnz).contiguous()
-            total = m_light + heavy_total
-            check(lib().skm_rows_emit(_ptr(rows), H, S, _ptr(blk_off), _ptr(row_dst), _ptr(heavy.contiguous()), _ptr(keys), _ptr(vals), total, _stream()))
-            keys, vals = keys[:total], vals[:total]
-            return (keys, vals, totals) if want_totals else (keys, vals)
-    kl, vl = learn_sparse(batch, alphabet, k, ann_light, n_ann)
+    # The heavy blocks' sizes first (the rows are counted already), then the light list is sorted slice by slice and
+    # written STRAIGHT to its final places between the heavy blocks, adding its counts to the Totals on the way
+    # (skm_learn_sparse_group_place): no column-sum pass over the light list and no copy of it.
+    blk_off, row_nnz, cum, heavy_total = _row_blocks(rows, H, S)
+    ins_pos = torch.full((H,), INT64_MAX, dtype=torch.int64, device=dev)
+    placed = _learn_grouped(batch, tab, k, ann_light, n_ann, _Placement(heavy, cum, ins_pos, totals, heavy_total))
+    if placed is None:
+        return _learn_sorted(batch, tab, k, ann_id, n_ann, want_totals)
+    keys, vals, m_light = placed
     if want_totals:
-        check(lib().skm_coo_colsum(_ptr(kl), _ptr(vl), kl.numel(), S, _ptr(totals), _stream()))
-        if rows is not None:
-            check(lib().skm_rows_colsum(_ptr(rows), rows.shape[0], S, _ptr(totals), _stream()))
-        else:                                           # no row machinery (empty batch / no annotations): count the rest directly
-            rest = torch.nonzero((ann_id < 0) | (ann_id >= n_ann)).reshape(-1)
-            if rest.numel():
-                g_res, g_off = gather_sequences(batch, rest)
-                basis_accumulate(SequenceBatch(g_res, g_off, g_off.cpu().numpy()), alphabet, k, totals, None, 0)
-    if H == 0:
-        return (kl, vl, totals) if want_totals else (kl, vl)
-    # heavy part: non-zeros per block -> places -> emit
-    blk = lib().skm_rows_block()
-    nblk = (S + blk - 1) // blk
-    counts = torch.empty((H, nblk), dtype=torch.int32, device=dev)
-    check(lib().skm_rows_block_counts(_ptr(rows), H, S, _ptr(counts), _stream()))
-    c64 = counts.to(torch.int64)
-    incl = torch.cumsum(c64, dim=1)
-    blk_off = (incl - c64).contiguous()                  # exclusive inside a row
-    row_nnz = incl[:, -1].contiguous()
-    # where the heavy blocks go: position in the light list (entries of smaller annotations) + heavy entries before
-    ins_pos = torch.searchsorted(kl, heavy * S).contiguous()
-    cum = torch.cumsum(row_nnz, 0).contiguous()          # inclusive
-    row_dst = (ins_pos + cum - row_nnz).contiguous()
-    total = int(kl.numel()) + int(cum[-1].item())        # one sync
-    keys = torch.empty(max(total, 1), dtype=torch.int64, device=dev)
-    vals = torch.empty(max(total, 1), dtype=torch.int64, device=dev)
-    check(lib().skm_coo_shift_copy(_ptr(kl), _ptr(vl), kl.numel(), _ptr(ins_pos), _ptr(cum), H, _ptr(keys), _ptr(vals), _stream()))
-    check(lib().skm_rows_emit(_ptr(rows), H, S, _ptr(blk_off), _ptr(row_dst), _ptr(heavy.contiguous()), _ptr(keys), _ptr(vals), total, _stream()))
+        check(lib().skm_rows_colsum(_ptr(rows), rows.shape[0], S, _ptr(totals), _stream()))
+    total = m_light + heavy_total
+    if H:
+        # light entries in front of block h = the smallest recorded index over the blocks from h on (none: all of them)
+        tail = torch.cat([ins_pos, torch.tensor([m_light], dtype=torch.int64, device=dev)])
+        before = torch.flip(torch.cummin(torch.flip(tail, [0]), 0).values, [0])[:H]
+        row_dst = (before + cum - row_nnz).contiguous()
+        check(lib().skm_rows_emit(_ptr(rows), H, S, _ptr(blk_off), _ptr(row_dst), _ptr(heavy.contiguous()), _ptr(keys), _ptr(vals), total, _stream()))
     keys, vals = keys[:total], vals[:total]
     return (keys, vals, totals) if want_totals else (keys, vals)
 
 
-ONCHIP_HEAVY_SCALE = float(os.environ.get("SKM_ONCHIP_HEAVY_SCALE", "0.75"))   # dense rows beyond scale * sqrt(task capacity * S) residues
-ONCHIP_FILL = 0.8                                                      # target fill of a task cut from the code histogram
-
-
-def _hist_bins(nsym: int, k: int, S: int) -> Tuple[int, int]:
-    """(n_bins, bin_width) of the per-annotation code histogram: the leading j symbols of a code, nsym^j <= 8192."""
-    j = 0
-    while j < k and nsym ** (j + 1) <= 8192:
-        j += 1
-    return nsym ** j, nsym ** (k - j)
-
-
-def learn_sparse_onchip(batch: SequenceBatch, alphabet, k: int, ann_id: torch.Tensor, n_ann: int, want_totals: bool = False,
-                        heavy_scale: float = ONCHIP_HEAVY_SCALE):
-    """learn_sparse without a device-wide sort.  Annotations with more than heavy_scale * sqrt(task capacity * S) residues
-    (where a dense row of S counters — ~20 bytes of traffic per code — costs less than the n^2 / capacity window scans of
-    the tasks the annotation would be cut into; C3: 158 k residues) are
-    counted into dense L2-resident rows (skm_rows_*); every other annotation is sorted ON CHIP by skm_ann_sort: one CTA
-    per task (annotation x code range, at most skm_ann_sort_cap() windows) scans, radix-sorts and run-length-encodes in
-    shared memory and writes its entries at their final place of the one sorted COO list.  Annotations larger than a task
-    are cut into code ranges from an exact histogram (skm_ann_hist).  Same result as learn_sparse, bit for bit; falls
-    back to learn_sparse_hybrid when a histogram bin alone exceeds a task (degenerate low-complexity input).
-    want_totals: also the Totals row (learn.smk:380)."""
+def learn_sparse_hybrid(batch: SequenceBatch, alphabet, k: int, ann_id: torch.Tensor, n_ann: int, want_totals: bool = False,
+                        heavy_div: int = HEAVY_ROW_DIV):
+    """learn_sparse for heavy-tailed family sizes: annotations with more residues than S / heavy_div are COUNTED into
+    dense L2-resident rows (skm_rows_accumulate; their sequences gathered together), the others are sorted
+    (skm_learn_sparse_group_place) straight into the gaps between the heavy rows' entries.  Same result as learn_sparse,
+    bit for bit; inputs the grouped sort cannot take (a slice of GROUP_MAX_RES residues or more, no sequences, no
+    annotations) get the all-sorted result.  want_totals: also return the Totals row (int64 [S], occurrences over ALL
+    sequences, learn.smk:380) — the unannotated sequences are then counted into a row of their own and the totals are
+    column sums."""
     tab = alphabet_tables(alphabet, batch.device)
-    dev = batch.device
     S = code_space(tab.nsym, k)
-    ann_id = ann_id.to(device=dev, dtype=torch.int32).contiguous()
-    assert ann_id.numel() == batch.n
     if S > _native.SKM_DENSE_MAX_SPACE:
         raise SkmError(-3, f"code space {tab.nsym}^{k} exceeds the table limit 2^27")
-    if batch.n == 0 or n_ann == 0:
-        return learn_sparse_hybrid(batch, alphabet, k, ann_id, n_ann, want_totals=want_totals)
-    T = int(lib().skm_ann_sort_cap())
-    thr = max(T, int(heavy_scale * (float(T) * float(S)) ** 0.5))
-    max_rows = max(int(HEAVY_ROWS_MAX_BYTES // (4 * S)) - 1, 0)
-    ok_id = (ann_id >= 0) & (ann_id < n_ann)
-    safe = torch.where(ok_id, ann_id, torch.full_like(ann_id, n_ann)).to(torch.int64)
-    lens = batch.offsets[1:] - batch.offsets[:-1]
-    per_ann = torch.zeros(n_ann + 1, dtype=torch.int64, device=dev)
-    per_ann.index_add_(0, safe, lens)
-    heavy = torch.nonzero(per_ann[:n_ann] > thr).reshape(-1)
-    if heavy.numel() > max_rows:                                      # keep the largest ones as rows
-        heavy = torch.sort(heavy[torch.argsort(per_ann[heavy], descending=True)[:max_rows]]).values
-    # ---- task annotations: sequences gathered in annotation order -------------------------------------------------------
-    is_heavy = torch.zeros(n_ann + 1, dtype=torch.bool, device=dev)
-    is_heavy[heavy] = True
-    key = torch.where(ok_id & ~is_heavy[safe], ann_id, torch.full_like(ann_id, n_ann))
-    sk, order = torch.sort(key, stable=True)
-    uniq, per = torch.unique_consecutive(sk, return_counts=True)
-    if uniq.numel() and int(uniq[-1].item()) == n_ann:                # the unselected sequences sort last
-        uniq, per = uniq[:-1], per[:-1]
-    A = int(uniq.numel())
-    n_tasks = 0
-    if A:
-        seq_hi = torch.cumsum(per, 0)
-        seq_lo = seq_hi - per
-        n_sel = int(seq_hi[-1].item())
-        g_res, g_off = gather_sequences(batch, order[:n_sel])
-        nres_g = int(g_off[-1].item())
-        ares = g_off[seq_hi] - g_off[seq_lo]                          # residues per task annotation
-        medium = ares > T
-        mi = torch.nonzero(medium).reshape(-1)
-        M = int(mi.numel())
-        t_ann = [uniq[~medium].to(torch.int64)]
-        t_lo, t_hi = [seq_lo[~medium]], [seq_hi[~medium]]
-        t_c0 = [torch.zeros(A - M, dtype=torch.int64, device=dev)]
-        t_c1 = [torch.full((A - M,), S, dtype=torch.int64, device=dev)]
-        if M:
-            n_bins, width = _hist_bins(tab.nsym, k, S)
-            hist = torch.empty((M, n_bins), dtype=torch.int32, device=dev)
-            m_lo, m_hi = seq_lo[mi].to(torch.int32).contiguous(), seq_hi[mi].to(torch.int32).contiguous()
-            check(lib().skm_ann_hist(_ptr(g_res), nres_g, _ptr(g_off), n_sel, _ptr(tab.lut), tab.nsym, int(k), _ptr(m_lo), _ptr(m_hi), M,
-                                     width, n_bins, _ptr(hist), _stream()))
-            fill = int(T * ONCHIP_FILL)
-            # an annotation with one bin beyond what a task can absorb (low-complexity families) gets a dense row instead
-            hot = hist.max(dim=1).values.to(torch.int64) > T - fill
-            n_hot = int(hot.sum().item())
-            if n_hot:
-                heavy = torch.sort(torch.cat([heavy, uniq[mi][hot].to(torch.int64)])).values
-                if heavy.numel() > max_rows:
-                    return learn_sparse_hybrid(batch, alphabet, k, ann_id, n_ann, want_totals=want_totals)
-                keep = torch.nonzero(~hot).reshape(-1)
-                mi, hist = mi[keep], hist[keep]
-                M = int(mi.numel())
-        if M:
-            h64 = hist.to(torch.int64)
-            cum = torch.cumsum(h64, 1)
-            q = torch.div((cum - 1).clamp_(min=0), fill, rounding_mode="floor")
-            start = torch.ones_like(q, dtype=torch.bool)
-            start[:, 1:] = q[:, 1:] != q[:, :-1]
-            rb = torch.nonzero(start)                                 # (medium row, first bin) of every task, row-major
-            r_, b_ = rb[:, 0], rb[:, 1]
-            b_hi = torch.full_like(b_, n_bins)
-            b_hi[:-1] = torch.where(r_[1:] == r_[:-1], b_[1:], b_hi[:-1])
-            t_ann.append(uniq[mi][r_].to(torch.int64))
-            t_lo.append(seq_lo[mi][r_])
-            t_hi.append(seq_hi[mi][r_])
-            t_c0.append(b_ * width)
-            t_c1.append(torch.clamp(b_hi * width, max=S))
-        t_ann, t_lo, t_hi, t_c0, t_c1 = (torch.cat(x) for x in (t_ann, t_lo, t_hi, t_c0, t_c1))
-        perm = torch.argsort(t_ann * (S + 1) + t_c0)
-        t_ann = t_ann[perm].contiguous()
-        t_lo, t_hi = t_lo[perm].to(torch.int32).contiguous(), t_hi[perm].to(torch.int32).contiguous()
-        t_c0, t_c1 = t_c0[perm].to(torch.int32).contiguous(), t_c1[perm].to(torch.int32).contiguous()     # uint32 patterns (S <= 2^27)
-        n_tasks = int(t_ann.numel())
-    # ---- heavy rows (+ the row of the unannotated sequences): counted, then entries per row -------------------------------
-    rows, heavy, rest_row = _learn_rows(batch, tab, k, ann_id, n_ann, S, want_totals, heavy_div=S + 1, heavy_ids=heavy)
-    H = int(heavy.numel())
-    totals = torch.zeros(S, dtype=torch.int64, device=dev) if want_totals else None
-    if H:
-        blk = lib().skm_rows_block()
-        nblk = (S + blk - 1) // blk
-        counts = torch.empty((H, nblk), dtype=torch.int32, device=dev)
-        check(lib().skm_rows_block_counts(_ptr(rows), H, S, _ptr(counts), _stream()))
-        c64 = counts.to(torch.int64)
-        incl = torch.cumsum(c64, dim=1)
-        blk_off = (incl - c64).contiguous()
-        row_nnz = incl[:, -1].contiguous()
-        heavy_cum = torch.cat([torch.zeros(1, dtype=torch.int64, device=dev), torch.cumsum(row_nnz, 0)])    # exclusive, H + 1
-    else:
-        heavy_cum = torch.zeros(1, dtype=torch.int64, device=dev)
-    if n_tasks:
-        out_base = heavy_cum[torch.searchsorted(heavy, t_ann)].contiguous() if H else torch.zeros(n_tasks, dtype=torch.int64, device=dev)
-    heavy_total = int(heavy_cum[-1].item()) if H else 0
-    capacity = heavy_total + (nres_g if A else 0)
-    keys = torch.empty(max(capacity, 1), dtype=torch.int64, device=dev)
-    vals = torch.empty(max(capacity, 1), dtype=torch.int64, device=dev)
-    task_total = torch.zeros(1, dtype=torch.int64, device=dev)
-    flag = torch.zeros(1, dtype=torch.int32, device=dev)
-    if n_tasks:
-        task_prefix = torch.empty(n_tasks, dtype=torch.int64, device=dev)
-        ws_bytes = lib().skm_ann_sort_workspace(n_tasks)
-        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-        check(lib().skm_ann_sort(_ptr(g_res), nres_g, _ptr(g_off), n_sel, _ptr(tab.lut), tab.nsym, int(k), _ptr(t_lo), _ptr(t_hi), _ptr(t_c0),
-                                 _ptr(t_c1), _ptr(t_ann), _ptr(out_base), n_tasks, _ptr(keys), _ptr(vals), capacity, _ptr(task_prefix),
-                                 _ptr(totals), _ptr(task_total), _ptr(flag), _ptr(ws), ws_bytes, _stream()))
-    if rows is not None and want_totals:
-        check(lib().skm_rows_colsum(_ptr(rows), rows.shape[0], S, _ptr(totals), _stream()))
-    if H:
-        # a heavy annotation's block starts after its own heavy predecessors and after the task entries of smaller annotations
-        if n_tasks:
-            tp = torch.cat([task_prefix, task_total])
-            row_dst = (heavy_cum[:-1] + tp[torch.searchsorted(t_ann, heavy)]).contiguous()
-        else:
-            row_dst = heavy_cum[:-1].contiguous()
-        check(lib().skm_rows_emit(_ptr(rows), H, S, _ptr(blk_off), _ptr(row_dst), _ptr(heavy.contiguous()), _ptr(keys), _ptr(vals), capacity, _stream()))
-    n_task_entries, bad = torch.cat([task_total, flag.to(torch.int64)]).tolist()          # one sync
-    if bad:
-        return learn_sparse_hybrid(batch, alphabet, k, ann_id, n_ann, want_totals=want_totals)
-    total = heavy_total + n_task_entries
-    keys, vals = keys[:total], vals[:total]
-    return (keys, vals, totals) if want_totals else (keys, vals)
+    ann_id = ann_id.to(device=batch.device, dtype=torch.int32).contiguous()
+    assert ann_id.numel() == batch.n
+    return _learn_hybrid(batch, tab, k, ann_id, n_ann, S, want_totals, heavy_div)
 
 
-def learn_sparse_with_totals(batch: SequenceBatch, alphabet, k: int, ann_id: torch.Tensor, n_ann: int, method: Optional[str] = None):
+def learn_sparse_with_totals(batch: SequenceBatch, alphabet, k: int, ann_id: torch.Tensor, n_ann: int, method: str = "hybrid"):
     """learn_sparse + the Totals row (k-mer occurrences over ALL sequences, learn.smk:380) -> (keys, vals, totals int64 [S]).
     method "hybrid" (default): heavy annotations and the unannotated sequences are counted into dense rows, the Totals are
     column sums (learn_sparse_hybrid).  "sorted": everything through the sort; the annotated share of the totals is the
-    column sums of the matrix (one atomic per entry instead of one per window) and the unannotated sequences are
-    counted window by window (the round-1 path, kept as the cross-check)."""
+    column sums of the matrix and the unannotated sequences are counted window by window (the round-1 path, kept as the
+    cross-check)."""
+    if method not in ("hybrid", "sorted"):
+        raise ValueError(f"learn_sparse_with_totals: method must be 'hybrid' or 'sorted', not {method!r}")
     tab = alphabet_tables(alphabet, batch.device)
-    dev = batch.device
     S = code_space(tab.nsym, k)
     if S > _native.SKM_DENSE_MAX_SPACE:
         raise SkmError(-3, f"code space {tab.nsym}^{k} exceeds the table limit 2^27")
-    ann_id = ann_id.to(device=dev, dtype=torch.int32).contiguous()
-    method = method or os.environ.get("SKM_LEARN_METHOD", "hybrid")
-    if method == "onchip":
-        return learn_sparse_onchip(batch, alphabet, k, ann_id, n_ann, want_totals=True)
+    ann_id = ann_id.to(device=batch.device, dtype=torch.int32).contiguous()
+    assert ann_id.numel() == batch.n
     if method == "hybrid":
-        return learn_sparse_hybrid(batch, alphabet, k, ann_id, n_ann, want_totals=True)
-    keys, vals = learn_sparse(batch, alphabet, k, ann_id, n_ann)
-    totals = torch.zeros(S, dtype=torch.int64, device=dev)
-    check(lib().skm_coo_colsum(_ptr(keys), _ptr(vals), keys.numel(), S, _ptr(totals), _stream()))
-    rest = torch.nonzero((ann_id < 0) | (ann_id >= n_ann)).reshape(-1)
-    if rest.numel():
-        g_res, g_off = gather_sequences(batch, rest)
-        off_host = g_off.cpu().numpy()
-        sub = SequenceBatch(g_res, g_off, off_host)
-        basis_accumulate(sub, alphabet, k, totals, None, 0)
-    return keys, vals, totals
+        return _learn_hybrid(batch, tab, k, ann_id, n_ann, S, True, HEAVY_ROW_DIV)
+    return _learn_sorted(batch, tab, k, ann_id, n_ann, True)
 
 
 @dataclass

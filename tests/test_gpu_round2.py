@@ -271,6 +271,7 @@ def test_vectorize_rule_beyond_the_dense_envelope(a, k, n, tmp_path):
     ("miqs", 3, 2000, 40, 1.5, 0.5, 1),         # S = 1000, threshold S: only the biggest families
     (5, 4, 1500, 7, 1.1, 0.9, 4),               # few annotations, mostly unannotated
     (2, 8, 600, 5, 1.1, 0.0, 1 << 30),          # threshold 0: EVERY annotation is heavy, the light list is empty
+    (2, 8, 600, 300, 0.0, 0.2, 4),              # no heavy annotation: the light list alone, Totals added on the way
 ])
 def test_learn_sparse_hybrid_equals_sorted(a, k, n_seq, n_ann, zipf, frac_un, div):
     """Dense-row counting of the heavy annotations + sort of the light ones == the all-sorted path, bit for bit (keys,
@@ -281,6 +282,12 @@ def test_learn_sparse_hybrid_equals_sorted(a, k, n_seq, n_ann, zipf, frac_un, di
     ann = rng.permutation(n_ann)[rng.choice(n_ann, size=n_seq, p=w / w.sum())].astype(np.int32)      # heavy ids scattered
     ann[rng.random(n_seq) < frac_un] = -1
     ann[:3] = [n_ann + 5, -7, n_ann]                                      # ids outside [0, n_ann) count as unannotated
+    lut, syms = O.build_lut(a)
+    S = len(syms) ** k
+    ok = (ann >= 0) & (ann < n_ann)
+    per_ann = np.bincount(ann[ok], weights=np.array([len(s) for s in seqs])[ok], minlength=n_ann)
+    if (n_seq, n_ann) == (600, 300):
+        assert per_ann.max() <= S // div
     batch = E.SequenceBatch.from_strings(seqs)
     d_ann = torch.from_numpy(ann)
     k1, v1, t1 = E.learn_sparse_with_totals(batch, a, k, d_ann, n_ann, method="sorted")
@@ -288,19 +295,50 @@ def test_learn_sparse_hybrid_equals_sorted(a, k, n_seq, n_ann, zipf, frac_un, di
     assert torch.equal(k1, k2) and torch.equal(v1, v2) and torch.equal(t1, t2)
     k3, v3 = E.learn_sparse_hybrid(batch, a, k, d_ann, n_ann, want_totals=False, heavy_div=div)
     assert torch.equal(k1, k3) and torch.equal(v1, v3)
-    lut, syms = O.build_lut(a)
-    S = len(syms) ** k
     res, offs = O.pack(seqs)
     si, pos, code, valid = O.window_codes(res, offs, lut, len(syms), k)
     C = O.count_matrix(si, code, valid, n_seq, np.arange(S, dtype=np.uint64)).astype(np.int64)
     M = np.zeros((n_ann, S), dtype=np.int64)
-    ok = (ann >= 0) & (ann < n_ann)
     np.add.at(M, ann[ok], C[ok])
     got = np.zeros_like(M)
     kk = k2.cpu().numpy()
     got[kk // S, kk % S] = v2.cpu().numpy()
     assert np.array_equal(got, M) and np.array_equal(t2.cpu().numpy(), C.sum(axis=0))
     assert bool((k2[1:] > k2[:-1]).all()) if k2.numel() > 1 else True
+
+
+def test_learn_sparse_hybrid_falls_back_to_sorted(monkeypatch):
+    """Inputs the grouped sort cannot take get the all-sorted result, bit for bit: a slice of GROUP_MAX_RES residues or
+    more (the limit lowered below one slice; heavy rows are counted first), an empty batch, no annotations."""
+    a, k, n_ann = 2, 8, 300
+    rng = np.random.default_rng(77)
+    seqs = _rand_seqs(rng, 4000, 0, 300)
+    w = 1.0 / np.arange(1, n_ann + 1) ** 1.1
+    ann = rng.permutation(n_ann)[rng.choice(n_ann, size=len(seqs), p=w / w.sum())].astype(np.int32)
+    ann[rng.random(len(seqs)) < 0.3] = -1
+    S = len(O.build_lut(a)[1]) ** k
+    ok = ann >= 0
+    per_ann = np.bincount(ann[ok], weights=np.array([len(s) for s in seqs])[ok], minlength=n_ann)
+    assert per_ann.max() > S // E.HEAVY_ROW_DIV                          # the input has heavy rows
+    batch, d_ann = E.SequenceBatch.from_strings(seqs), torch.from_numpy(ann)
+    empty, no_ids = E.SequenceBatch.from_strings([]), torch.zeros(0, dtype=torch.int32)
+    k1, v1, t1 = E.learn_sparse_with_totals(batch, a, k, d_ann, n_ann, method="sorted")
+    edge_cases = [(empty, no_ids, n_ann), (batch, d_ann, 0)]
+    want_edge = [E.learn_sparse_with_totals(b, a, k, ids, n, method="sorted") for b, ids, n in edge_cases]
+    calls = []
+    sorted_path = E._learn_sorted
+    monkeypatch.setattr(E, "_learn_sorted", lambda *args: calls.append(1) or sorted_path(*args))
+    monkeypatch.setattr(E, "GROUP_MAX_RES", 1000)
+    k2, v2, t2 = E.learn_sparse_hybrid(batch, a, k, d_ann, n_ann, want_totals=True)
+    assert torch.equal(k1, k2) and torch.equal(v1, v2) and torch.equal(t1, t2)
+    k3, v3 = E.learn_sparse_hybrid(batch, a, k, d_ann, n_ann, want_totals=False)
+    assert torch.equal(k1, k3) and torch.equal(v1, v3)
+    k4, v4, t4 = E.learn_sparse_with_totals(batch, a, k, d_ann, n_ann)
+    assert torch.equal(k1, k4) and torch.equal(v1, v4) and torch.equal(t1, t4)
+    assert len(calls) == 3
+    for (b, ids, n), want in zip(edge_cases, want_edge):
+        got = E.learn_sparse_with_totals(b, a, k, ids, n)
+        assert all(torch.equal(x, y) for x, y in zip(got, want))
 
 
 def _syn6():
@@ -432,55 +470,6 @@ def test_packed_exchange_format_merges_like_the_unpacked_one(n_runs, count_bits,
             bigk = keys.clone()
             bigk[0] = 1 << (64 - count_bits)
             assert E.coo_pack(bigk, vals, count_bits)[1]
-
-
-@pytest.mark.parametrize("a,k,n_seq,n_ann,zipf,frac_un,scale", [
-    ("hydro", 10, 3000, 50, 1.1, 0.3, 0.75),     # S = 1024: everything above one task is a dense row
-    (2, 8, 4000, 300, 1.1, 0.3, 0.75),           # S = 6561: heavy head, small tail
-    (2, 8, 4000, 300, 0.0, 0.0, 0.75),           # uniform sizes: small tasks only
-    ("syn6", 8, 3000, 40, 1.1, 0.2, 10.0),       # S = 1,679,616, no dense rows: the head is cut into code-range tasks
-    ("syn6", 8, 3000, 40, 1.1, 0.2, 1e-6),       # same data, everything above one task is a dense row
-    ("syn6", 8, 2500, 3, 0.0, 0.0, 0.75),        # three annotations of ~125 k residues each: histogram-cut tasks
-    (5, 4, 1500, 7, 1.1, 0.9, 0.75),             # few annotations, mostly unannotated
-    ("miqs", 3, 50, 60, 0.0, 0.0, 0.75),         # more annotations than sequences: empty annotations
-])
-def test_learn_sparse_onchip_equals_sorted(a, k, n_seq, n_ann, zipf, frac_un, scale):
-    """skm_ann_sort / skm_ann_hist (one CTA sorts one annotation x code-range task in shared memory, decoupled look-back
-    for the output places) + dense rows for the heavy annotations == the all-sorted path, bit for bit (keys, values,
-    Totals)."""
-    if a == "syn6":
-        _syn6()
-    rng = np.random.default_rng(n_seq + n_ann)
-    seqs = _rand_seqs(rng, n_seq, 0, 300)
-    w = 1.0 / np.arange(1, n_ann + 1) ** zipf
-    ann = rng.permutation(n_ann)[rng.choice(n_ann, size=n_seq, p=w / w.sum())].astype(np.int32)
-    ann[rng.random(n_seq) < frac_un] = -1
-    ann[:3] = [n_ann + 5, -7, n_ann]
-    batch = E.SequenceBatch.from_strings(seqs)
-    d_ann = torch.from_numpy(ann)
-    k1, v1, t1 = E.learn_sparse_with_totals(batch, a, k, d_ann, n_ann, method="sorted")
-    k2, v2, t2 = E.learn_sparse_onchip(batch, a, k, d_ann, n_ann, want_totals=True, heavy_scale=scale)
-    assert k1.numel() == k2.numel(), (k1.numel(), k2.numel())
-    assert torch.equal(k1, k2) and torch.equal(v1, v2) and torch.equal(t1, t2)
-    k3, v3 = E.learn_sparse_onchip(batch, a, k, d_ann, n_ann, want_totals=False, heavy_scale=scale)
-    assert torch.equal(k1, k3) and torch.equal(v1, v3)
-
-
-def test_learn_sparse_onchip_degenerate_inputs():
-    """Low-complexity families (one histogram bin larger than a task -> the sorted fallback), windows shorter than k,
-    invalid residues only, an empty batch."""
-    _syn6()
-    rng = np.random.default_rng(5)
-    seqs = ["A" * 400] * 120 + ["AG" * 150] * 40 + _rand_seqs(rng, 300, 0, 200) + ["X" * 50, "AGI", ""]
-    ann = np.array([0] * 120 + [1] * 40 + list(rng.integers(0, 6, size=300)) + [2, 3, 4], dtype=np.int32)
-    batch = E.SequenceBatch.from_strings(seqs)
-    for scale in (10.0, 0.75):
-        k1, v1, t1 = E.learn_sparse_with_totals(batch, "syn6", 8, torch.from_numpy(ann), 6, method="sorted")
-        k2, v2, t2 = E.learn_sparse_onchip(batch, "syn6", 8, torch.from_numpy(ann), 6, want_totals=True, heavy_scale=scale)
-        assert torch.equal(k1, k2) and torch.equal(v1, v2) and torch.equal(t1, t2)
-    empty = E.SequenceBatch.from_strings([])
-    k0, v0, t0 = E.learn_sparse_onchip(empty, "syn6", 8, torch.zeros(0, dtype=torch.int32), 6, want_totals=True)
-    assert k0.numel() == 0 and v0.numel() == 0 and int(t0.sum().item()) == 0
 
 
 @pytest.mark.parametrize("a,k,n", [("miqs", 3, 3000), ("miqs", 3, 12), (2, 4, 400), ("hydro", 10, 2000), (0, 3, 40)])

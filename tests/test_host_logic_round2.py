@@ -1,5 +1,6 @@
 """CPU tests of the host-side logic added in round 2 (no GPU, no compute calls into the library)."""
 import numpy as np
+import pytest
 
 from snekmer_b200 import dist as D
 from snekmer_b200 import engine as E
@@ -25,12 +26,12 @@ def test_push_plan_layout_matches_all_to_all_order():
     assert D.push_plan(np.zeros((1, 1), dtype=np.int64), 0)[2] == 0
 
 
-def test_hist_bins_cover_the_code_space():
-    for nsym, k in [(6, 8), (2, 10), (10, 3), (20, 5), (3, 1), (7, 4)]:
-        S = nsym ** k
-        n_bins, width = E._hist_bins(nsym, k, S)
-        assert n_bins * width == S and 1 <= n_bins <= 8192
-        assert n_bins == S or n_bins * nsym > 8192          # the finest split that still fits the histogram
+def test_learn_methods_are_checked():
+    """An unknown learn method is an error, not a silent switch to another algorithm."""
+    with pytest.raises(ValueError, match="hybrid"):
+        E.learn_sparse_with_totals(None, "miqs", 3, None, 4, method="typo")
+    with pytest.raises(ValueError, match="grouped"):
+        E.learn_sparse(None, "miqs", 3, None, 4, method="sorted")
 
 
 def test_host_coo_unpacks_the_exchange_format():
