@@ -60,7 +60,7 @@ __global__ void __launch_bounds__(TS_THREADS) basis_kernel(const uint8_t *__rest
     const int tid = threadIdx.x;
     ts_lut_init(s_lut, lut);
     if (SMALL) for (int i = tid; i < S; i += blockDim.x) { if (!ORDER) s_cnt[i] = 0; s_min[i] = 0xFFFFFFFFu; }
-    if (tid == 0) { cta_seq_range(off, nseq, &s_range[0], &s_range[1]); s_nstart = 0; }
+    if (tid == 0) { seq_range(off, nseq, blockIdx.x, gridDim.x, &s_range[0], &s_range[1]); s_nstart = 0; }
     __syncthreads();
     const int64_t lo = s_range[0], hi = s_range[1];
     const int64_t r_lo = (lo < hi) ? __ldg(off + lo) : 0, r_hi = (lo < hi) ? __ldg(off + hi) : 0;
@@ -188,7 +188,6 @@ __global__ void colmap_scatter_kernel(const uint64_t *__restrict__ codes, int64_
     }
 }
 
-static size_t align_up(size_t x) { return (x + 255) & ~size_t(255); }
 
 // CTAs of a basis_kernel launch over nres residues with `smem` bytes of dynamic shared memory each
 static int64_t basis_grid(int64_t nres, size_t smem) {
@@ -299,7 +298,7 @@ size_t skm_basis_finalize_workspace(int64_t S) {
     size_t temp = 0;
     cub::DeviceRadixSort::SortPairs(nullptr, temp, (const uint64_t *)nullptr, (uint64_t *)nullptr,
                                     (const uint64_t *)nullptr, (uint64_t *)nullptr, (int64_t)S);
-    return 4 * align_up(size_t(S) * 8) + align_up(temp) + 256;
+    return 4 * align256(size_t(S) * 8) + align256(temp) + 256;
 }
 
 int skm_basis_finalize(const uint64_t *d_count, const uint64_t *d_first, int64_t S, int64_t min_filter,
@@ -314,7 +313,7 @@ int skm_basis_finalize(const uint64_t *d_count, const uint64_t *d_first, int64_t
     const size_t need = skm_basis_finalize_workspace(S);
     if (!workspace || workspace_bytes < need) { set_error("skm_basis_finalize: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t seg = align_up(size_t(S) * 8);
+    const size_t seg = align256(size_t(S) * 8);
     char *p = reinterpret_cast<char *>(workspace);
     p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(p) + 255) & ~uintptr_t(255));
     uint64_t *keys_in = (uint64_t *)p, *keys_out = (uint64_t *)(p + seg);

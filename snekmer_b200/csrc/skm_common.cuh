@@ -146,6 +146,22 @@ inline bool code_space(int nsym, int k, unsigned __int128 *out) {
     return true;
 }
 
+// host: workspace regions start on 256-byte boundaries
+inline size_t align256(size_t x) { return (x + 255) & ~size_t(255); }
+// host: smallest b in [1, 64] with 2^b >= n (the radix-sort bits that hold every value below n)
+inline int bits_for(unsigned __int128 n) { int b = 1; while (b < 64 && (((unsigned __int128)1) << b) < n) ++b; return b; }
+
+// column of `code` in a basis given as its ascending code list and the column of every entry; -1 when absent
+__device__ __forceinline__ int32_t lookup_column(const uint64_t *__restrict__ sorted_codes, const int32_t *__restrict__ col_of_sorted,
+                                                 int64_t K, uint64_t code) {
+    int64_t lo = 0, hi = K;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (__ldg(sorted_codes + mid) < code) lo = mid + 1; else hi = mid;
+    }
+    return (lo < K && __ldg(sorted_codes + lo) == code) ? __ldg(col_of_sorted + lo) : -1;
+}
+
 int check_common(const void *d_residues, int64_t nres, const void *d_offsets, int64_t nseq,
                  const void *d_lut, int nsym, int k);
 

@@ -13,9 +13,9 @@
 //   output element written once.  Algorithmic bytes per sequence:
 //   L + 8 + K*sizeof(out).
 //
-// Sparse path (skm_count_csr): window codes -> columns, segmented radix sort of
-// each sequence's keys, run-length encode into CSR.
-#include <cstdlib>
+// Sparse paths (skm_count_csr, 32-bit keys = columns; skm_count_csr_wide, 64-bit codes with an optional sorted
+// basis): window keys -> segmented radix sort of each sequence's keys -> run-length encode into CSR.  Both are the
+// cross-checks of skm_count_csr_sorted (skm_csrsort.cu).
 #include <cstring>
 
 #include <cub/cub.cuh>
@@ -144,8 +144,7 @@ __global__ void __launch_bounds__(TS_THREADS) count_dense_kernel(const uint8_t *
 // (12 per lane; the mean protein fits one segment); the finished row leaves with one bulk shared->global copy.
 // ~48 independent warps per SM hide each other's load, bulk-store and shared-atomic latencies.
 constexpr int CW_WARPS = 8;
-constexpr int CW_C = 12;                          // residues per lane and segment (4 * odd: conflict-free byte reads)
-constexpr int CW_SEG = 32 * CW_C;
+constexpr int CW_SEG = 32 * TS_WALK_C;
 constexpr int CW_SYM = ts_sym_bytes(CW_SEG);      // 480
 
 // MAP: 0 = identity basis (column = code), 1 = col_of_code staged in shared memory as uint16 columns (S <= 16384;
@@ -179,8 +178,42 @@ __device__ __forceinline__ void cw_emit_sel(uint32_t code, bool ok, uint32_t cnt
     cnt_ops<OutT>::add(cnt_addr, col);
 }
 
+// Column map (MAP 1) and this warp's zeroed counter row, before the kernel's one CTA-wide barrier.
+template <int MAP>
+__device__ __forceinline__ void cw_prologue(uint16_t *s_col, const int32_t *__restrict__ col_of_code, int S, int K,
+                                            uint4 *s_cnt4, uint32_t row_bytes, int lane) {
+    if (MAP == 1) {
+        for (int i = threadIdx.x; i < S; i += blockDim.x) {
+            const int32_t c = __ldg(col_of_code + i);
+            s_col[i] = uint16_t(c >= 0 ? c : K);                                // K = the dummy counter
+        }
+        if (threadIdx.x == 0) s_col[S] = uint16_t(K);                           // entry S: where invalid windows go
+    }
+    for (int i = lane; i < int(row_bytes >> 4); i += 32) s_cnt4[i] = make_uint4(0u, 0u, 0u, 0u);
+}
+
+// Flush the finished row to dst (one contiguous K * sizeof(OutT) range of the output) and re-zero it.
+template <typename OutT>
+__device__ __forceinline__ void cw_flush_row(OutT *dst, uint8_t *mine, uint32_t cnt_addr, int K, uint32_t row_bytes,
+                                             int bulk_ok, int lane) {
+    if (bulk_ok) {
+        ts_bulk_fence();
+        __syncwarp();
+        if (lane == 0) { ts_bulk_store(dst, cnt_addr, uint32_t(K) * uint32_t(sizeof(OutT))); ts_bulk_wait_read(); }
+        __syncwarp();
+    } else {
+        __syncwarp();
+        const OutT *s_cnt = reinterpret_cast<const OutT *>(mine);
+        for (int i = lane; i < K; i += 32) dst[i] = s_cnt[i];
+        __syncwarp();
+    }
+    uint4 *s_cnt4 = reinterpret_cast<uint4 *>(mine);
+    for (int i = lane; i < int(row_bytes >> 4); i += 32) s_cnt4[i] = make_uint4(0u, 0u, 0u, 0u);
+    __syncwarp();
+}
+
 // First version of the warp kernel (round 1): translated symbols staged as bytes, two LDS.U8 per residue, a run
-// counter.  Still the path for k - 1 > 4 (and the A/B reference: SKM_CDW_BYTES=1).
+// counter (ts_group_walk).  The path for k - 1 > 4.
 template <typename OutT, int MAP>
 __global__ void __launch_bounds__(32 * CW_WARPS, 6)
 count_dense_warp_bytes_kernel(const uint8_t *__restrict__ res, int64_t nres, const int64_t *__restrict__ off, int64_t nseq,
@@ -190,114 +223,27 @@ count_dense_warp_bytes_kernel(const uint8_t *__restrict__ res, int64_t nres, con
     extern __shared__ __align__(128) uint8_t s_raw[];
     __shared__ uint8_t s_lut[256];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    uint16_t *s_col = reinterpret_cast<uint16_t *>(s_raw);                       // [S] when MAP == 1
+    uint16_t *s_col = reinterpret_cast<uint16_t *>(s_raw);                       // [S + 1] when MAP == 1
     uint8_t *mine = s_raw + map_bytes + size_t(warp) * (row_bytes + CW_SYM);
-    uint4 *s_cnt4 = reinterpret_cast<uint4 *>(mine);
     uint8_t *s_sym = mine + row_bytes;
     uint32_t cnt_addr = smem_addr(mine), sym_addr = smem_addr(s_sym), col_addr = smem_addr(s_col);
     asm volatile("" : "+r"(cnt_addr), "+r"(sym_addr), "+r"(col_addr));      // keep the window addresses in registers
     ts_lut_init(s_lut, lut);
-    if (MAP == 1)
-        for (int i = threadIdx.x; i < S; i += blockDim.x) {
-            const int32_t c = __ldg(col_of_code + i);
-            s_col[i] = uint16_t(c >= 0 ? c : K);                                // K = the dummy counter
-        }
-    for (int i = lane; i < int(row_bytes >> 4); i += 32) s_cnt4[i] = make_uint4(0u, 0u, 0u, 0u);
+    cw_prologue<MAP>(s_col, col_of_code, S, K, reinterpret_cast<uint4 *>(mine), row_bytes, lane);
     __syncthreads();                                        // LUT and column map; the only CTA-wide barrier
     // this warp's sequences: those that start in the w-th 1/W of the residue buffer
     int64_t lo = 0, hi = 0;
-    if (lane == 0) {
-        const int64_t W = int64_t(gridDim.x) * CW_WARPS, w = int64_t(blockIdx.x) * CW_WARPS + warp;
-        const int64_t r0 = __ldg(off), span = __ldg(off + nseq) - r0;
-        lo = (w == 0) ? 0 : lower_bound_off(off, nseq, r0 + (int64_t)(((__int128)span * w) / W));
-        hi = (w + 1 == W) ? nseq : lower_bound_off(off, nseq, r0 + (int64_t)(((__int128)span * (w + 1)) / W));
-    }
+    if (lane == 0) seq_range(off, nseq, int64_t(blockIdx.x) * CW_WARPS + warp, int64_t(gridDim.x) * CW_WARPS, &lo, &hi);
     lo = __shfl_sync(FULL, lo, 0);
     hi = __shfl_sync(FULL, hi, 0);
-    const uint32_t uk = uint32_t(k);
     int64_t e = (lo < hi) ? __ldg(off + lo) : 0;
     for (int64_t s = lo; s < hi; ++s) {
         const int64_t b = e;
         e = __ldg(off + s + 1);
-        bool first = true;
-        uint32_t tail0 = 0, tail1 = 0;                      // the last k-1 symbols of the previous segment (k-1 <= 63)
-        for (int64_t a = b; a < e;) {
-            const int64_t a2 = min(e, (a + CW_SEG) & ~int64_t(15));
-            if (!first) {
-                if (lane < k - 1) s_sym[TS_PAD - (k - 1) + lane] = uint8_t(tail0);
-                if (lane + 32 < k - 1) s_sym[TS_PAD - (k - 1) + lane + 32] = uint8_t(tail1);
-            }
-            // stage: [a & ~15, a2) translated into s_sym[TS_PAD ...), one 16-byte vector per lane (at most 25)
-            const int64_t base = a & ~int64_t(15);
-            const int lo_i = TS_PAD + int(a - base), hi_i = lo_i + int(a2 - a);
-            const int nvec = int((a2 - base + 15) >> 4);
-            if (lane < nvec) {
-                const int64_t p = base + 16 * int64_t(lane);
-                uint4 x;
-                if (p + 16 <= nres) {
-                    x = __ldg(reinterpret_cast<const uint4 *>(res + p));
-                } else {
-                    uint32_t w4[4] = {0, 0, 0, 0};
-                    for (int j = 0; j < 16; ++j)
-                        if (p + j < nres) w4[j >> 2] |= uint32_t(res[p + j]) << (8 * (j & 3));
-                    x = make_uint4(w4[0], w4[1], w4[2], w4[3]);
-                }
-                x.x = ts_translate4(x.x, s_lut);
-                x.y = ts_translate4(x.y, s_lut);
-                x.z = ts_translate4(x.z, s_lut);
-                x.w = ts_translate4(x.w, s_lut);
-                reinterpret_cast<uint4 *>(s_sym + TS_PAD)[lane] = x;
-            }
-            __syncwarp();
-            if (first) {                                    // nothing in front of the sequence start is a residue of it
-                for (int i = lane; i < lo_i; i += 32) s_sym[i] = uint8_t(SYM_BAD);
-                __syncwarp();
-            }
-            // scan: lane owns symbols [i0, i1), warms up on the k-1 symbols in front of them
-            const int n = hi_i - lo_i;
-            const int C = ((((n + 31) >> 5) + 3) >> 2 | 1) << 2;     // smallest 4 * odd >= ceil(n / 32)
-            const int i0 = lo_i + lane * C, i1 = min(i0 + C, hi_i);
-            if (i0 < i1) {
-                uint32_t run = 0, code = 0;
-                uint32_t p = sym_addr + uint32_t(i0) - (uk - 1u);
-                for (uint32_t j = 1; j < uk; ++j, ++p) {
-                    const uint32_t sy = lds_u8<0>(p);
-                    run = (sy >= SYM_BAD) ? 0u : run + 1u;
-                    code = code * nsym + sy;
-                }
-                const uint32_t pend = sym_addr + uint32_t(i1);
-                const uint32_t back = uk - 1u;
-#pragma unroll 4
-                for (; p < pend; ++p) {
-                    const uint32_t sy = lds_u8<0>(p);
-                    run = (sy >= SYM_BAD) ? 0u : run + 1u;
-                    code = code * nsym + sy;
-                    if (run >= uk) cw_emit<OutT, MAP>(code, cnt_addr, col_addr, col_of_code, K);
-                    code -= lds_u8<0>(p - back) * pow_k1;
-                }
-            }
-            __syncwarp();
-            if (lane < k - 1) tail0 = s_sym[hi_i - (k - 1) + lane];
-            if (lane + 32 < k - 1) tail1 = s_sym[hi_i - (k - 1) + lane + 32];
-            __syncwarp();
-            first = false;
-            a = a2;
-        }
-        // ---- flush: the row is one contiguous K * sizeof(OutT) range of the output ----
-        OutT *dst = out + s * K;
-        if (bulk_ok) {
-            ts_bulk_fence();
-            __syncwarp();
-            if (lane == 0) { ts_bulk_store(dst, cnt_addr, uint32_t(K) * uint32_t(sizeof(OutT))); ts_bulk_wait_read(); }
-            __syncwarp();
-        } else {
-            __syncwarp();
-            const OutT *s_cnt = reinterpret_cast<const OutT *>(mine);
-            for (int i = lane; i < K; i += 32) dst[i] = s_cnt[i];
-            __syncwarp();
-        }
-        for (int i = lane; i < int(row_bytes >> 4); i += 32) s_cnt4[i] = make_uint4(0u, 0u, 0u, 0u);
-        __syncwarp();
+        ts_group_walk<32, 4, uint32_t>(res, nres, b, e, s_lut, s_sym, sym_addr, k, nsym, pow_k1, lane, [&](int64_t, uint32_t code, bool ok) {
+            if (ok) cw_emit<OutT, MAP>(code, cnt_addr, col_addr, col_of_code, K);
+        });
+        cw_flush_row(out + s * K, mine, cnt_addr, K, row_bytes, bulk_ok, lane);
     }
 }
 
@@ -327,30 +273,18 @@ count_dense_warp_kernel(const uint8_t *__restrict__ res, int64_t nres, const int
     extern __shared__ __align__(128) uint8_t s_raw[];
     __shared__ __align__(16) uint8_t s_lut[256];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    uint16_t *s_col = reinterpret_cast<uint16_t *>(s_raw);                       // [S] when MAP == 1
+    uint16_t *s_col = reinterpret_cast<uint16_t *>(s_raw);                       // [S + 1] when MAP == 1
     uint8_t *mine = s_raw + map_bytes + size_t(warp) * (row_bytes + CW_SYM);
-    uint4 *s_cnt4 = reinterpret_cast<uint4 *>(mine);
     uint8_t *s_res = mine + row_bytes;                                           // raw residue bytes of the segment
     uint32_t cnt_addr = smem_addr(mine), raw_addr = smem_addr(s_res), col_addr = smem_addr(s_col), lut_addr = smem_addr(s_lut);
     asm volatile("" : "+r"(cnt_addr), "+r"(raw_addr), "+r"(col_addr), "+r"(lut_addr));
     ts_lut_init(s_lut, lut);                                                     // invalid bytes -> SYM_BAD (0x40)
     if (threadIdx.x == 0) s_lut[0] = uint8_t(SYM_BAD);                           // byte 0 pads the staged segment: never a symbol
-    if (MAP == 1)
-        for (int i = threadIdx.x; i < S; i += blockDim.x) {
-            const int32_t c = __ldg(col_of_code + i);
-            s_col[i] = uint16_t(c >= 0 ? c : K);                                // K = the dummy counter
-        }
-    if (MAP == 1 && threadIdx.x == 0) s_col[S] = uint16_t(K);                   // entry S: where invalid windows go
-    for (int i = lane; i < int(row_bytes >> 4); i += 32) s_cnt4[i] = make_uint4(0u, 0u, 0u, 0u);
+    cw_prologue<MAP>(s_col, col_of_code, S, K, reinterpret_cast<uint4 *>(mine), row_bytes, lane);
     __syncthreads();                                        // LUT and column map; the only CTA-wide barrier
     // this warp's sequences: those that start in the w-th 1/W of the residue buffer
     int64_t lo = 0, hi = 0;
-    if (lane == 0) {
-        const int64_t W = int64_t(gridDim.x) * CW_WARPS, w = int64_t(blockIdx.x) * CW_WARPS + warp;
-        const int64_t r0 = __ldg(off), span = __ldg(off + nseq) - r0;
-        lo = (w == 0) ? 0 : lower_bound_off(off, nseq, r0 + (int64_t)(((__int128)span * w) / W));
-        hi = (w + 1 == W) ? nseq : lower_bound_off(off, nseq, r0 + (int64_t)(((__int128)span * (w + 1)) / W));
-    }
+    if (lane == 0) seq_range(off, nseq, int64_t(blockIdx.x) * CW_WARPS + warp, int64_t(gridDim.x) * CW_WARPS, &lo, &hi);
     lo = __shfl_sync(FULL, lo, 0);
     hi = __shfl_sync(FULL, hi, 0);
     if (lo >= hi) return;
@@ -447,59 +381,103 @@ count_dense_warp_kernel(const uint8_t *__restrict__ res, int64_t nres, const int
                 first = false;
                 a = a2;
             }
-            // ---- flush: the row is one contiguous K * sizeof(OutT) range of the output ----
-            OutT *dst = out + (s0 + i) * K;
-            if (bulk_ok) {
-                ts_bulk_fence();
-                __syncwarp();
-                if (lane == 0) { ts_bulk_store(dst, cnt_addr, uint32_t(K) * uint32_t(sizeof(OutT))); ts_bulk_wait_read(); }
-                __syncwarp();
-            } else {
-                __syncwarp();
-                const OutT *s_cnt = reinterpret_cast<const OutT *>(mine);
-                for (int j = lane; j < K; j += 32) dst[j] = s_cnt[j];
-                __syncwarp();
-            }
-            for (int j = lane; j < int(row_bytes >> 4); j += 32) s_cnt4[j] = make_uint4(0u, 0u, 0u, 0u);
-            __syncwarp();
+            cw_flush_row(out + (s0 + i) * K, mine, cnt_addr, K, row_bytes, bulk_ok, lane);
         }
     }
 }
 
+// Everything a dense count launch passes to its kernel besides the launch shape.
+struct DenseArgs {
+    const uint8_t *res;
+    int64_t nres;
+    const int64_t *off;
+    int64_t nseq;
+    const uint8_t *lut;
+    uint32_t nsym;
+    int k;
+    uint32_t pow_k1;
+    const int32_t *col_of_code;
+    int S, K;
+    void *out;
+    cudaStream_t st;
+};
+
+constexpr int CD_THREADS = 128;   // threads of the tile kernel
+
+template <typename OutT>
+static int launch_dense_tile(const DenseArgs &a, int grid, size_t smem, int T, int seg_cap) {
+    const auto kern = a.col_of_code ? count_dense_kernel<OutT, true> : count_dense_kernel<OutT, false>;
+    SKM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<grid, CD_THREADS, smem, a.st>>>(a.res, a.nres, a.off, a.nseq, a.lut, a.nsym, a.k, a.pow_k1, a.col_of_code, a.K, T,
+                                           seg_cap, static_cast<OutT *>(a.out));
+    SKM_LAUNCH_CHECK("count_dense_kernel");
+    return SKM_OK;
+}
+
+// words: the round-2 kernel (k - 1 <= 4), else the byte-wise one; map_mode selects MAP
+template <typename OutT>
+static int launch_dense_warp(const DenseArgs &a, bool words, int map_mode, int grid, size_t smem, uint32_t row_bytes,
+                             uint32_t map_bytes, int bulk_ok) {
+    using Kern = decltype(&count_dense_warp_kernel<OutT, 0>);
+    const Kern kerns[2][3] = {{count_dense_warp_bytes_kernel<OutT, 0>, count_dense_warp_bytes_kernel<OutT, 1>, count_dense_warp_bytes_kernel<OutT, 2>},
+                              {count_dense_warp_kernel<OutT, 0>, count_dense_warp_kernel<OutT, 1>, count_dense_warp_kernel<OutT, 2>}};
+    const Kern kern = kerns[words][map_mode];
+    SKM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<grid, 32 * CW_WARPS, smem, a.st>>>(a.res, a.nres, a.off, a.nseq, a.lut, a.nsym, a.k, a.pow_k1, a.col_of_code, a.S,
+                                              a.K, row_bytes, map_bytes, bulk_ok, static_cast<OutT *>(a.out));
+    SKM_LAUNCH_CHECK(words ? "count_dense_warp_kernel" : "count_dense_warp_bytes_kernel");
+    return SKM_OK;
+}
+
 // ---------------------------------------------------------------------------
-// sparse (CSR)
+// sparse (CSR): the two segmented-sort paths, 32-bit and 64-bit keys
 // ---------------------------------------------------------------------------
-// one warp per sequence over its sorted keys: count (and optionally write) the runs
-__global__ void __launch_bounds__(256) csr_runs_kernel(const uint32_t *__restrict__ keys, const int64_t *__restrict__ off,
-                                                       int64_t seq0, int64_t nseq, int64_t res0,
-                                                       int64_t *__restrict__ rowptr, uint32_t *__restrict__ cols,
-                                                       int32_t *__restrict__ vals) {
+// One warp per sequence over its sorted keys: count the runs (fill = false: rowptr[s + 1] = runs of row s) or write them
+// at rowptr[s] (fill = true).  32-bit keys (already columns) always go to keys_out.  64-bit keys: with a sorted basis,
+// runs whose code it does not hold are dropped and the column of every run goes to cols_out; keys_out and cols_out
+// may each be NULL.
+template <typename KeyT>
+__global__ void __launch_bounds__(256) csr_runs_kernel(const KeyT *__restrict__ keys, const int64_t *__restrict__ off,
+                                                       int64_t nseq, const uint64_t *__restrict__ sorted_codes,
+                                                       const int32_t *__restrict__ col_of_sorted, int64_t K, bool fill,
+                                                       int64_t *__restrict__ rowptr, KeyT *__restrict__ keys_out,
+                                                       uint32_t *__restrict__ cols_out, int32_t *__restrict__ vals) {
+    constexpr KeyT NONE = code_traits<KeyT>::none;
+    constexpr bool WIDE = sizeof(KeyT) == 8;       // 32-bit keys: no basis, the keys are the output
     const int lane = threadIdx.x & 31;
     const int64_t warp = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
     const int64_t nwarps = (int64_t(gridDim.x) * blockDim.x) >> 5;
-    for (int64_t s = seq0 + warp; s < seq0 + nseq; s += nwarps) {
-        const int64_t b = __ldg(off + s) - res0, e = __ldg(off + s + 1) - res0;
+    for (int64_t s = warp; s < nseq; s += nwarps) {
+        const int64_t b = __ldg(off + s), e = __ldg(off + s + 1);
         int64_t nrun = 0;
-        const int64_t wbase = cols ? rowptr[s] : 0;
+        const int64_t wbase = fill ? rowptr[s] : 0;
         for (int64_t p0 = b; p0 < e; p0 += 32) {
             const int64_t p = p0 + lane;
-            const uint32_t key = (p < e) ? keys[p] : 0xFFFFFFFFu;
-            const uint32_t prevk = (p > b && p < e) ? keys[p - 1] : 0xFFFFFFFFu;
-            const bool head = (p < e) && key != 0xFFFFFFFFu && (p == b || key != prevk);
+            const KeyT key = (p < e) ? keys[p] : NONE;
+            const KeyT prevk = (p > b && p < e) ? keys[p - 1] : NONE;
+            bool head = (p < e) && key != NONE && (p == b || key != prevk);
+            int32_t col = -1;
+            if (WIDE && head && sorted_codes) { col = lookup_column(sorted_codes, col_of_sorted, K, key); head = col >= 0; }
             const unsigned m = __ballot_sync(FULL, head);
-            if (cols && head) {
-                // run length: scan forward (runs are short: a k-mer repeated within one protein)
+            if (fill && head) {
                 int64_t q = p + 1;
-                while (q < e && keys[q] == key) ++q;
+                while (q < e && keys[q] == key) ++q;       // runs are short: a k-mer repeated within one protein
                 const int64_t slot = wbase + nrun + __popc(m & ((1u << lane) - 1u));
-                cols[slot] = key;
+                if (!WIDE || keys_out) keys_out[slot] = key;
+                if (WIDE && cols_out) cols_out[slot] = uint32_t(col);
                 vals[slot] = int32_t(q - p);
             }
             nrun += __popc(m);
         }
-        if (!cols && lane == 0) rowptr[s + 1] = nrun;
+        if (!fill && lane == 0) rowptr[s + 1] = nrun;
     }
 }
+
+// skm_wide.cu: argument checks of the 64-bit paths and the 64-bit key of every window
+int wide_check(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq, const uint8_t *d_lut,
+               int nsym, int k, const char *who, unsigned __int128 *S);
+int launch_window_codes64(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq, const uint8_t *d_lut,
+                          int nsym, int k, uint64_t *d_keys, cudaStream_t st);
 
 }  // namespace skm
 
@@ -535,97 +513,69 @@ int skm_count_dense(const uint8_t *d_residues, int64_t nres, const int64_t *d_of
         set_error("skm_count_dense: K=%lld rows do not fit shared memory; use skm_count_csr", (long long)K);
         return SKM_ERR_UNSUPPORTED;
     }
-    cudaStream_t st = (cudaStream_t)stream;
     uint32_t pow_k1 = 1;
     for (int i = 0; i + 1 < k; ++i) pow_k1 *= (uint32_t)nsym;
+    const DenseArgs args{d_residues, nres, d_offsets, nseq, d_lut, (uint32_t)nsym, k, pow_k1, d_col_of_code, (int)S, (int)K,
+                         d_counts, (cudaStream_t)stream};
     // Rows up to ~9 KB: one warp per sequence with a private counter row (>= 24 warps per SM).  One extra (dummy)
     // counter behind the row absorbs the windows whose code is filtered out of the basis.
     const uint32_t row_bytes = uint32_t((size_t(K + 1) * out_bytes + 15) & ~size_t(15));
-    const char *force_tile = getenv("SKM_CD_TILE");
-    if (row_bytes + CW_SYM <= 9 * 1024 + 256 && K < 65535 && !(force_tile && atoi(force_tile))) {
+    if (row_bytes + CW_SYM <= 9 * 1024 + 256 && K < 65535) {
         const int map_mode = !d_col_of_code ? 0 : (S <= 16384 ? 1 : 2);
         const uint32_t map_bytes = map_mode == 1 ? uint32_t((size_t(S + 1) * 2 + 127) & ~size_t(127)) : 0u;     // + the entry for invalid windows
-        const char *force_bytes = getenv("SKM_CDW_BYTES");                      // A/B switch: the byte-wise scan of round 1
-        const bool words = k - 1 <= 4 && !(force_bytes && atoi(force_bytes));
+        const bool words = k - 1 <= 4;
         const size_t smem_w = map_bytes + size_t(CW_WARPS) * (row_bytes + CW_SYM);
         int per_sm_w = int((227 * 1024) / (smem_w + 1024 + 256));
         if (per_sm_w > 6) per_sm_w = 6;
         if (per_sm_w < 1) per_sm_w = 1;
         const int grid_w = (int)std::min<int64_t>((nseq + CW_WARPS - 1) / CW_WARPS, int64_t(sm_count()) * per_sm_w);
         const int bulk_ok = ((size_t(K) * out_bytes) % 16 == 0) ? 1 : 0;
-#define SKM_LAUNCH_DENSE_W(OUT, MAP)                                                                                 \
-    {                                                                                                                \
-        if (!words) {                                                                                                \
-            auto kern = count_dense_warp_bytes_kernel<OUT, MAP>;                                                     \
-            SKM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_w));      \
-            kern<<<grid_w, 32 * CW_WARPS, smem_w, st>>>(d_residues, nres, d_offsets, nseq, d_lut, (uint32_t)nsym, k, pow_k1, \
-                                                        d_col_of_code, (int)S, (int)K, row_bytes, map_bytes, bulk_ok, (OUT *)d_counts); \
-        } else {                                                                                                     \
-            auto kern = count_dense_warp_kernel<OUT, MAP>;                                                           \
-            SKM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_w));      \
-            kern<<<grid_w, 32 * CW_WARPS, smem_w, st>>>(d_residues, nres, d_offsets, nseq, d_lut, (uint32_t)nsym, k, pow_k1, \
-                                                        d_col_of_code, (int)S, (int)K, row_bytes, map_bytes, bulk_ok, (OUT *)d_counts); \
-        }                                                                                                            \
-    }
-#define SKM_LAUNCH_DENSE_WM(OUT)                                                                                     \
-    { if (map_mode == 0) SKM_LAUNCH_DENSE_W(OUT, 0) else if (map_mode == 1) SKM_LAUNCH_DENSE_W(OUT, 1) else SKM_LAUNCH_DENSE_W(OUT, 2) }
-        if (out_bits == 32) SKM_LAUNCH_DENSE_WM(int32_t) else SKM_LAUNCH_DENSE_WM(uint16_t)
-#undef SKM_LAUNCH_DENSE_WM
-#undef SKM_LAUNCH_DENSE_W
-        SKM_LAUNCH_CHECK("count_dense_warp_kernel");
-        return SKM_OK;
+        return out_bits == 32 ? launch_dense_warp<int32_t>(args, words, map_mode, grid_w, smem_w, row_bytes, map_bytes, bulk_ok)
+                              : launch_dense_warp<uint16_t>(args, words, map_mode, grid_w, smem_w, row_bytes, map_bytes, bulk_ok);
     }
     // Tile shape.  Many small CTAs per SM (each with its own tile in flight) hide the staging-load, barrier
     // and bulk-store latencies of one another: 128 threads, ~16 KB of counters, rows a multiple of
     // 4 (int32) / 8 (uint16) so that every tile start is 16-byte aligned and leaves as one bulk copy.
     int64_t align_rows = 16 / (int64_t)out_bytes;           // rows per 16 bytes of output in the worst case ...
     while (align_rows > 1 && (size_t(align_rows / 2) * K * out_bytes) % 16 == 0) align_rows /= 2;   // ... fewer when K allows
-    int threads = 128;
     int64_t T = int64_t((16 * 1024) / (size_t(K) * out_bytes));
-    if (const char *e = getenv("SKM_CD_THREADS")) { const int v = atoi(e); if (v >= 32 && v <= 256 && v % 32 == 0) threads = v; }
-    if (const char *e = getenv("SKM_CD_ROWS")) { const int v = atoi(e); if (v > 0) T = v; }
     if (T >= align_rows) T -= T % align_rows;
     if (T < align_rows) T = (size_t(align_rows) * K * out_bytes <= 64 * 1024) ? align_rows : 1;
     if (T > CD_MAX_ROWS) T = CD_MAX_ROWS;
-    const int seg_cap = ts_seg_cap(28, threads);
+    const int seg_cap = ts_seg_cap(28, CD_THREADS);
     const size_t sym_bytes = (size_t)ts_sym_bytes(seg_cap);
     const size_t sm_bytes = 227 * 1024, per_cta_reserved = 1024 + 512;
     const size_t smem = ((size_t(T) * K * out_bytes + 15) & ~size_t(15)) + sym_bytes;
     const int64_t ntiles = (nseq + T - 1) / T;
     int per_sm = int(sm_bytes / (smem + per_cta_reserved));
-    if (per_sm > 2048 / threads) per_sm = 2048 / threads;
+    if (per_sm > 2048 / CD_THREADS) per_sm = 2048 / CD_THREADS;
     if (per_sm > 32) per_sm = 32;
     if (per_sm < 1) per_sm = 1;
     const int grid = (int)std::min<int64_t>(ntiles, int64_t(sm_count()) * per_sm);
-#define SKM_LAUNCH_DENSE(OUT, MAP)                                                                                   \
-    {                                                                                                                \
-        auto kern = count_dense_kernel<OUT, MAP>;                                                                    \
-        SKM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
-        kern<<<grid, threads, smem, st>>>(d_residues, nres, d_offsets, nseq, d_lut, (uint32_t)nsym, k, pow_k1,       \
-                                             d_col_of_code, (int)K, (int)T, seg_cap, (OUT *)d_counts);               \
-    }
-    if (out_bits == 32) { if (d_col_of_code) SKM_LAUNCH_DENSE(int32_t, true) else SKM_LAUNCH_DENSE(int32_t, false) }
-    else { if (d_col_of_code) SKM_LAUNCH_DENSE(uint16_t, true) else SKM_LAUNCH_DENSE(uint16_t, false) }
-#undef SKM_LAUNCH_DENSE
-    SKM_LAUNCH_CHECK("count_dense_kernel");
-    return SKM_OK;
+    return out_bits == 32 ? launch_dense_tile<int32_t>(args, grid, smem, (int)T, seg_cap)
+                          : launch_dense_tile<uint16_t>(args, grid, smem, (int)T, seg_cap);
 }
 
 // cub::DeviceSegmentedSort takes 32-bit item counts: one call handles < 2^30 residues (callers shard above that).
 static const int64_t CSR_MAX_RES = (1ll << 30);
 
-static size_t csr_align(size_t x) { return (x + 255) & ~size_t(255); }
-
-size_t skm_count_csr_workspace(int64_t nres, int64_t nseq) {
+// workspace of one segmented sort of key_bytes-wide keys: two key buffers and the larger of the sort's and the scan's temp
+static size_t csr_segsort_workspace(int64_t nres, int64_t nseq, size_t key_bytes) {
+    using namespace skm;
     if (nres <= 0 || nseq <= 0) return 256;
-    const int64_t items = std::min<int64_t>(nres, CSR_MAX_RES);
+    const int items = (int)std::min<int64_t>(nres, CSR_MAX_RES), segs = (int)std::min<int64_t>(nseq, (1ll << 31) - 1);
     size_t t_sort = 0, t_scan = 0;
-    cub::DeviceSegmentedSort::SortKeys(nullptr, t_sort, (const uint32_t *)nullptr, (uint32_t *)nullptr, (int)items,
-                                       (int)std::min<int64_t>(nseq, (1ll << 31) - 1), (const int64_t *)nullptr,
-                                       (const int64_t *)nullptr);
+    if (key_bytes == 8)
+        cub::DeviceSegmentedSort::SortKeys(nullptr, t_sort, (const uint64_t *)nullptr, (uint64_t *)nullptr, items, segs,
+                                           (const int64_t *)nullptr, (const int64_t *)nullptr);
+    else
+        cub::DeviceSegmentedSort::SortKeys(nullptr, t_sort, (const uint32_t *)nullptr, (uint32_t *)nullptr, items, segs,
+                                           (const int64_t *)nullptr, (const int64_t *)nullptr);
     cub::DeviceScan::InclusiveSum(nullptr, t_scan, (const int64_t *)nullptr, (int64_t *)nullptr, nseq);
-    return 2 * csr_align((size_t)nres * 4) + csr_align(std::max(t_sort, t_scan)) + 1024;
+    return 2 * align256((size_t)nres * key_bytes) + align256(std::max(t_sort, t_scan)) + 1024;
 }
+
+size_t skm_count_csr_workspace(int64_t nres, int64_t nseq) { return csr_segsort_workspace(nres, nseq, 4); }
 
 int skm_count_csr(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq,
                   const uint8_t *d_lut, int nsym, int k, const int32_t *d_col_of_code, int64_t S,
@@ -646,7 +596,7 @@ int skm_count_csr(const uint8_t *d_residues, int64_t nres, const int64_t *d_offs
     if (nres >= CSR_MAX_RES || nseq >= (1ll << 31)) { set_error("skm_count_csr: more than 2^30 residues per call; split the shard"); return SKM_ERR_UNSUPPORTED; }
     const size_t need = skm_count_csr_workspace(nres, nseq);
     if (!workspace || workspace_bytes < need) { set_error("skm_count_csr: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
-    const size_t seg = csr_align((size_t)nres * 4);
+    const size_t seg = align256((size_t)nres * 4);
     char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
     uint32_t *keys_a = (uint32_t *)p, *keys_b = (uint32_t *)(p + seg);
     void *temp = p + 2 * seg;
@@ -659,11 +609,52 @@ int skm_count_csr(const uint8_t *d_residues, int64_t nres, const int64_t *d_offs
     if (rc) return rc;
     SKM_CUDA_TRY(cub::DeviceSegmentedSort::SortKeys(temp, temp_bytes, keys_a, keys_b, (int)nres, (int)nseq, d_offsets,
                                                     d_offsets + 1, st));
-    csr_runs_kernel<<<grid, 256, 0, st>>>(keys_b, d_offsets, 0, nseq, 0, d_rowptr, nullptr, nullptr);
+    csr_runs_kernel<uint32_t><<<grid, 256, 0, st>>>(keys_b, d_offsets, nseq, nullptr, nullptr, 0, false, d_rowptr, nullptr, nullptr, nullptr);
     SKM_LAUNCH_CHECK("csr_runs_kernel(count)");
     temp_bytes = workspace_bytes - (size_t)((char *)temp - (char *)workspace);
     SKM_CUDA_TRY(cub::DeviceScan::InclusiveSum(temp, temp_bytes, d_rowptr + 1, d_rowptr + 1, nseq, st));
-    csr_runs_kernel<<<grid, 256, 0, st>>>(keys_b, d_offsets, 0, nseq, 0, d_rowptr, d_cols, d_vals);
+    csr_runs_kernel<uint32_t><<<grid, 256, 0, st>>>(keys_b, d_offsets, nseq, nullptr, nullptr, 0, true, d_rowptr, d_cols, nullptr, d_vals);
+    SKM_LAUNCH_CHECK("csr_runs_kernel(fill)");
+    return SKM_OK;
+}
+
+size_t skm_count_csr_wide_workspace(int64_t nres, int64_t nseq) { return csr_segsort_workspace(nres, nseq, 8); }
+
+int skm_count_csr_wide(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq,
+                       const uint8_t *d_lut, int nsym, int k, const uint64_t *d_sorted_codes,
+                       const int32_t *d_col_of_sorted, int64_t K, int64_t *d_rowptr, uint64_t *d_codes_out,
+                       uint32_t *d_cols_out, int32_t *d_vals, void *workspace, size_t workspace_bytes,
+                       skm_stream_t stream) {
+    using namespace skm;
+    unsigned __int128 S;
+    int rc = wide_check(d_residues, nres, d_offsets, nseq, d_lut, nsym, k, "skm_count_csr_wide", &S);
+    if (rc) return rc;
+    if (!d_rowptr) { set_error("skm_count_csr_wide: d_rowptr is NULL"); return SKM_ERR_INVALID; }
+    if (d_sorted_codes && (!d_col_of_sorted || K < 0)) { set_error("skm_count_csr_wide: basis given without its column map"); return SKM_ERR_INVALID; }
+    if (d_cols_out && !d_sorted_codes) { set_error("skm_count_csr_wide: d_cols_out needs a basis"); return SKM_ERR_INVALID; }
+    cudaStream_t st = (cudaStream_t)stream;
+    SKM_CUDA_TRY(cudaMemsetAsync(d_rowptr, 0, 8 * (size_t)(nseq + 1), st));
+    if (nseq == 0 || nres == 0) return SKM_OK;
+    if (!d_vals || (!d_codes_out && !d_cols_out)) { set_error("skm_count_csr_wide: NULL output"); return SKM_ERR_INVALID; }
+    const size_t need = skm_count_csr_wide_workspace(nres, nseq);
+    if (!workspace || workspace_bytes < need) { set_error("skm_count_csr_wide: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
+    char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
+    const size_t seg = align256(size_t(nres) * 8);
+    uint64_t *keys_a = (uint64_t *)p, *keys_b = (uint64_t *)(p + seg);
+    void *temp = p + 2 * seg;
+    const size_t temp_cap = workspace_bytes - (size_t)((char *)temp - (char *)workspace);
+    size_t temp_bytes = temp_cap;
+    // keys are indexed by the absolute position of the window's last residue; positions outside every sequence are
+    // never read by the segmented sort
+    rc = launch_window_codes64(d_residues, nres, d_offsets, nseq, d_lut, nsym, k, keys_a, st);
+    if (rc) return rc;
+    SKM_CUDA_TRY(cub::DeviceSegmentedSort::SortKeys(temp, temp_bytes, keys_a, keys_b, (int)nres, (int)nseq, d_offsets, d_offsets + 1, st));
+    const int grid = sm_count() * 8;
+    csr_runs_kernel<uint64_t><<<grid, 256, 0, st>>>(keys_b, d_offsets, nseq, d_sorted_codes, d_col_of_sorted, K, false, d_rowptr, nullptr, nullptr, nullptr);
+    SKM_LAUNCH_CHECK("csr_runs_kernel(count)");
+    temp_bytes = temp_cap;
+    SKM_CUDA_TRY(cub::DeviceScan::InclusiveSum(temp, temp_bytes, d_rowptr + 1, d_rowptr + 1, nseq, st));
+    csr_runs_kernel<uint64_t><<<grid, 256, 0, st>>>(keys_b, d_offsets, nseq, d_sorted_codes, d_col_of_sorted, K, true, d_rowptr, d_codes_out, d_cols_out, d_vals);
     SKM_LAUNCH_CHECK("csr_runs_kernel(fill)");
     return SKM_OK;
 }

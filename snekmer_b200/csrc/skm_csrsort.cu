@@ -4,8 +4,8 @@
 // sequences: proteins (mean 350 residues) fall into CUB's "large segment" kernel, one 256-thread CTA per protein,
 // and the step ran at 4 G keys/s — 15 ms per 200 k proteins, 1 % of the HBM roofline.  Here a WARP owns a sequence
 // from the residue bytes to its finished CSR row:
-//   scan     residues -> LUT -> symbols in the warp's shared buffer -> rolling codes (the count_dense_warp_kernel
-//            scanner); the key of every window (code, or basis column) goes to the warp's key buffer in shared memory;
+//   scan     residues -> LUT -> symbols in the warp's shared buffer -> rolling codes (ts_group_walk, the scanner of
+//            count_dense_warp_bytes_kernel); the key of every window (code, or basis column) goes to the warp's key buffer in shared memory;
 //   sort     bitonic network, all compare-exchanges ascending (flip formulation), so n need not be a power of two:
 //            partners at or beyond n act as +infinity.  32-bit keys of sequences up to 512 windows are sorted in
 //            REGISTERS (16 keys per lane, shuffles for the cross-lane steps: 75 instructions per key instead of ~250),
@@ -26,7 +26,6 @@
 
 namespace skm {
 
-constexpr int CS_C = 12;                       // residues per thread and segment (4 * odd)
 constexpr int CS_WARPS = 8;                    // warps (= sequences in flight) per CTA of the warp kernel
 constexpr int CS_KCAP_W = 1024;                // keys per warp buffer
 constexpr int CS_REG_KEYS = 512;               // sequences up to this many windows are sorted in registers (16 keys per lane)
@@ -36,8 +35,6 @@ constexpr int CS_LONG_THREADS = 256;
 template <typename T> struct key_none;
 template <> struct key_none<uint32_t> { static constexpr uint32_t v = 0xFFFFFFFFu; };
 template <> struct key_none<uint64_t> { static constexpr uint64_t v = ~0ull; };
-
-template <int GT> __device__ __forceinline__ void gsync() { if (GT == 32) __syncwarp(); else __syncthreads(); }
 
 // basis lookup: sorted code list + column of each entry; `bucket` (nullable) = start index of every 2^shift-wide
 // code range, so the binary search runs over a handful of entries
@@ -246,8 +243,7 @@ csr_sort_kernel(const uint8_t *__restrict__ res, int64_t nres, const int64_t *__
                 int kcap, int64_t *long_list, unsigned long long *n_long, KeyT *gscratch, int64_t gscratch_stride,
                 KeyT *__restrict__ tmp_keys, int32_t *__restrict__ tmp_vals, int64_t *__restrict__ rowcount) {
     constexpr int GT = LONG ? CS_LONG_THREADS : 32;
-    constexpr int SEG = GT * CS_C;
-    constexpr int SYM_BYTES = ts_sym_bytes(SEG);
+    constexpr int SYM_BYTES = ts_sym_bytes(GT * TS_WALK_C);
     constexpr KeyT NONE = key_none<KeyT>::v;
     extern __shared__ __align__(128) uint8_t s_raw[];
     __shared__ uint8_t s_lut[256];
@@ -266,19 +262,13 @@ csr_sort_kernel(const uint8_t *__restrict__ res, int64_t nres, const int64_t *__
     // ---- which sequences ----
     int64_t lo = 0, hi = 0;
     if (!LONG) {
-        if (lane == 0) {
-            const int64_t W = int64_t(gridDim.x) * CS_WARPS, w = int64_t(blockIdx.x) * CS_WARPS + grp;
-            const int64_t r0 = __ldg(off), span = __ldg(off + nseq) - r0;
-            lo = (w == 0) ? 0 : lower_bound_off(off, nseq, r0 + (int64_t)(((__int128)span * w) / W));
-            hi = (w + 1 == W) ? nseq : lower_bound_off(off, nseq, r0 + (int64_t)(((__int128)span * (w + 1)) / W));
-        }
+        if (lane == 0) seq_range(off, nseq, int64_t(blockIdx.x) * CS_WARPS + grp, int64_t(gridDim.x) * CS_WARPS, &lo, &hi);
         lo = __shfl_sync(FULL, lo, 0);
         hi = __shfl_sync(FULL, hi, 0);
     } else {
         lo = blockIdx.x;
         hi = int64_t(*n_long);
     }
-    const uint32_t uk = uint32_t(k);
     for (int64_t it = lo; it < hi; it += (LONG ? int64_t(gridDim.x) : 1)) {
         const int64_t s = LONG ? long_list[it] : it;
         const int64_t b = __ldg(off + s), e = __ldg(off + s + 1);
@@ -293,79 +283,17 @@ csr_sort_kernel(const uint8_t *__restrict__ res, int64_t nres, const int64_t *__
         // 32-bit keys of sequences up to 512 windows are sorted in registers (padded buffer layout); 64-bit keys stay on
         // the shared-memory network (twice the shuffles and 80 registers made the register version slower: 4.9 vs 3.8 ms)
         const bool in_regs = !LONG && sizeof(KeyT) == 4 && n <= CS_REG_KEYS;
-        // ---- scan: key of the window ending at residue b + (k-1) + i goes to keys[i] ----
-        bool first = true;
-        uint32_t tail0 = 0, tail1 = 0;
-        for (int64_t a = b; a < e;) {
-            const int64_t a2 = min(e, (a + SEG) & ~int64_t(15));
-            if (!first) {
-                if (g < k - 1) s_sym[TS_PAD - (k - 1) + g] = uint8_t(tail0);
-                if (g + 32 < k - 1) s_sym[TS_PAD - (k - 1) + g + 32] = uint8_t(tail1);
-            }
-            const int64_t base = a & ~int64_t(15);
-            const int lo_i = TS_PAD + int(a - base), hi_i = lo_i + int(a2 - a);
-            const int nvec = int((a2 - base + 15) >> 4);
-            if (g < nvec) {
-                const int64_t p = base + 16 * int64_t(g);
-                uint4 x;
-                if (p + 16 <= nres) {
-                    x = __ldg(reinterpret_cast<const uint4 *>(res + p));
-                } else {
-                    uint32_t w4[4] = {0, 0, 0, 0};
-                    for (int j = 0; j < 16; ++j)
-                        if (p + j < nres) w4[j >> 2] |= uint32_t(res[p + j]) << (8 * (j & 3));
-                    x = make_uint4(w4[0], w4[1], w4[2], w4[3]);
+        // ---- scan: key of window i (residues b + i .. b + i + k-1) goes to keys[i] ----
+        ts_group_walk<GT, 2, KeyT>(res, nres, b, e, s_lut, s_sym, sym_addr, k, nsym, pow_k1, g, [&](int64_t widx, KeyT code, bool ok) {
+            if (widx >= 0) {
+                KeyT key = NONE;
+                if (ok) {
+                    if (MODE == 1) { const int32_t c = __ldg(col_of_code + code); if (c >= 0) key = KeyT(c); }
+                    else key = code;
                 }
-                x.x = ts_translate4(x.x, s_lut);
-                x.y = ts_translate4(x.y, s_lut);
-                x.z = ts_translate4(x.z, s_lut);
-                x.w = ts_translate4(x.w, s_lut);
-                reinterpret_cast<uint4 *>(s_sym + TS_PAD)[g] = x;
+                keys[in_regs ? int64_t(kpad(int(widx))) : widx] = key;
             }
-            gsync<GT>();
-            if (first) {
-                for (int i = g; i < lo_i; i += GT) s_sym[i] = uint8_t(SYM_BAD);
-                gsync<GT>();
-            }
-            const int nn = hi_i - lo_i;
-            const int C = ((((nn + GT - 1) / GT) + 3) >> 2 | 1) << 2;       // smallest 4 * odd >= ceil(nn / GT)
-            const int i0 = lo_i + g * C, i1 = min(i0 + C, hi_i);
-            if (i0 < i1) {
-                uint32_t run = 0;
-                KeyT code = 0;
-                uint32_t p = sym_addr + uint32_t(i0) - (uk - 1u);
-                for (uint32_t j = 1; j < uk; ++j, ++p) {
-                    const uint32_t sy = lds_u8<0>(p);
-                    run = (sy >= SYM_BAD) ? 0u : run + 1u;
-                    code = code * nsym + KeyT(sy);
-                }
-                const uint32_t pend = sym_addr + uint32_t(i1);
-                const uint32_t back = uk - 1u;
-                // index of the window ending at symbol p: (a - b) + (p - sym_addr - lo_i) - (k - 1)
-                int64_t widx = (a - b) + int64_t(i0 - lo_i) - int64_t(k - 1);
-#pragma unroll 2
-                for (; p < pend; ++p, ++widx) {
-                    const uint32_t sy = lds_u8<0>(p);
-                    run = (sy >= SYM_BAD) ? 0u : run + 1u;
-                    code = code * nsym + KeyT(sy);
-                    if (widx >= 0) {
-                        KeyT key = NONE;
-                        if (run >= uk) {
-                            if (MODE == 1) { const int32_t c = __ldg(col_of_code + code); if (c >= 0) key = KeyT(c); }
-                            else key = code;
-                        }
-                        keys[in_regs ? int64_t(kpad(int(widx))) : widx] = key;
-                    }
-                    code -= KeyT(lds_u8<0>(p - back)) * pow_k1;
-                }
-            }
-            gsync<GT>();
-            if (g < k - 1) tail0 = s_sym[hi_i - (k - 1) + g];
-            if (g + 32 < k - 1) tail1 = s_sym[hi_i - (k - 1) + g + 32];
-            gsync<GT>();
-            first = false;
-            a = a2;
-        }
+        });
         int total = 0;
         if (sizeof(KeyT) == 4 && in_regs) {
             // ---- sort + encode in registers (one instantiation: several unrolled networks thrash the instruction cache) ----
@@ -483,11 +411,9 @@ __global__ void __launch_bounds__(256) bucket_index_kernel(const uint64_t *__res
     }
 }
 
-static size_t cal(size_t x) { return (x + 255) & ~size_t(255); }
 constexpr int64_t CS_MAX_RES = 1ll << 30;
 constexpr int CS_BUCKET_BITS = 20;
 
-static int cs_bits_for(unsigned __int128 n) { int b = 1; while (b < 64 && (((unsigned __int128)1) << b) < n) ++b; return b; }
 
 struct CsPlan {
     size_t key_bytes;
@@ -505,7 +431,7 @@ static CsPlan cs_plan(int64_t nres, int64_t nseq, int64_t max_len, size_t key_by
     size_t t_scan = 0;
     cub::DeviceScan::InclusiveSum(nullptr, t_scan, (const int64_t *)nullptr, (int64_t *)nullptr, nseq + 1);
     size_t o = 0;
-    auto take = [&](size_t bytes) { const size_t at = o; o += cal(bytes); return at; };
+    auto take = [&](size_t bytes) { const size_t at = o; o += align256(bytes); return at; };
     p.tmp_keys = take(size_t(nres) * key_bytes);
     p.tmp_cols = take(with_cols ? size_t(nres) * 4 : 0);
     p.tmp_vals = take(size_t(nres) * 4);
@@ -537,7 +463,7 @@ static int cs_run(const uint8_t *d_residues, int64_t nres, const int64_t *d_offs
     SKM_CUDA_TRY(cudaMemsetAsync(rowcount, 0, 8, st));
     // warp kernel
     {
-        constexpr int SYM_W = ts_sym_bytes(32 * CS_C);
+        constexpr int SYM_W = ts_sym_bytes(32 * TS_WALK_C);
         const size_t smem = size_t(CS_WARPS) * (size_t(CS_KCAP_W + (CS_KCAP_W >> 5)) * sizeof(KeyT) + SYM_W);
         auto kern = csr_sort_kernel<KeyT, MODE, false>;
         SKM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -551,7 +477,7 @@ static int cs_run(const uint8_t *d_residues, int64_t nres, const int64_t *d_offs
     }
     // long sequences (the list may be empty: the CTAs then exit at once)
     if (max_len - (k - 1) > CS_KCAP_W) {
-        constexpr int SYM_C = ts_sym_bytes(CS_LONG_THREADS * CS_C);
+        constexpr int SYM_C = ts_sym_bytes(CS_LONG_THREADS * TS_WALK_C);
         const size_t smem = size_t(CS_KCAP_C) * sizeof(KeyT) + SYM_C;
         auto kern = csr_sort_kernel<KeyT, MODE, true>;
         SKM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -616,7 +542,7 @@ int skm_count_csr_sorted(const uint8_t *d_residues, int64_t nres, const int64_t 
     char *ws = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
     SortedBasis sb{d_sorted_codes, d_col_of_sorted, nullptr, K, 0};
     if (with_bucket) {
-        const int bits = cs_bits_for(S128);
+        const int bits = bits_for(S128);
         sb.shift = bits > CS_BUCKET_BITS ? bits - CS_BUCKET_BITS : 0;
         const int64_t nbucket = int64_t((S128 - 1) >> sb.shift) + 1;            // <= 2^20
         uint32_t *bucket = reinterpret_cast<uint32_t *>(ws + pl.bucket);

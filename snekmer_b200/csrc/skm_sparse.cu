@@ -409,8 +409,6 @@ __global__ void __launch_bounds__(256) csc_pack_kernel(const int32_t *__restrict
         packed[i] = (uint32_t(mvals[i]) << 16) | (uint32_t(rows[i]) & 0xFFFFu);      // value high, annotation low
 }
 
-static size_t al(size_t x) { return (x + 255) & ~size_t(255); }
-static int bits_for(unsigned __int128 n) { int b = 1; while (b < 64 && (((unsigned __int128)1) << b) < n) ++b; return b; }
 
 }  // namespace skm
 
@@ -439,7 +437,7 @@ size_t skm_learn_sparse_workspace(int64_t nres) {
     cub::DeviceRadixSort::SortKeys(nullptr, t_sort, (const uint64_t *)nullptr, (uint64_t *)nullptr, nres, 0, 64);
     cub::DeviceRunLengthEncode::Encode(nullptr, t_rle, (const uint64_t *)nullptr, (uint64_t *)nullptr, (int64_t *)nullptr,
                                        (int64_t *)nullptr, (int)std::min<int64_t>(nres, (1ll << 31) - 1));
-    return 2 * al(size_t(nres) * 8) + al(std::max(t_sort, t_rle)) + 1024;
+    return 2 * align256(size_t(nres) * 8) + align256(std::max(t_sort, t_rle)) + 1024;
 }
 
 int skm_learn_sparse(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq,
@@ -463,7 +461,7 @@ int skm_learn_sparse(const uint8_t *d_residues, int64_t nres, const int64_t *d_o
     const size_t need = skm_learn_sparse_workspace(nres);
     if (!workspace || workspace_bytes < need) { set_error("skm_learn_sparse: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
     char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-    const size_t seg = al(size_t(nres) * 8);
+    const size_t seg = align256(size_t(nres) * 8);
     uint64_t *keys_a = (uint64_t *)p, *keys_b = (uint64_t *)(p + seg);
     void *temp = p + 2 * seg;
     size_t temp_bytes = workspace_bytes - size_t((char *)temp - (char *)workspace);
@@ -504,7 +502,7 @@ size_t skm_learn_sparse_group_workspace(int64_t nres) {
     cub::DeviceRadixSort::SortKeys(nullptr, t_sort, (const uint32_t *)nullptr, (uint32_t *)nullptr, nres, 0, 32);
     cub::DeviceRunLengthEncode::Encode(nullptr, t_rle, (const uint32_t *)nullptr, (uint32_t *)nullptr, (int32_t *)nullptr,
                                        (int64_t *)nullptr, (int)std::min<int64_t>(nres, (1ll << 31) - 1));
-    return 4 * al(size_t(nres) * 4) + al(std::max(t_sort, t_rle)) + 1024;
+    return 4 * align256(size_t(nres) * 4) + align256(std::max(t_sort, t_rle)) + 1024;
 }
 
 namespace skm {
@@ -589,7 +587,7 @@ int skm_learn_sparse_group_place(const uint8_t *d_residues, int64_t nres, const 
     if (!workspace || workspace_bytes < need) { set_error("skm_learn_sparse_group: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
     cudaStream_t st = (cudaStream_t)stream;
     char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-    const size_t seg = al(size_t(nres) * 4);
+    const size_t seg = align256(size_t(nres) * 4);
     uint32_t *keys_a = (uint32_t *)p, *keys_b = (uint32_t *)(p + seg), *uniq = (uint32_t *)(p + 2 * seg);
     int32_t *counts = (int32_t *)(p + 3 * seg);
     void *temp = p + 4 * seg;
@@ -631,7 +629,7 @@ size_t skm_coo_merge_workspace(int64_t n) {
                                     (int64_t *)nullptr, n, 0, 64);
     cub::DeviceReduce::ReduceByKey(nullptr, t_red, (const uint64_t *)nullptr, (uint64_t *)nullptr, (const int64_t *)nullptr,
                                    (int64_t *)nullptr, (int64_t *)nullptr, cub::Sum(), n);
-    return 2 * al(size_t(n) * 8) + al(std::max(t_sort, t_red)) + 1024;
+    return 2 * align256(size_t(n) * 8) + align256(std::max(t_sort, t_red)) + 1024;
 }
 
 int skm_coo_merge(const uint64_t *d_keys_in, const int64_t *d_vals_in, int64_t n, uint64_t key_bound, uint64_t *d_keys_out,
@@ -646,7 +644,7 @@ int skm_coo_merge(const uint64_t *d_keys_in, const int64_t *d_vals_in, int64_t n
     const size_t need = skm_coo_merge_workspace(n);
     if (!workspace || workspace_bytes < need) { set_error("skm_coo_merge: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
     char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-    const size_t seg = al(size_t(n) * 8);
+    const size_t seg = align256(size_t(n) * 8);
     uint64_t *sk = (uint64_t *)p;
     int64_t *sv = (int64_t *)(p + seg);
     void *temp = p + 2 * seg;
@@ -695,7 +693,7 @@ size_t skm_coo_merge_runs_workspace(int64_t n, int n_runs) {
                                  (const int64_t *)nullptr, half, (uint64_t *)nullptr, (int64_t *)nullptr);
     cub::DeviceReduce::ReduceByKey(nullptr, t_red, (const uint64_t *)nullptr, (uint64_t *)nullptr, (const int64_t *)nullptr,
                                    (int64_t *)nullptr, (int64_t *)nullptr, cub::Sum(), n);
-    return 4 * al(size_t(n) * 8) + al(std::max(t_m, t_red)) + 1024;
+    return 4 * align256(size_t(n) * 8) + align256(std::max(t_m, t_red)) + 1024;
 }
 
 int skm_coo_merge_runs(const uint64_t *d_keys_in, const int64_t *d_vals_in, const int64_t *run_offsets_host, int n_runs,
@@ -715,7 +713,7 @@ int skm_coo_merge_runs(const uint64_t *d_keys_in, const int64_t *d_vals_in, cons
     const size_t need = skm_coo_merge_runs_workspace(n, n_runs);
     if (!workspace || workspace_bytes < need) { set_error("skm_coo_merge_runs: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
     char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-    const size_t seg = al(size_t(n) * 8);
+    const size_t seg = align256(size_t(n) * 8);
     uint64_t *kb[2] = {(uint64_t *)p, (uint64_t *)(p + seg)};
     int64_t *vb[2] = {(int64_t *)(p + 2 * seg), (int64_t *)(p + 3 * seg)};
     void *temp = p + 4 * seg;
@@ -891,7 +889,7 @@ size_t skm_coo_merge_runs_packed_workspace(int64_t n, int n_runs) {
     const size_t n_tiles = size_t((n + PR_TILE - 1) / PR_TILE);
     size_t t_scan = 0;
     cub::DeviceScan::ExclusiveSum(nullptr, t_scan, (const int64_t *)nullptr, (int64_t *)nullptr, (int64_t)n_tiles);
-    return 2 * al(size_t(n) * 8) + al(std::max(std::max(t_m, t_red), t_scan)) + 2 * al(n_tiles * 8) + 1024;
+    return 2 * align256(size_t(n) * 8) + align256(std::max(std::max(t_m, t_red), t_scan)) + 2 * align256(n_tiles * 8) + 1024;
 }
 
 int skm_coo_merge_runs_packed(const uint64_t *d_packed_in, const int64_t *run_offsets_host, int n_runs, int count_bits,
@@ -911,7 +909,7 @@ int skm_coo_merge_runs_packed(const uint64_t *d_packed_in, const int64_t *run_of
     const size_t need = skm_coo_merge_runs_packed_workspace(n, n_runs);
     if (!workspace || workspace_bytes < need) { set_error("skm_coo_merge_runs_packed: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
     char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-    const size_t seg = al(size_t(n) * 8);
+    const size_t seg = align256(size_t(n) * 8);
     uint64_t *kb[2] = {(uint64_t *)p, (uint64_t *)(p + seg)};
     void *temp = p + 2 * seg;
     const size_t temp_cap = workspace_bytes - size_t((char *)temp - (char *)workspace);
@@ -942,7 +940,7 @@ int skm_coo_merge_runs_packed(const uint64_t *d_packed_in, const int64_t *run_of
     }
     // reduce the runs of equal keys + unpack: count heads per tile, scan, emit (packed_heads_kernel / packed_emit_kernel)
     const int64_t n_tiles = (n + PR_TILE - 1) / PR_TILE;
-    const size_t tiles_seg = al(size_t(n_tiles) * 8);
+    const size_t tiles_seg = align256(size_t(n_tiles) * 8);
     char *tail = reinterpret_cast<char *>(workspace) + workspace_bytes - 2 * tiles_seg - 256;
     tail = reinterpret_cast<char *>(reinterpret_cast<uintptr_t>(tail) & ~uintptr_t(255));
     int64_t *tile_heads = reinterpret_cast<int64_t *>(tail), *tile_off = reinterpret_cast<int64_t *>(tail + tiles_seg);
@@ -957,12 +955,12 @@ int skm_coo_merge_runs_packed(const uint64_t *d_packed_in, const int64_t *run_of
 
 size_t skm_csc_build_workspace(int64_t nnz, int64_t n_ann) {
     using namespace skm;
-    if (nnz <= 0) return 256 + al(size_t(std::max<int64_t>(n_ann, 1)) * 8);
+    if (nnz <= 0) return 256 + align256(size_t(std::max<int64_t>(n_ann, 1)) * 8);
     size_t t_sort = 0, t_scan = 0;
     cub::DeviceRadixSort::SortPairs(nullptr, t_sort, (const uint64_t *)nullptr, (uint64_t *)nullptr, (const int64_t *)nullptr,
                                     (int64_t *)nullptr, nnz, 0, 64);
     cub::DeviceScan::InclusiveSum(nullptr, t_scan, (const int64_t *)nullptr, (int64_t *)nullptr, (int64_t)1 << 27);
-    return 4 * al(size_t(nnz) * 8) + al(size_t(n_ann) * 8) + al(std::max(t_sort, t_scan)) + 1024;
+    return 4 * align256(size_t(nnz) * 8) + align256(size_t(n_ann) * 8) + align256(std::max(t_sort, t_scan)) + 1024;
 }
 
 int skm_csc_build(const uint64_t *d_keys, const int64_t *d_vals, int64_t nnz, int64_t S, int64_t n_ann,
@@ -980,11 +978,11 @@ int skm_csc_build(const uint64_t *d_keys, const int64_t *d_vals, int64_t nnz, in
     const size_t need = skm_csc_build_workspace(nnz, n_ann);
     if (!workspace || workspace_bytes < need) { set_error("skm_csc_build: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
     char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-    const size_t seg = al(size_t(nnz) * 8);
+    const size_t seg = align256(size_t(nnz) * 8);
     uint64_t *k_in = (uint64_t *)p, *k_out = (uint64_t *)(p + seg);
     int64_t *perm_in = (int64_t *)(p + 2 * seg), *perm_out = (int64_t *)(p + 3 * seg);
     unsigned long long *norm2 = (unsigned long long *)(p + 4 * seg);
-    void *temp = p + 4 * seg + al(size_t(n_ann) * 8);
+    void *temp = p + 4 * seg + align256(size_t(n_ann) * 8);
     size_t temp_bytes = workspace_bytes - size_t((char *)temp - (char *)workspace);
     const int grid = (int)std::min<int64_t>((nnz + 255) / 256, int64_t(sm_count()) * 16);
     SKM_CUDA_TRY(cudaMemsetAsync(norm2, 0, size_t(n_ann) * 8, st));

@@ -186,16 +186,99 @@ __device__ __forceinline__ int64_t lower_bound_off(const int64_t *__restrict__ o
     return lo;
 }
 
-// CTA i owns the sequences whose start lies in [R*i/G, R*(i+1)/G): contiguous and residue-balanced.
-__device__ __forceinline__ void cta_seq_range(const int64_t *__restrict__ off, int64_t nseq, int64_t *lo, int64_t *hi) {
-    const int64_t r0 = __ldg(off), r1 = __ldg(off + nseq);
-    const int64_t span = r1 - r0;
-    const int64_t G = gridDim.x, i = blockIdx.x;
-    const int64_t t0 = r0 + (int64_t)(((__int128)span * i) / G);
-    const int64_t t1 = r0 + (int64_t)(((__int128)span * (i + 1)) / G);
-    *lo = lower_bound_off(off, nseq, t0);
-    *hi = (i + 1 == G) ? nseq : lower_bound_off(off, nseq, t1);
-    if (i == 0) *lo = 0;
+// Part i of `parts` owns the sequences whose start lies in [R*i/parts, R*(i+1)/parts) of the residue span R:
+// contiguous and residue-balanced.  Part 0 starts at sequence 0 and the last part ends at nseq.
+__device__ __forceinline__ void seq_range(const int64_t *__restrict__ off, int64_t nseq, int64_t part, int64_t parts,
+                                          int64_t *lo, int64_t *hi) {
+    const int64_t r0 = __ldg(off), span = __ldg(off + nseq) - r0;
+    const auto start = [&](int64_t i) { return lower_bound_off(off, nseq, r0 + (int64_t)(((__int128)span * i) / parts)); };
+    *lo = (part == 0) ? 0 : start(part);
+    *hi = (part + 1 == parts) ? nseq : start(part + 1);
+}
+
+template <int GT> __device__ __forceinline__ void gsync() { if (GT == 32) __syncwarp(); else __syncthreads(); }
+
+constexpr int TS_WALK_C = 12;                      // residues per thread and segment of ts_group_walk (4 * odd)
+
+// ---- a group of GT threads (one warp, or a whole CTA) walks ONE sequence [b, e) byte-wise -------------------------
+// Segments of GT * TS_WALK_C residues are staged into s_sym (ts_sym_bytes of that, at shared address sym_addr) through
+// the LUT, one 16-byte vector per thread; the first segment's front reads as invalid, the k-1 symbols in front of every
+// later segment are carried over from the previous one.  Thread g owns a 4*odd chunk of every segment, warms up on the
+// k-1 symbols in front of it and rolls the code with a run counter.  emit(widx, code, ok) is called at every position
+// of the chunk: widx = index of the window ending there (window i covers residues b+i .. b+i+k-1; negative in front of
+// the first window), ok = the window is valid (never for widx < 0).  All GT threads call this, converged.
+template <int GT, int UNROLL, typename KeyT, typename Emit>
+__device__ __forceinline__ void ts_group_walk(const uint8_t *__restrict__ res, int64_t nres, int64_t b, int64_t e,
+                                              const uint8_t *s_lut, uint8_t *s_sym, uint32_t sym_addr, int k, KeyT nsym,
+                                              KeyT pow_k1, int g, Emit &&emit) {
+    constexpr int SEG = GT * TS_WALK_C;
+    const uint32_t uk = uint32_t(k);
+    bool first = true;
+    uint32_t tail0 = 0, tail1 = 0;                      // the last k-1 symbols of the previous segment (k-1 <= 63)
+    for (int64_t a = b; a < e;) {
+        const int64_t a2 = min(e, (a + SEG) & ~int64_t(15));
+        if (!first) {
+            if (g < k - 1) s_sym[TS_PAD - (k - 1) + g] = uint8_t(tail0);
+            if (g + 32 < k - 1) s_sym[TS_PAD - (k - 1) + g + 32] = uint8_t(tail1);
+        }
+        // stage: [a & ~15, a2) translated into s_sym[TS_PAD ...), one 16-byte vector per thread
+        const int64_t base = a & ~int64_t(15);
+        const int lo_i = TS_PAD + int(a - base), hi_i = lo_i + int(a2 - a);
+        const int nvec = int((a2 - base + 15) >> 4);
+        if (g < nvec) {
+            const int64_t p = base + 16 * int64_t(g);
+            uint4 x;
+            if (p + 16 <= nres) {
+                x = __ldg(reinterpret_cast<const uint4 *>(res + p));
+            } else {
+                uint32_t w4[4] = {0, 0, 0, 0};
+                for (int j = 0; j < 16; ++j)
+                    if (p + j < nres) w4[j >> 2] |= uint32_t(res[p + j]) << (8 * (j & 3));
+                x = make_uint4(w4[0], w4[1], w4[2], w4[3]);
+            }
+            x.x = ts_translate4(x.x, s_lut);
+            x.y = ts_translate4(x.y, s_lut);
+            x.z = ts_translate4(x.z, s_lut);
+            x.w = ts_translate4(x.w, s_lut);
+            reinterpret_cast<uint4 *>(s_sym + TS_PAD)[g] = x;
+        }
+        gsync<GT>();
+        if (first) {                                    // nothing in front of the sequence start is a residue of it
+            for (int i = g; i < lo_i; i += GT) s_sym[i] = uint8_t(SYM_BAD);
+            gsync<GT>();
+        }
+        // scan: thread g owns symbols [i0, i1), warms up on the k-1 symbols in front of them
+        const int n = hi_i - lo_i;
+        const int C = ((int(unsigned(n + GT - 1) / GT) + 3) >> 2 | 1) << 2;     // smallest 4 * odd >= ceil(n / GT)
+        const int i0 = lo_i + g * C, i1 = min(i0 + C, hi_i);
+        if (i0 < i1) {
+            uint32_t run = 0;
+            KeyT code = 0;
+            uint32_t p = sym_addr + uint32_t(i0) - (uk - 1u);
+            for (uint32_t j = 1; j < uk; ++j, ++p) {
+                const uint32_t sy = lds_u8<0>(p);
+                run = (sy >= SYM_BAD) ? 0u : run + 1u;
+                code = code * nsym + KeyT(sy);
+            }
+            const uint32_t pend = sym_addr + uint32_t(i1);
+            const uint32_t back = uk - 1u;
+            int64_t widx = (a - b) + int64_t(i0 - lo_i) - int64_t(k - 1);
+#pragma unroll UNROLL
+            for (; p < pend; ++p, ++widx) {
+                const uint32_t sy = lds_u8<0>(p);
+                run = (sy >= SYM_BAD) ? 0u : run + 1u;
+                code = code * nsym + KeyT(sy);
+                emit(widx, code, run >= uk);
+                code -= KeyT(lds_u8<0>(p - back)) * pow_k1;
+            }
+        }
+        gsync<GT>();
+        if (g < k - 1) tail0 = s_sym[hi_i - (k - 1) + g];
+        if (g + 32 < k - 1) tail1 = s_sym[hi_i - (k - 1) + g + 32];
+        gsync<GT>();
+        first = false;
+        a = a2;
+    }
 }
 
 // ---- a CTA walks its share of the residue buffer, with the sequence index of every window -----------
@@ -217,7 +300,7 @@ __device__ __forceinline__ void ts_range_scan_rows(const uint8_t *__restrict__ r
                                                    int64_t origin, int64_t *s_ctl, Emit &&emit, Post &&post) {
     const int tid = threadIdx.x;
     unsigned int *s_nstart = reinterpret_cast<unsigned int *>(s_ctl + 2);
-    if (tid == 0) { cta_seq_range(off, nseq, &s_ctl[0], &s_ctl[1]); *s_nstart = 0; }
+    if (tid == 0) { seq_range(off, nseq, blockIdx.x, gridDim.x, &s_ctl[0], &s_ctl[1]); *s_nstart = 0; }
     __syncthreads();
     const int64_t lo = s_ctl[0], hi = s_ctl[1];
     if (lo >= hi) return;

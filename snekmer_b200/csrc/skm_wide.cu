@@ -13,10 +13,9 @@
 //                             GPUs): sort by code, reduce (sum of counts, min of first), drop count <=
 //                             min_filter, order by first position => basis codes in the reference's order, plus
 //                             the sorted code list with the column of every entry (the lookup structure).
-//  skm_count_csr_wide         per-sequence distinct codes + counts (CSR): segmented sort of each sequence's
-//                             64-bit codes, runs -> (code, count); with a basis, the code of every run is
-//                             looked up (binary search in the sorted code list) and runs outside it are dropped.
-//  skm_codes_to_columns       the lookup on its own.
+//  skm_codes_to_columns       the code -> column lookup in the sorted code list.
+// The per-sequence counts over a wide basis are skm_count_csr_sorted (skm_csrsort.cu) and its segmented-sort
+// cross-check skm_count_csr_wide (skm_count.cu), which use wide_check and launch_window_codes64 from here.
 // Everything is atomic-free and bit-reproducible.
 #include <cub/cub.cuh>
 
@@ -99,16 +98,6 @@ __global__ void __launch_bounds__(256) basis_emit_kernel(const uint64_t *__restr
     }
 }
 
-__device__ __forceinline__ int32_t lookup_column(const uint64_t *__restrict__ sorted_codes, const int32_t *__restrict__ col_of_sorted,
-                                                 int64_t K, uint64_t code) {
-    int64_t lo = 0, hi = K;
-    while (lo < hi) {
-        const int64_t mid = (lo + hi) >> 1;
-        if (__ldg(sorted_codes + mid) < code) lo = mid + 1; else hi = mid;
-    }
-    return (lo < K && __ldg(sorted_codes + lo) == code) ? __ldg(col_of_sorted + lo) : -1;
-}
-
 __global__ void __launch_bounds__(256) codes_to_columns_kernel(const uint64_t *__restrict__ codes, int64_t n,
                                                                const uint64_t *__restrict__ sorted_codes,
                                                                const int32_t *__restrict__ col_of_sorted, int64_t K,
@@ -117,51 +106,14 @@ __global__ void __launch_bounds__(256) codes_to_columns_kernel(const uint64_t *_
         cols[i] = lookup_column(sorted_codes, col_of_sorted, K, codes[i]);
 }
 
-// one warp per sequence over its sorted 64-bit keys: count (cols == vals == codes_out == NULL) or write the runs.
-// With a basis, runs whose code it does not hold are dropped and the column is written next to the code.
-__global__ void __launch_bounds__(256) csr_runs64_kernel(const uint64_t *__restrict__ keys, const int64_t *__restrict__ off,
-                                                         int64_t nseq, const uint64_t *__restrict__ sorted_codes,
-                                                         const int32_t *__restrict__ col_of_sorted, int64_t K, bool fill,
-                                                         int64_t *__restrict__ rowptr, uint64_t *__restrict__ codes_out,
-                                                         uint32_t *__restrict__ cols_out, int32_t *__restrict__ vals) {
-    const int lane = threadIdx.x & 31;
-    const int64_t warp = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
-    const int64_t nwarps = (int64_t(gridDim.x) * blockDim.x) >> 5;
-    for (int64_t s = warp; s < nseq; s += nwarps) {
-        const int64_t b = __ldg(off + s), e = __ldg(off + s + 1);
-        int64_t nrun = 0;
-        const int64_t wbase = fill ? rowptr[s] : 0;
-        for (int64_t p0 = b; p0 < e; p0 += 32) {
-            const int64_t p = p0 + lane;
-            const uint64_t key = (p < e) ? keys[p] : WD_NONE;
-            const uint64_t prevk = (p > b && p < e) ? keys[p - 1] : WD_NONE;
-            bool head = (p < e) && key != WD_NONE && (p == b || key != prevk);
-            int32_t col = -1;
-            if (head && sorted_codes) { col = lookup_column(sorted_codes, col_of_sorted, K, key); head = col >= 0; }
-            const unsigned m = __ballot_sync(FULL, head);
-            if (fill && head) {
-                int64_t q = p + 1;
-                while (q < e && keys[q] == key) ++q;       // runs are short: a k-mer repeated within one protein
-                const int64_t slot = wbase + nrun + __popc(m & ((1u << lane) - 1u));
-                if (codes_out) codes_out[slot] = key;
-                if (cols_out) cols_out[slot] = uint32_t(col);
-                vals[slot] = int32_t(q - p);
-            }
-            nrun += __popc(m);
-        }
-        if (!fill && lane == 0) rowptr[s + 1] = nrun;
-    }
-}
-
 struct MinI64 {
     __device__ __forceinline__ int64_t operator()(const int64_t &a, const int64_t &b) const { return a < b ? a : b; }
 };
 
-static size_t wal(size_t x) { return (x + 255) & ~size_t(255); }
-static int wbits_for(unsigned __int128 n) { int b = 1; while (b < 64 && (((unsigned __int128)1) << b) < n) ++b; return b; }
 constexpr int64_t WD_MAX_RES = 1ll << 30;
 
-static int wide_check(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq, const uint8_t *d_lut,
+// argument checks shared by the 64-bit entry points
+int wide_check(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq, const uint8_t *d_lut,
                       int nsym, int k, const char *who, unsigned __int128 *S) {
     int rc = check_common(d_residues, nres, d_offsets, nseq, d_lut, nsym, k);
     if (rc) return rc;
@@ -172,7 +124,8 @@ static int wide_check(const uint8_t *d_residues, int64_t nres, const int64_t *d_
     return SKM_OK;
 }
 
-static int launch_window_codes64(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq, const uint8_t *d_lut,
+// keys[p] = 64-bit code of the window ending at position p (positions outside every sequence are left alone)
+int launch_window_codes64(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq, const uint8_t *d_lut,
                                  int nsym, int k, uint64_t *d_keys, cudaStream_t st) {
     uint64_t pow_k1 = 1;
     for (int i = 0; i + 1 < k; ++i) pow_k1 *= (uint64_t)nsym;
@@ -198,7 +151,7 @@ size_t skm_basis_sorted_local_workspace(int64_t nres) {
     cub::DeviceRunLengthEncode::Encode(nullptr, t_rle, (const uint64_t *)nullptr, (uint64_t *)nullptr, (int64_t *)nullptr,
                                        (int64_t *)nullptr, (int)std::min<int64_t>(nres, (1ll << 31) - 1));
     cub::DeviceScan::ExclusiveSum(nullptr, t_scan, (const int64_t *)nullptr, (int64_t *)nullptr, nres);
-    return 2 * wal(size_t(nres) * 8) + 2 * wal(size_t(nres) * 4) + wal(std::max(t_sort, std::max(t_rle, t_scan))) + 1024;
+    return 2 * align256(size_t(nres) * 8) + 2 * align256(size_t(nres) * 4) + align256(std::max(t_sort, std::max(t_rle, t_scan))) + 1024;
 }
 
 int skm_basis_sorted_local(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq,
@@ -217,7 +170,7 @@ int skm_basis_sorted_local(const uint8_t *d_residues, int64_t nres, const int64_
     const size_t need = skm_basis_sorted_local_workspace(nres);
     if (!workspace || workspace_bytes < need) { set_error("skm_basis_sorted_local: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
     char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-    const size_t seg8 = wal(size_t(nres) * 8), seg4 = wal(size_t(nres) * 4);
+    const size_t seg8 = align256(size_t(nres) * 8), seg4 = align256(size_t(nres) * 4);
     uint64_t *keys_a = (uint64_t *)p, *keys_b = (uint64_t *)(p + seg8);
     uint32_t *pos_a = (uint32_t *)(p + 2 * seg8), *pos_b = (uint32_t *)(p + 2 * seg8 + seg4);
     void *temp = p + 2 * seg8 + 2 * seg4;
@@ -229,7 +182,7 @@ int skm_basis_sorted_local(const uint8_t *d_residues, int64_t nres, const int64_
     iota_u32_kernel<<<grid, 256, 0, st>>>(pos_a, nres);
     SKM_LAUNCH_CHECK("iota_u32_kernel");
     // valid codes are < S <= 2^end_bit - 1 = the low bits of the all-ones key, which therefore still sorts last
-    const int end_bit = wbits_for(S + 1);
+    const int end_bit = bits_for(S + 1);
     SKM_CUDA_TRY(cub::DeviceRadixSort::SortPairs(temp, temp_bytes, keys_a, keys_b, pos_a, pos_b, nres, 0, end_bit, st));
     int64_t *num_runs = reinterpret_cast<int64_t *>(keys_a);                // keys_a is free after the sort
     temp_bytes = workspace_bytes - size_t((char *)temp - (char *)workspace);
@@ -261,7 +214,7 @@ size_t skm_basis_sorted_finalize_workspace(int64_t n) {
     cub::DeviceSelect::Flagged(nullptr, t2, (const uint64_t *)nullptr, (const uint8_t *)nullptr, (uint64_t *)nullptr, (int64_t *)nullptr, n);
     t = std::max(t, t2);
     // keys_a keys_b (u64) | v1 v2 v3 (i64) | idx_a idx_b (u32) | flags (u8) | temp
-    return 5 * wal(size_t(n) * 8) + 2 * wal(size_t(n) * 4) + wal(size_t(n)) + wal(t) + 1024;
+    return 5 * align256(size_t(n) * 8) + 2 * align256(size_t(n) * 4) + align256(size_t(n)) + align256(t) + 1024;
 }
 
 int skm_basis_sorted_finalize(const uint64_t *d_codes, const int64_t *d_counts, const int64_t *d_first, int64_t n,
@@ -278,12 +231,12 @@ int skm_basis_sorted_finalize(const uint64_t *d_codes, const int64_t *d_counts, 
     const size_t need = skm_basis_sorted_finalize_workspace(n);
     if (!workspace || workspace_bytes < need) { set_error("skm_basis_sorted_finalize: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
     char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-    const size_t seg8 = wal(size_t(n) * 8), seg4 = wal(size_t(n) * 4);
+    const size_t seg8 = align256(size_t(n) * 8), seg4 = align256(size_t(n) * 4);
     uint64_t *keys_a = (uint64_t *)p, *keys_b = (uint64_t *)(p + seg8);
     int64_t *v1 = (int64_t *)(p + 2 * seg8), *v2 = (int64_t *)(p + 3 * seg8), *v3 = (int64_t *)(p + 4 * seg8);
     uint32_t *idx_a = (uint32_t *)(p + 5 * seg8), *idx_b = (uint32_t *)(p + 5 * seg8 + seg4);
     uint8_t *flags = (uint8_t *)(p + 5 * seg8 + 2 * seg4);
-    void *temp = p + 5 * seg8 + 2 * seg4 + wal(size_t(n));
+    void *temp = p + 5 * seg8 + 2 * seg4 + align256(size_t(n));
     const size_t temp_cap = workspace_bytes - size_t((char *)temp - (char *)workspace);
     size_t temp_bytes;
     const int grid = (int)std::min<int64_t>((n + 255) / 256, int64_t(sm_count()) * 16);
@@ -339,7 +292,7 @@ int skm_basis_sorted_finalize(const uint64_t *d_codes, const int64_t *d_counts, 
     SKM_LAUNCH_CHECK("iota_u32_kernel");
     temp_bytes = temp_cap;
     // positions are < first_bound <= 2^end_bit - 1 = the low bits of the padding value, which therefore still sorts last
-    const int order_bits = first_bound > 0 ? wbits_for((unsigned __int128)first_bound + 1) : 64;
+    const int order_bits = first_bound > 0 ? bits_for((unsigned __int128)first_bound + 1) : 64;
     SKM_CUDA_TRY(cub::DeviceRadixSort::SortPairs(temp, temp_bytes, reinterpret_cast<const uint64_t *>(first_sel), keys_b, idx_a, idx_b, n, 0, order_bits, st));
     basis_emit_kernel<<<grid, 256, 0, st>>>(d_sorted_codes_out, cnt_sel, idx_b, d_K_out, d_basis_out, d_basis_counts_out, d_col_of_sorted_out);
     SKM_LAUNCH_CHECK("basis_emit_kernel");
@@ -355,57 +308,6 @@ int skm_codes_to_columns(const uint64_t *d_codes, int64_t n, const uint64_t *d_s
     const int grid = (int)std::min<int64_t>((n + 255) / 256, int64_t(sm_count()) * 16);
     codes_to_columns_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(d_codes, n, d_sorted_codes, d_col_of_sorted, K, d_cols_out);
     SKM_LAUNCH_CHECK("codes_to_columns_kernel");
-    return SKM_OK;
-}
-
-size_t skm_count_csr_wide_workspace(int64_t nres, int64_t nseq) {
-    using namespace skm;
-    if (nres <= 0 || nseq <= 0) return 256;
-    const int64_t items = std::min<int64_t>(nres, WD_MAX_RES);
-    size_t t_sort = 0, t_scan = 0;
-    cub::DeviceSegmentedSort::SortKeys(nullptr, t_sort, (const uint64_t *)nullptr, (uint64_t *)nullptr, (int)items,
-                                       (int)std::min<int64_t>(nseq, (1ll << 31) - 1), (const int64_t *)nullptr,
-                                       (const int64_t *)nullptr);
-    cub::DeviceScan::InclusiveSum(nullptr, t_scan, (const int64_t *)nullptr, (int64_t *)nullptr, nseq);
-    return 2 * wal(size_t(nres) * 8) + wal(std::max(t_sort, t_scan)) + 1024;
-}
-
-int skm_count_csr_wide(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq,
-                       const uint8_t *d_lut, int nsym, int k, const uint64_t *d_sorted_codes,
-                       const int32_t *d_col_of_sorted, int64_t K, int64_t *d_rowptr, uint64_t *d_codes_out,
-                       uint32_t *d_cols_out, int32_t *d_vals, void *workspace, size_t workspace_bytes,
-                       skm_stream_t stream) {
-    using namespace skm;
-    unsigned __int128 S;
-    int rc = wide_check(d_residues, nres, d_offsets, nseq, d_lut, nsym, k, "skm_count_csr_wide", &S);
-    if (rc) return rc;
-    if (!d_rowptr) { set_error("skm_count_csr_wide: d_rowptr is NULL"); return SKM_ERR_INVALID; }
-    if (d_sorted_codes && (!d_col_of_sorted || K < 0)) { set_error("skm_count_csr_wide: basis given without its column map"); return SKM_ERR_INVALID; }
-    if (d_cols_out && !d_sorted_codes) { set_error("skm_count_csr_wide: d_cols_out needs a basis"); return SKM_ERR_INVALID; }
-    cudaStream_t st = (cudaStream_t)stream;
-    SKM_CUDA_TRY(cudaMemsetAsync(d_rowptr, 0, 8 * (size_t)(nseq + 1), st));
-    if (nseq == 0 || nres == 0) return SKM_OK;
-    if (!d_vals || (!d_codes_out && !d_cols_out)) { set_error("skm_count_csr_wide: NULL output"); return SKM_ERR_INVALID; }
-    const size_t need = skm_count_csr_wide_workspace(nres, nseq);
-    if (!workspace || workspace_bytes < need) { set_error("skm_count_csr_wide: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
-    char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-    const size_t seg = wal(size_t(nres) * 8);
-    uint64_t *keys_a = (uint64_t *)p, *keys_b = (uint64_t *)(p + seg);
-    void *temp = p + 2 * seg;
-    const size_t temp_cap = workspace_bytes - (size_t)((char *)temp - (char *)workspace);
-    size_t temp_bytes = temp_cap;
-    // keys are indexed by the absolute position of the window's last residue; positions outside every sequence are
-    // never read by the segmented sort
-    rc = launch_window_codes64(d_residues, nres, d_offsets, nseq, d_lut, nsym, k, keys_a, st);
-    if (rc) return rc;
-    SKM_CUDA_TRY(cub::DeviceSegmentedSort::SortKeys(temp, temp_bytes, keys_a, keys_b, (int)nres, (int)nseq, d_offsets, d_offsets + 1, st));
-    const int grid = sm_count() * 8;
-    csr_runs64_kernel<<<grid, 256, 0, st>>>(keys_b, d_offsets, nseq, d_sorted_codes, d_col_of_sorted, K, false, d_rowptr, nullptr, nullptr, nullptr);
-    SKM_LAUNCH_CHECK("csr_runs64_kernel(count)");
-    temp_bytes = temp_cap;
-    SKM_CUDA_TRY(cub::DeviceScan::InclusiveSum(temp, temp_bytes, d_rowptr + 1, d_rowptr + 1, nseq, st));
-    csr_runs64_kernel<<<grid, 256, 0, st>>>(keys_b, d_offsets, nseq, d_sorted_codes, d_col_of_sorted, K, true, d_rowptr, d_codes_out, d_cols_out, d_vals);
-    SKM_LAUNCH_CHECK("csr_runs64_kernel(fill)");
     return SKM_OK;
 }
 

@@ -1399,18 +1399,16 @@ def count_csr_wide(batch: SequenceBatch, alphabet: AlphabetT, k: int, basis: Opt
     if basis is not None and basis.K == 0:           # nothing can match an empty basis
         return (torch.zeros(batch.n + 1, dtype=torch.int64, device=dev), torch.zeros(0, dtype=torch.int64, device=dev),
                 torch.zeros(0, dtype=torch.int32, device=dev), torch.zeros(0, dtype=torch.int32, device=dev))
-    rowptrs, codes_p, cols_p, vals_p = [], [], [], []
-    base_nnz = 0
-    for lo, hi in _chunks_by_residues(batch.offsets_host, max_chunk_res):
-        sub = batch if (lo == 0 and hi == batch.n) else _sub_batch(batch, lo, hi)
+    b_codes = None if basis is None else _ptr(basis.sorted_codes)
+    b_cols = None if basis is None else _ptr(basis.col_of_sorted)
+    b_K = 0 if basis is None else basis.K
+
+    def count(sub: SequenceBatch):
         cap = max(sub.nres, 1)
         rowptr = torch.empty(sub.n + 1, dtype=torch.int64, device=dev)
         codes = torch.empty(cap, dtype=torch.int64, device=dev)
         cols = torch.empty(cap, dtype=torch.int32, device=dev) if basis is not None else None
         vals = torch.empty(cap, dtype=torch.int32, device=dev)
-        b_codes = None if basis is None else _ptr(basis.sorted_codes)
-        b_cols = None if basis is None else _ptr(basis.col_of_sorted)
-        b_K = 0 if basis is None else basis.K
         if method == "segsort":          # the first implementation (window keys in HBM + cub::DeviceSegmentedSort), a cross-check
             ws_bytes = lib().skm_count_csr_wide_workspace(sub.nres, sub.n)
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
@@ -1424,20 +1422,28 @@ def count_csr_wide(batch: SequenceBatch, alphabet: AlphabetT, k: int, basis: Opt
                                              None, 0, b_codes, b_cols, b_K, max_len, _ptr(rowptr), _ptr(codes), _ptr(cols), _ptr(vals),
                                              _ptr(ws), ws_bytes, _stream()))
         nnz = int(rowptr[-1].item()) if sub.n else 0
-        rowptrs.append(rowptr[(1 if rowptrs else 0):] + base_nnz)
-        codes_p.append(codes[:nnz].clone())
-        vals_p.append(vals[:nnz].clone())
-        if cols is not None:
-            cols_p.append(cols[:nnz].clone())
-        base_nnz += nnz
-        del ws, codes, cols, vals
+        return rowptr, codes[:nnz].clone(), (cols[:nnz].clone() if cols is not None else None), vals[:nnz].clone()
+
+    return _csr_by_chunks(batch, max_chunk_res, (torch.int64, torch.int32 if basis is not None else None, torch.int32), count)
+
+
+def _csr_by_chunks(batch: SequenceBatch, max_chunk_res: int, dtypes, count):
+    """CSR of `batch` from `count(sub) -> (rowptr, *entry arrays)` run on every chunk of at most `max_chunk_res`
+    residues: the chunks' rowptrs are rebased onto one running nnz and their entry arrays concatenated (an array that
+    is None stays None).  `dtypes` are the entry arrays' dtypes (None: the array is None) for a batch with no chunk."""
+    dev = batch.device
+    rowptrs, parts, base = [], [], 0
+    for lo, hi in _chunks_by_residues(batch.offsets_host, max_chunk_res):
+        sub = batch if (lo == 0 and hi == batch.n) else _sub_batch(batch, lo, hi)
+        rowptr, *arrays = count(sub)
+        rowptrs.append(rowptr[(1 if rowptrs else 0):] + base)
+        parts.append(arrays)
+        base += int(arrays[-1].numel())
     if not rowptrs:
-        z = torch.zeros(1, dtype=torch.int64, device=dev)
-        e64 = torch.zeros(0, dtype=torch.int64, device=dev)
-        e32 = torch.zeros(0, dtype=torch.int32, device=dev)
-        return z, e64, (e32 if basis is not None else None), e32.clone()
+        return (torch.zeros(1, dtype=torch.int64, device=dev),
+                *(None if dt is None else torch.zeros(0, dtype=dt, device=dev) for dt in dtypes))
     cat = (lambda xs: xs[0] if len(xs) == 1 else torch.cat(xs))
-    return cat(rowptrs), cat(codes_p), (cat(cols_p) if basis is not None else None), cat(vals_p)
+    return (cat(rowptrs), *(None if xs[0] is None else cat(list(xs)) for xs in zip(*parts)))
 
 
 def build_basis_wide_distributed(batch: SequenceBatch, alphabet, k: int, min_filter: int = 0,
@@ -1491,17 +1497,9 @@ def vectorize(batch: SequenceBatch, alphabet: AlphabetT, k: int, min_filter: int
         basis = build_basis(batch, alphabet, k, min_filter)
         if basis.K <= dense_max_K:
             return Vectorized("dense", basis, counts=count_dense(batch, alphabet, k, basis))
-        parts, base = [], 0
-        for lo, hi in _chunks_by_residues(batch.offsets_host, (1 << 30) - 16):
-            sub = batch if (lo == 0 and hi == batch.n) else _sub_batch(batch, lo, hi)
-            rp, c, v = count_csr(sub, alphabet, k, basis)
-            parts.append((rp[(1 if parts else 0):] + base, c, v))
-            base += int(v.numel())
-        if not parts:
-            z32 = torch.zeros(0, dtype=torch.int32, device=batch.device)
-            return Vectorized("csr", basis, rowptr=torch.zeros(1, dtype=torch.int64, device=batch.device), cols=z32, vals=z32.clone())
-        cat = (lambda xs: xs[0] if len(xs) == 1 else torch.cat(xs))
-        return Vectorized("csr", basis, rowptr=cat([p[0] for p in parts]), cols=cat([p[1] for p in parts]), vals=cat([p[2] for p in parts]))
+        rowptr, cols, vals = _csr_by_chunks(batch, (1 << 30) - 16, (torch.int32, torch.int32),
+                                            lambda sub: count_csr(sub, alphabet, k, basis))
+        return Vectorized("csr", basis, rowptr=rowptr, cols=cols, vals=vals)
     basis = build_basis_wide(batch, alphabet, k, min_filter)
     rowptr, codes, cols, vals = count_csr_wide(batch, alphabet, k, basis)
     return Vectorized("wide", basis, rowptr=rowptr, cols=cols, vals=vals, codes=codes)

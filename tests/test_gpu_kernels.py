@@ -153,7 +153,11 @@ def test_golden_rule_fixtures(name):
     assert np.allclose(r.score1.cpu().numpy(), rs1, rtol=1e-5, atol=0)
 
 
-@pytest.mark.parametrize("a,k,mf", [(5, 3, 0), (2, 8, 0), (0, 12, 2), (None, 3, 0), (1, 4, 5), ("ptm", 2, 0), (4, 9, 0)])
+# Between them, the int32 and uint16 counts of these cases reach every dense count kernel: the tile kernel with and
+# without a column map, and both warp kernels (words: k <= 5, bytes: k > 5) with each column-map mode (identity, map in
+# shared memory for S <= 16384, map in global memory beyond; the last two filtered down to a few thousand columns).
+@pytest.mark.parametrize("a,k,mf", [(5, 3, 0), (2, 8, 0), (0, 12, 2), (None, 3, 0), (1, 4, 5), ("ptm", 2, 0), (4, 9, 0),
+                                    (0, 11, 0), (None, 4, 6), (2, 10, 14)])
 def test_basis_and_dense_counts_random(a, k, mf):
     rng = np.random.default_rng(hash((str(a), k)) % 2 ** 32)
     seqs = _rand_seqs(rng, 700, 0, 900)
@@ -166,12 +170,14 @@ def test_basis_and_dense_counts_random(a, k, mf):
     assert np.array_equal(basis.codes_host(), want_basis)
     assert np.array_equal(basis.counts.cpu().numpy(), want_tot)
     want = O.count_matrix(si, code, valid, len(seqs), want_basis)
-    got = E.count_dense(batch, a, k, basis).cpu().numpy()
-    assert np.array_equal(got, want)
+    for dtype in (torch.int32, torch.uint16):
+        got = E.count_dense(batch, a, k, basis, dtype=dtype).cpu().numpy()
+        assert np.array_equal(got, want)
     if len(syms) ** k <= 20000:
-        ident = E.count_dense(batch, a, k, None).cpu().numpy()
         full = O.count_matrix(si, code, valid, len(seqs), np.arange(len(syms) ** k, dtype=np.uint64))
-        assert np.array_equal(ident, full)
+        for dtype in (torch.int32, torch.uint16):
+            ident = E.count_dense(batch, a, k, None, dtype=dtype).cpu().numpy()
+            assert np.array_equal(ident, full)
 
 
 def test_dense_counts_long_sequences_use_32bit_counters():
