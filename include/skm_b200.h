@@ -223,6 +223,22 @@ SKM_API int skm_coo_merge(const uint64_t *d_keys_in, const int64_t *d_vals_in, i
                   uint64_t *d_keys_out, int64_t *d_vals_out, int64_t *d_n_out,
                   void *workspace, size_t workspace_bytes, skm_stream_t stream);
 
+/* (a12/a13 at nsym^k beyond the tables, up to 2^64 - 1) learn, wide: learn.smk:306-326,359-408 with the matrix keyed by
+ * BASIS COLUMN.  The basis is (d_sorted_codes uint64 [K] ascending, d_col_of_sorted int32 [K]: its column of each),
+ * K < 2^31, as skm_basis_sorted_finalize gives it.  Every valid window whose code the basis holds becomes the key
+ * a * K + col, with a = d_ann_id[s] when it is in [0, n_ann) and a = n_ann (the rest row) otherwise; keys are
+ * radix-sorted and run-length encoded (no atomics).  Output: a COO list sorted by key, capacity nres, the number of
+ * entries in *d_nnz (device int64).  The Totals row (learn.smk:380: occurrences over ALL sequences, restricted to the
+ * basis columns) is skm_coo_colsum of the whole list with S = K; the annotated matrix is its prefix key < n_ann * K.
+ * Needs (n_ann + 2) * K < 2^63.  One call handles < 2^30 residues: split larger shards and merge the chunks' sorted
+ * lists with skm_coo_merge_runs. */
+SKM_API size_t skm_learn_wide_workspace(int64_t nres);
+SKM_API int skm_learn_wide(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq,
+                   const uint8_t *d_lut, int nsym, int k, const int32_t *d_ann_id, int64_t n_ann,
+                   const uint64_t *d_sorted_codes, const int32_t *d_col_of_sorted, int64_t K,
+                   uint64_t *d_keys_out, int64_t *d_vals_out, int64_t *d_nnz, void *workspace,
+                   size_t workspace_bytes, skm_stream_t stream);
+
 /* ---- code spaces too large for tables (nsym^k > 2^27, up to 2^64 - 1: the alphabet/k sweep) ----------
  * (a7) basis of one shard as a table sorted by code: distinct window codes, their occurrence counts and the
  * position (res_base + index of the window's last residue) of their first occurrence — the dict of
@@ -282,8 +298,12 @@ SKM_API int skm_coo_merge_runs(const uint64_t *d_keys_in, const int64_t *d_vals_
  * d_colptr int64 [S+1], d_rows int32 [nnz] (annotation), d_mvals int32 [nnz] = M[a, c],
  * d_mnorm2 (nullable) = ||m_a||^2 (exact integer sum, as float64), d_inv_m32 (nullable) =
  * float32 1 / ||m_a|| (0 for empty rows), *d_max_m = largest entry (callers must check it
- * is < 2^31: larger entries do not fit d_mvals). */
+ * is < 2^31: larger entries do not fit d_mvals).  S <= 2^31 - 1 (S is the key stride: nsym^k, or the basis
+ * column count of a matrix keyed by column). */
 SKM_API size_t skm_csc_build_workspace(int64_t nnz, int64_t n_ann);
+/* skm_csc_build_workspace for S columns: S may be up to 2^31 - 1 (a learned matrix keyed by basis column,
+ * skm_learn_wide); for S <= SKM_DENSE_MAX_SPACE it equals skm_csc_build_workspace, which sizes for those. */
+SKM_API size_t skm_csc_build_workspace_cols(int64_t nnz, int64_t n_ann, int64_t S);
 SKM_API int skm_csc_build(const uint64_t *d_keys, const int64_t *d_vals, int64_t nnz, int64_t S,
                   int64_t n_ann, int64_t *d_colptr, int32_t *d_rows, int32_t *d_mvals,
                   double *d_mnorm2, float *d_inv_m32, int64_t *d_max_m, void *workspace,

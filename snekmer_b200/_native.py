@@ -55,6 +55,8 @@ SIGNATURES = {
     "skm_apply_dense": (_int, [_p, _i64, _i64, _p, _i64, _p, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "skm_learn_sparse_workspace": (_sz, [_i64]),
     "skm_learn_sparse": (_int, [_p, _i64, _p, _i64, _p, _int, _int, _p, _i64, _p, _p, _p, _p, _sz, _p]),
+    "skm_learn_wide_workspace": (_sz, [_i64]),
+    "skm_learn_wide": (_int, [_p, _i64, _p, _i64, _p, _int, _int, _p, _i64, _p, _p, _i64, _p, _p, _p, _p, _sz, _p]),
     "skm_basis_sorted_local_workspace": (_sz, [_i64]),
     "skm_basis_sorted_local": (_int, [_p, _i64, _p, _i64, _p, _int, _int, _i64, _p, _p, _p, _p, _p, _sz, _p]),
     "skm_basis_sorted_finalize_workspace": (_sz, [_i64]),
@@ -74,6 +76,7 @@ SIGNATURES = {
     "skm_coo_merge_runs_workspace": (_sz, [_i64, _int]),
     "skm_coo_merge_runs": (_int, [_p, _p, _p, _int, _p, _p, _p, _p, _sz, _p]),
     "skm_csc_build_workspace": (_sz, [_i64, _i64]),
+    "skm_csc_build_workspace_cols": (_sz, [_i64, _i64, _i64]),
     "skm_csc_build": (_int, [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "skm_csc_pack": (_int, [_p, _p, _i64, _p, _p]),
     "skm_apply_sparse": (_int, [_p, _p, _p, _i64, _p, _p, _p, _p, _p, _p, _i64, _int, _p, _p, _p, _p, _p, _p]),

@@ -162,6 +162,37 @@ __device__ __forceinline__ int32_t lookup_column(const uint64_t *__restrict__ so
     return (lo < K && __ldg(sorted_codes + lo) == code) ? __ldg(col_of_sorted + lo) : -1;
 }
 
+// basis lookup: sorted code list + column of each entry; `bucket` (nullable) = start index of every 2^shift-wide
+// code range, so the binary search runs over a handful of entries
+struct SortedBasis {
+    const uint64_t *codes;
+    const int32_t *col;
+    const uint32_t *bucket;     // [nbucket + 1]
+    int64_t K;
+    int shift;
+};
+__device__ __forceinline__ int32_t sorted_lookup(const SortedBasis &b, uint64_t code) {
+    int64_t lo = 0, hi = b.K;
+    if (b.bucket) {
+        const uint64_t q = code >> b.shift;
+        lo = __ldg(b.bucket + q);
+        hi = __ldg(b.bucket + q + 1);
+    }
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (__ldg(b.codes + mid) < code) lo = mid + 1; else hi = mid;
+    }
+    return (lo < b.K && __ldg(b.codes + lo) == code) ? __ldg(b.col + lo) : -1;
+}
+
+constexpr int SORTED_BUCKET_BITS = 20;
+// bytes of the bucket index sorted_basis_init may build
+constexpr size_t SORTED_BUCKET_BYTES = ((size_t(1) << SORTED_BUCKET_BITS) + 2) * 4;
+// host (skm_csrsort.cu): *sb = the lookup over (codes, col, K) in a code space of S codes; bases of more than 64 entries
+// get a bucket index of at most 2^20 + 1 entries, built into `bucket` (SORTED_BUCKET_BYTES) on stream st
+int sorted_basis_init(SortedBasis *sb, const uint64_t *codes, const int32_t *col, int64_t K, unsigned __int128 S,
+                      uint32_t *bucket, cudaStream_t st);
+
 int check_common(const void *d_residues, int64_t nres, const void *d_offsets, int64_t nseq,
                  const void *d_lut, int nsym, int k);
 

@@ -36,29 +36,6 @@ template <typename T> struct key_none;
 template <> struct key_none<uint32_t> { static constexpr uint32_t v = 0xFFFFFFFFu; };
 template <> struct key_none<uint64_t> { static constexpr uint64_t v = ~0ull; };
 
-// basis lookup: sorted code list + column of each entry; `bucket` (nullable) = start index of every 2^shift-wide
-// code range, so the binary search runs over a handful of entries
-struct SortedBasis {
-    const uint64_t *codes;
-    const int32_t *col;
-    const uint32_t *bucket;     // [nbucket + 1]
-    int64_t K;
-    int shift;
-};
-__device__ __forceinline__ int32_t sorted_lookup(const SortedBasis &b, uint64_t code) {
-    int64_t lo = 0, hi = b.K;
-    if (b.bucket) {
-        const uint64_t q = code >> b.shift;
-        lo = __ldg(b.bucket + q);
-        hi = __ldg(b.bucket + q + 1);
-    }
-    while (lo < hi) {
-        const int64_t mid = (lo + hi) >> 1;
-        if (__ldg(b.codes + mid) < code) lo = mid + 1; else hi = mid;
-    }
-    return (lo < b.K && __ldg(b.codes + lo) == code) ? __ldg(b.col + lo) : -1;
-}
-
 // ascending bitonic network over keys[0, n) by a group of GT threads (g = thread index in the group)
 template <typename KeyT, int GT>
 __device__ __forceinline__ void group_sort(KeyT *keys, int n, int g) {
@@ -411,8 +388,20 @@ __global__ void __launch_bounds__(256) bucket_index_kernel(const uint64_t *__res
     }
 }
 
+int sorted_basis_init(SortedBasis *sb, const uint64_t *codes, const int32_t *col, int64_t K, unsigned __int128 S,
+                      uint32_t *bucket, cudaStream_t st) {
+    *sb = SortedBasis{codes, col, nullptr, K, 0};
+    if (K <= 64) return SKM_OK;
+    const int bits = bits_for(S);
+    sb->shift = bits > SORTED_BUCKET_BITS ? bits - SORTED_BUCKET_BITS : 0;
+    const int64_t nbucket = int64_t((S - 1) >> sb->shift) + 1;            // <= 2^20
+    bucket_index_kernel<<<(int)std::min<int64_t>((nbucket + 256) / 256, 1024), 256, 0, st>>>(codes, K, sb->shift, nbucket, bucket);
+    SKM_LAUNCH_CHECK("bucket_index_kernel");
+    sb->bucket = bucket;
+    return SKM_OK;
+}
+
 constexpr int64_t CS_MAX_RES = 1ll << 30;
-constexpr int CS_BUCKET_BITS = 20;
 
 
 struct CsPlan {
@@ -440,7 +429,7 @@ static CsPlan cs_plan(int64_t nres, int64_t nseq, int64_t max_len, size_t key_by
     p.long_list = take(size_t(nseq) * 8);
     p.n_long = take(8);
     p.gscratch = take(size_t(p.gscratch_stride) * key_bytes * p.long_grid);
-    p.bucket = take(with_bucket ? ((size_t(1) << CS_BUCKET_BITS) + 2) * 4 : 0);
+    p.bucket = take(with_bucket ? SORTED_BUCKET_BYTES : 0);
     p.scan_temp = take(t_scan);
     p.total = o + 512;
     return p;
@@ -536,19 +525,13 @@ int skm_count_csr_sorted(const uint8_t *d_residues, int64_t nres, const int64_t 
     if (nres >= CS_MAX_RES || nseq >= (1ll << 31)) { set_error("skm_count_csr_sorted: more than 2^30 residues per call; split the shard"); return SKM_ERR_UNSUPPORTED; }
     if (max_len <= 0 || max_len > nres) max_len = nres;          // unknown: assume the worst
     const bool wide = key_bits == 64;
-    const bool with_bucket = wide && d_sorted_codes && K > 64;
     const CsPlan pl = cs_plan(nres, nseq, max_len, wide ? 8 : 4, wide, wide);
     if (!workspace || workspace_bytes < pl.total + 256) { set_error("skm_count_csr_sorted: workspace %zu < %zu", workspace_bytes, pl.total + 256); return SKM_ERR_WORKSPACE; }
     char *ws = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
-    SortedBasis sb{d_sorted_codes, d_col_of_sorted, nullptr, K, 0};
-    if (with_bucket) {
-        const int bits = bits_for(S128);
-        sb.shift = bits > CS_BUCKET_BITS ? bits - CS_BUCKET_BITS : 0;
-        const int64_t nbucket = int64_t((S128 - 1) >> sb.shift) + 1;            // <= 2^20
-        uint32_t *bucket = reinterpret_cast<uint32_t *>(ws + pl.bucket);
-        bucket_index_kernel<<<(int)std::min<int64_t>((nbucket + 256) / 256, 1024), 256, 0, st>>>(d_sorted_codes, K, sb.shift, nbucket, bucket);
-        SKM_LAUNCH_CHECK("bucket_index_kernel");
-        sb.bucket = bucket;
+    SortedBasis sb{};
+    if (wide && d_sorted_codes) {
+        rc = sorted_basis_init(&sb, d_sorted_codes, d_col_of_sorted, K, S128, reinterpret_cast<uint32_t *>(ws + pl.bucket), st);
+        if (rc) return rc;
     }
     if (!wide) {
         if (d_col_of_code) return cs_run<uint32_t, 1>(d_residues, nres, d_offsets, nseq, d_lut, nsym, k, d_col_of_code, nullptr, max_len, pl, ws, d_rowptr, (uint32_t *)d_keys_out, nullptr, d_vals, st);

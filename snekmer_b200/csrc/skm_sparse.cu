@@ -7,6 +7,8 @@
 //                     (key, count) list = the annotation x k-mer count matrix.  No atomics,
 //                     bit-reproducible.  Unannotated sequences only feed the Totals table
 //                     (skm_basis_accumulate gives it).
+//  skm_learn_wide     the same list over code spaces beyond the tables (up to 2^64 - 1), keyed by BASIS COLUMN:
+//                     ann * K + col, with a rest row for the unannotated sequences whose column sums are the Totals.
 //  skm_coo_merge      sum of COO lists with equal keys (sort by key + reduce by key):
 //                     Merge.merge_dataframes (learn.smk:467-494) for sparse matrices, and the
 //                     fan-in after an all-gather of per-GPU lists.
@@ -75,6 +77,47 @@ __global__ void __launch_bounds__(TS_THREADS) window_keys_kernel(const uint8_t *
                                      for (int i = threadIdx.x; i < n; i += blockDim.x) keys[rel_a + i] = s_keys[i];
                                  });
 }
+
+// keys[p] for the wide learn (skm_learn_wide): a * K + col for the window whose last residue sits at p, with col its
+// basis column (bucketed binary search) and a = ann_id[row], or n_ann (the rest row) when the sequence has no annotation
+// in [0, n_ann); `invalid` when the window is invalid or its code is not in the basis
+__global__ void __launch_bounds__(TS_THREADS) learn_wide_keys_kernel(const uint8_t *__restrict__ res, int64_t nres,
+                                                                     const int64_t *__restrict__ off, int64_t nseq,
+                                                                     const uint8_t *__restrict__ lut, uint64_t nsym, int k,
+                                                                     uint64_t pow_k1, const int32_t *__restrict__ ann_id,
+                                                                     int64_t n_ann, SortedBasis sb, uint64_t invalid,
+                                                                     uint64_t *__restrict__ keys) {
+    extern __shared__ __align__(128) uint8_t s_sym[];
+    __shared__ uint8_t s_lut[256];
+    __shared__ int64_t s_ctl[4];
+    uint64_t *s_keys = reinterpret_cast<uint64_t *>(s_sym + SP_SYM_BYTES);
+    ts_lut_init(s_lut, lut);
+    __syncthreads();
+    int64_t ann_row = -2;          // row whose annotation is cached
+    uint64_t ann_base = 0;
+    ts_range_scan_rows<uint64_t>(res, nres, off, nseq, s_lut, s_sym, SP_SEG, k, nsym, pow_k1, /*origin=*/0, s_ctl,
+                                 [&](int64_t, int64_t row, uint64_t code, bool ok, int local) {
+                                     uint64_t key = invalid;
+                                     if (ok) {
+                                         const int32_t c = sorted_lookup(sb, code);
+                                         if (c >= 0) {
+                                             if (row != ann_row) {
+                                                 ann_row = row;
+                                                 const int32_t a = __ldg(ann_id + row);
+                                                 ann_base = uint64_t(a >= 0 && a < n_ann ? int64_t(a) : n_ann) * uint64_t(sb.K);
+                                             }
+                                             key = ann_base + uint64_t(c);
+                                         }
+                                     }
+                                     s_keys[local] = key;
+                                 },
+                                 [&](int64_t rel_a, int n) {         // coalesced copy of the segment's keys
+                                     for (int i = threadIdx.x; i < n; i += blockDim.x) keys[rel_a + i] = s_keys[i];
+                                 });
+}
+
+int wide_check(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq, const uint8_t *d_lut,
+               int nsym, int k, const char *who, unsigned __int128 *S);      // skm_wide.cu
 
 // the runs of the invalid key (and of the all-ones fill outside the sequences) sort last: drop them
 __global__ void coo_finish_kernel(const uint64_t *__restrict__ uniq, const int64_t *__restrict__ num_runs, uint64_t invalid,
@@ -478,6 +521,66 @@ int skm_learn_sparse(const uint8_t *d_residues, int64_t nres, const int64_t *d_o
     window_keys_kernel<1, uint64_t><<<(unsigned)grid, TS_THREADS, sp_smem_bytes<uint64_t>(), st>>>(d_residues, nres, d_offsets, nseq, d_lut, (uint32_t)nsym, k,
                                                                                       pow_k1, nullptr, d_ann_id, S, invalid, keys_a);
     SKM_LAUNCH_CHECK("window_keys_kernel<1>");
+    // keys are < 2^end_bit except the all-ones fill, whose low bits are all ones too: it still sorts last
+    const int end_bit = bits_for((unsigned __int128)invalid + 1);
+    SKM_CUDA_TRY(cub::DeviceRadixSort::SortKeys(temp, temp_bytes, keys_a, keys_b, nres, 0, end_bit, st));
+    int64_t *num_runs = reinterpret_cast<int64_t *>(keys_a);     // keys_a is free after the sort
+    temp_bytes = workspace_bytes - size_t((char *)temp - (char *)workspace);
+    SKM_CUDA_TRY(cub::DeviceRunLengthEncode::Encode(temp, temp_bytes, keys_b, d_keys_out, d_vals_out, num_runs, (int)nres, st));
+    coo_finish_kernel<<<1, 1, 0, st>>>(d_keys_out, num_runs, invalid, d_nnz);
+    SKM_LAUNCH_CHECK("coo_finish_kernel");
+    return SKM_OK;
+}
+
+// ---- wide learn: the matrix keyed by basis column (code spaces beyond the tables, up to 2^64 - 1) --------------
+// Every window whose code the basis holds becomes the key a * K + col (skm_learn_sparse's key with the stride K of the
+// basis in place of S); unannotated sequences get the rest row a = n_ann, so the column sums of the whole list are the
+// Totals over all sequences (learn.smk:380) and the annotated matrix is the prefix key < n_ann * K.
+size_t skm_learn_wide_workspace(int64_t nres) {
+    using namespace skm;
+    if (nres <= 0) return 256;
+    return skm_learn_sparse_workspace(nres) + align256(SORTED_BUCKET_BYTES);
+}
+
+int skm_learn_wide(const uint8_t *d_residues, int64_t nres, const int64_t *d_offsets, int64_t nseq,
+                   const uint8_t *d_lut, int nsym, int k, const int32_t *d_ann_id, int64_t n_ann,
+                   const uint64_t *d_sorted_codes, const int32_t *d_col_of_sorted, int64_t K,
+                   uint64_t *d_keys_out, int64_t *d_vals_out, int64_t *d_nnz, void *workspace,
+                   size_t workspace_bytes, skm_stream_t stream) {
+    using namespace skm;
+    unsigned __int128 S128;
+    int rc = wide_check(d_residues, nres, d_offsets, nseq, d_lut, nsym, k, "skm_learn_wide", &S128);
+    if (rc) return rc;
+    if (n_ann < 0 || K < 0 || K >= (1ll << 31)) { set_error("skm_learn_wide: n_ann=%lld K=%lld outside [0, 2^31)", (long long)n_ann, (long long)K); return SKM_ERR_INVALID; }
+    if ((unsigned __int128)(n_ann + 2) * (unsigned __int128)K >= ((unsigned __int128)1 << 63)) { set_error("skm_learn_wide: (n_ann + 2) * K does not fit 63 bits"); return SKM_ERR_UNSUPPORTED; }
+    if (!d_nnz) { set_error("skm_learn_wide: d_nnz is NULL"); return SKM_ERR_INVALID; }
+    cudaStream_t st = (cudaStream_t)stream;
+    SKM_CUDA_TRY(cudaMemsetAsync(d_nnz, 0, 8, st));
+    if (nseq == 0 || nres == 0 || K == 0) return SKM_OK;
+    if (!d_ann_id || !d_sorted_codes || !d_col_of_sorted || !d_keys_out || !d_vals_out) { set_error("skm_learn_wide: NULL argument"); return SKM_ERR_INVALID; }
+    const size_t need = skm_learn_wide_workspace(nres);
+    if (!workspace || workspace_bytes < need) { set_error("skm_learn_wide: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
+    char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
+    const size_t seg = align256(size_t(nres) * 8);
+    uint64_t *keys_a = (uint64_t *)p, *keys_b = (uint64_t *)(p + seg);
+    uint32_t *bucket = (uint32_t *)(p + 2 * seg);
+    void *temp = p + 2 * seg + align256(SORTED_BUCKET_BYTES);
+    size_t temp_bytes = workspace_bytes - size_t((char *)temp - (char *)workspace);
+    SortedBasis sb;
+    rc = sorted_basis_init(&sb, d_sorted_codes, d_col_of_sorted, K, S128, bucket, st);
+    if (rc) return rc;
+    const uint64_t invalid = uint64_t(n_ann + 1) * uint64_t(K);
+    uint64_t pow_k1 = 1;
+    for (int i = 0; i + 1 < k; ++i) pow_k1 *= (uint64_t)nsym;
+    int64_t grid = int64_t(sm_count()) * 8;
+    const int64_t max_grid = (nres + SP_SEG - 1) / SP_SEG;
+    if (grid > max_grid) grid = max_grid < 1 ? 1 : max_grid;
+    // positions outside [off[0], off[nseq]) are not written by the kernel
+    SKM_CUDA_TRY(cudaMemsetAsync(keys_a, 0xFF, size_t(nres) * 8, st));
+    SKM_CUDA_TRY(cudaFuncSetAttribute(learn_wide_keys_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, sp_smem_bytes<uint64_t>()));
+    learn_wide_keys_kernel<<<(unsigned)grid, TS_THREADS, sp_smem_bytes<uint64_t>(), st>>>(d_residues, nres, d_offsets, nseq, d_lut, (uint64_t)nsym, k,
+                                                                                      pow_k1, d_ann_id, n_ann, sb, invalid, keys_a);
+    SKM_LAUNCH_CHECK("learn_wide_keys_kernel");
     // keys are < 2^end_bit except the all-ones fill, whose low bits are all ones too: it still sorts last
     const int end_bit = bits_for((unsigned __int128)invalid + 1);
     SKM_CUDA_TRY(cub::DeviceRadixSort::SortKeys(temp, temp_bytes, keys_a, keys_b, nres, 0, end_bit, st));
@@ -953,21 +1056,27 @@ int skm_coo_merge_runs_packed(const uint64_t *d_packed_in, const int64_t *run_of
     return SKM_OK;
 }
 
-size_t skm_csc_build_workspace(int64_t nnz, int64_t n_ann) {
+constexpr int64_t SKM_CSC_MAX_COLS = (1ll << 31) - 1;
+
+size_t skm_csc_build_workspace_cols(int64_t nnz, int64_t n_ann, int64_t S) {
     using namespace skm;
     if (nnz <= 0) return 256 + align256(size_t(std::max<int64_t>(n_ann, 1)) * 8);
     size_t t_sort = 0, t_scan = 0;
     cub::DeviceRadixSort::SortPairs(nullptr, t_sort, (const uint64_t *)nullptr, (uint64_t *)nullptr, (const int64_t *)nullptr,
                                     (int64_t *)nullptr, nnz, 0, 64);
-    cub::DeviceScan::InclusiveSum(nullptr, t_scan, (const int64_t *)nullptr, (int64_t *)nullptr, (int64_t)1 << 27);
+    // the colptr scan: sized for 2^27 columns, or for S + 1 beyond that
+    const int64_t scan_n = std::max<int64_t>((int64_t)1 << 27, std::min<int64_t>(S, SKM_CSC_MAX_COLS) + 1);
+    cub::DeviceScan::InclusiveSum(nullptr, t_scan, (const int64_t *)nullptr, (int64_t *)nullptr, scan_n);
     return 4 * align256(size_t(nnz) * 8) + align256(size_t(n_ann) * 8) + align256(std::max(t_sort, t_scan)) + 1024;
 }
+
+size_t skm_csc_build_workspace(int64_t nnz, int64_t n_ann) { return skm_csc_build_workspace_cols(nnz, n_ann, SKM_DENSE_MAX_SPACE); }
 
 int skm_csc_build(const uint64_t *d_keys, const int64_t *d_vals, int64_t nnz, int64_t S, int64_t n_ann,
                   int64_t *d_colptr, int32_t *d_rows, int32_t *d_mvals, double *d_mnorm2, float *d_inv_m32,
                   int64_t *d_max_m, void *workspace, size_t workspace_bytes, skm_stream_t stream) {
     using namespace skm;
-    if (nnz < 0 || S <= 0 || S > SKM_DENSE_MAX_SPACE || n_ann < 0 || !d_colptr) { set_error("skm_csc_build: bad arguments"); return SKM_ERR_INVALID; }
+    if (nnz < 0 || S <= 0 || S > SKM_CSC_MAX_COLS || n_ann < 0 || !d_colptr) { set_error("skm_csc_build: bad arguments"); return SKM_ERR_INVALID; }
     cudaStream_t st = (cudaStream_t)stream;
     SKM_CUDA_TRY(cudaMemsetAsync(d_colptr, 0, size_t(S + 1) * 8, st));
     if (d_mnorm2 && n_ann > 0) SKM_CUDA_TRY(cudaMemsetAsync(d_mnorm2, 0, size_t(n_ann) * 8, st));
@@ -975,7 +1084,7 @@ int skm_csc_build(const uint64_t *d_keys, const int64_t *d_vals, int64_t nnz, in
     if (d_max_m) SKM_CUDA_TRY(cudaMemsetAsync(d_max_m, 0, 8, st));
     if (nnz == 0) return SKM_OK;
     if (!d_keys || !d_vals || !d_rows || !d_mvals || !d_max_m) { set_error("skm_csc_build: NULL argument"); return SKM_ERR_INVALID; }
-    const size_t need = skm_csc_build_workspace(nnz, n_ann);
+    const size_t need = skm_csc_build_workspace_cols(nnz, n_ann, S);
     if (!workspace || workspace_bytes < need) { set_error("skm_csc_build: workspace %zu < %zu", workspace_bytes, need); return SKM_ERR_WORKSPACE; }
     char *p = reinterpret_cast<char *>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
     const size_t seg = align256(size_t(nnz) * 8);

@@ -1187,7 +1187,7 @@ def csc_build(keys: torch.Tensor, vals: torch.Tensor, S: int, n_ann: int, ann_lo
         keys = (keys[i0:i1] - ann_lo * S).contiguous()
         vals = vals[i0:i1].contiguous()
     nnz = keys.numel()
-    ws_bytes = lib().skm_csc_build_workspace(nnz, n_ann)
+    ws_bytes = lib().skm_csc_build_workspace_cols(nnz, n_ann, int(S))
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
     colptr = torch.empty(S + 1, dtype=torch.int64, device=dev)
     rows = torch.empty(max(nnz, 1), dtype=torch.int32, device=dev)
@@ -1444,6 +1444,71 @@ def _csr_by_chunks(batch: SequenceBatch, max_chunk_res: int, dtypes, count):
                 *(None if dt is None else torch.zeros(0, dtype=dt, device=dev) for dt in dtypes))
     cat = (lambda xs: xs[0] if len(xs) == 1 else torch.cat(xs))
     return (cat(rowptrs), *(None if xs[0] is None else cat(list(xs)) for xs in zip(*parts)))
+
+
+def learn_wide(batch: SequenceBatch, alphabet: AlphabetT, k: int, basis: WideBasis, ann_id: torch.Tensor, n_ann: int,
+               max_chunk_res: int = WIDE_MAX_CHUNK_RES) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """learn_sparse_with_totals for any nsym^k <= 2^64 - 1, with the matrix keyed by BASIS COLUMN:
+    -> (keys int64 [nnz] sorted, key = ann * K + col; vals int64 [nnz]; totals int64 [K]: occurrences of every basis
+    column over ALL sequences, learn.smk:380).  Windows outside the basis count nowhere.  Sequences with ann_id
+    outside [0, n_ann) go to a rest row that only feeds the Totals (skm_learn_wide)."""
+    tab = alphabet_tables(alphabet, batch.device)
+    dev = batch.device
+    ann_id = ann_id.to(device=dev, dtype=torch.int32).contiguous()
+    assert ann_id.numel() == batch.n
+    K, n_ann = int(basis.K), int(n_ann)
+    if (n_ann + 2) * K >= 2 ** 63:
+        raise SkmError(-3, f"learn_wide: (n_ann + 2) * K = {(n_ann + 2) * K} does not fit 63 bits")
+    parts_k, parts_v = [], []
+    for lo, hi in _chunks_by_residues(batch.offsets_host, max_chunk_res):
+        sub = batch if (lo == 0 and hi == batch.n) else _sub_batch(batch, lo, hi)
+        ws_bytes = lib().skm_learn_wide_workspace(sub.nres)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        ok = torch.empty(max(sub.nres, 1), dtype=torch.int64, device=dev)
+        ov = torch.empty(max(sub.nres, 1), dtype=torch.int64, device=dev)
+        dn = torch.zeros(1, dtype=torch.int64, device=dev)
+        check(lib().skm_learn_wide(_ptr(sub.residues), sub.nres, _ptr(sub.offsets), sub.n, _ptr(tab.lut), tab.nsym, int(k),
+                                   _ptr(ann_id[lo:hi]), n_ann, _ptr(basis.sorted_codes), _ptr(basis.col_of_sorted), K,
+                                   _ptr(ok), _ptr(ov), _ptr(dn), _ptr(ws), ws_bytes, _stream()))
+        m = int(dn.item())
+        parts_k.append(ok[:m].clone())
+        parts_v.append(ov[:m].clone())
+        del ws, ok, ov
+    if not parts_k:
+        keys = vals = torch.zeros(0, dtype=torch.int64, device=dev)
+    elif len(parts_k) == 1:
+        keys, vals = parts_k[0], parts_v[0]
+    else:
+        keys, vals = coo_merge_runs(torch.cat(parts_k), torch.cat(parts_v), [p.numel() for p in parts_k])
+    totals = torch.zeros(max(K, 1), dtype=torch.int64, device=dev)
+    if keys.numel():
+        check(lib().skm_coo_colsum(_ptr(keys), _ptr(vals), keys.numel(), K, _ptr(totals), _stream()))
+    m = int(torch.searchsorted(keys, torch.tensor([n_ann * K], dtype=torch.int64, device=dev)).item()) if keys.numel() else 0
+    return keys[:m], vals[:m], totals[:K]
+
+
+def query_csr_wide(batch: SequenceBatch, alphabet: AlphabetT, k: int, basis: WideBasis,
+                   restrict: Optional[WideBasis] = None) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Queries for apply against a matrix keyed by the columns of `basis`: (rowptr int64 [N+1], cols int32, vals int32)
+    over EVERY valid window (the query norm runs over all of them, apply.smk:268-276).  An entry the basis does not hold
+    gets the empty column K: it adds to the norm and to no dot.  restrict: keep only the codes this basis holds (the
+    query file's own kmerlist, apply.smk:262-289)."""
+    rowptr, codes, _, vals = count_csr_wide(batch, alphabet, k)
+    if restrict is not None:
+        keep = codes_to_columns(codes, restrict) >= 0
+        csum = torch.zeros(keep.numel() + 1, dtype=torch.int64, device=codes.device)
+        torch.cumsum(keep, 0, out=csum[1:])
+        rowptr, codes, vals = csum[rowptr], codes[keep].contiguous(), vals[keep].contiguous()
+    cols = codes_to_columns(codes, basis)
+    cols = torch.where(cols < 0, torch.full_like(cols, basis.K), cols)
+    return rowptr, cols, vals
+
+
+def apply_wide(rowptr: torch.Tensor, cols: torch.Tensor, vals: torch.Tensor, keys: torch.Tensor, mvals: torch.Tensor, K: int,
+               n_ann: int, tile: Optional[int] = None) -> ApplyResult:
+    """apply_sparse_tiled for a matrix keyed by basis column (learn_wide, key = ann * K + col) and queries from
+    query_csr_wide: the matrix is re-keyed to the stride K + 1, whose last column is the empty one."""
+    return apply_sparse_tiled(rowptr, cols, vals, keys + keys // K if K else keys, mvals, K + 1, n_ann, tile)
 
 
 def build_basis_wide_distributed(batch: SequenceBatch, alphabet, k: int, min_filter: int = 0,

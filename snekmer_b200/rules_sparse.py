@@ -13,6 +13,9 @@ Row / column conventions are the reference's: annotation rows in order of first 
 sequences, a repeated sequence id keeps its first position and last value, the query norm runs over all valid windows of
 the query (its own k-mer list), ties go to the lowest annotation index.  ``sidecar.export_counts_csv`` /
 ``export_totals_csv`` turn a side-car back into the reference's CSV when the matrix is small enough to be one.
+
+Code spaces beyond the tables (``len(symbols)^k > 2^27``) are keyed by basis column instead of code: the matrix carries
+its column table (``SparseCounts.columns``), the k-mers that occur in first-occurrence order (engine.learn_wide).
 """
 from __future__ import annotations
 
@@ -29,19 +32,30 @@ from .rules import _ACCESSION, ScoreResult, _unique_last, _write_arrow_csv, delt
 
 @dataclass
 class SparseCounts:
-    """A learned count matrix on the device: sorted COO keys ``ann * S + code`` over the reduced alphabet ``symbols``."""
+    """A learned count matrix on the device: sorted COO keys ``ann * S + code`` over the reduced alphabet ``symbols``,
+    or, with a column table (code spaces beyond 2^27), ``ann * K + col`` over the K columns of ``columns``."""
     annotations: List[str]
     seq_count: np.ndarray           # int64 [A]
     symbols: str
     k: int
     keys: torch.Tensor              # int64 [nnz], sorted
     vals: torch.Tensor              # int64 [nnz]
-    totals: torch.Tensor            # int64 [S]: occurrences over ALL sequences
+    totals: torch.Tensor            # int64 [S] (or [K] with columns): occurrences over ALL sequences
     total_seqs: int
+    columns: Optional[E.WideBasis] = None   # column table: column j holds the k-mer code columns.codes[j]
 
     @property
     def S(self) -> int:
         return len(self.symbols) ** self.k
+
+    @property
+    def stride(self) -> int:
+        """Key stride: S, or the number of columns K of a matrix keyed by column."""
+        return self.S if self.columns is None else self.columns.K
+
+
+def _wide(symbols: str, k: int) -> bool:
+    return len(symbols) ** int(k) > E._native.SKM_DENSE_MAX_SPACE
 
 
 def annotation_ids(ids: Sequence[str], seq_annot: Dict[str, str]):
@@ -74,6 +88,11 @@ def learn_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], symbols
     tab = E.alphabet_tables_from_symbols(symbols)
     batch = E.SequenceBatch.from_strings([str(s) for s in reduced_seqs])
     ann_id, annotations, seq_count, total = annotation_ids(ids, seq_annot)
+    if _wide(tab.symbols, k):
+        # columns: every k-mer that occurs, in first-occurrence order (the wide analogue of "every code")
+        columns = E.build_basis_wide(batch, tab, int(k), 0)
+        keys, vals, totals = E.learn_wide(batch, tab, int(k), columns, torch.from_numpy(ann_id), len(annotations))
+        return SparseCounts(annotations, seq_count, tab.symbols, int(k), keys, vals, totals, total, columns)
     keys, vals, totals = E.learn_sparse_with_totals(batch, tab, int(k), torch.from_numpy(ann_id), len(annotations))
     return SparseCounts(annotations, seq_count, tab.symbols, int(k), keys, vals, totals, total)
 
@@ -81,9 +100,26 @@ def learn_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], symbols
 def write_counts_sidecar(path: str, sc: SparseCounts, kmers: Optional[Sequence[str]] = None) -> None:
     """``.skmc`` of a learned matrix: rows ``Totals`` + annotations, columns = `kmers` (default: the k-mers that occur, in
     code order; pass the vectorize rule's kmerlist to get the reference's column order), CSR values."""
-    S = sc.S
+    S = sc.stride
     totals = sc.totals.cpu().numpy()
-    if kmers is None:
+    # col_of_code: file column of every key % S (a code, or a learned column when the matrix has a column table)
+    if sc.columns is not None:
+        learned = sc.columns.codes_host()
+        col_of_code = np.full(S, -1, dtype=np.int64)
+        if kmers is None:
+            occ = np.flatnonzero(totals)
+            kmers = list(E.decode_kmers(learned[occ], sc.symbols, sc.k))
+            col_of_code[occ] = np.arange(len(occ))
+        else:
+            kmers = [str(x) for x in kmers]
+            codes, ok = E.encode_kmers(kmers, sc.symbols, sc.k)
+            fcol = np.flatnonzero(ok)
+            order = np.argsort(codes[fcol], kind="stable")
+            fcodes = codes[fcol][order]
+            j = np.minimum(np.searchsorted(fcodes, learned), max(len(fcodes) - 1, 0))
+            hit = (fcodes[j] == learned) if len(fcodes) else np.zeros(len(learned), dtype=bool)
+            col_of_code[hit] = fcol[order][j[hit]]
+    elif kmers is None:
         codes = np.flatnonzero(totals).astype(np.uint64)
         kmers = list(E.decode_kmers(codes, sc.symbols, sc.k))
         col_of_code = np.full(S, -1, dtype=np.int64)
@@ -119,38 +155,48 @@ def write_counts_sidecar(path: str, sc: SparseCounts, kmers: Optional[Sequence[s
 
 
 def read_counts_sidecar(path: str, symbols: Optional[str] = None) -> SparseCounts:
-    """``.skmc`` -> device COO.  The reduced alphabet is the set of characters of the k-mer columns unless given."""
+    """``.skmc`` -> device COO.  The reduced alphabet is the set of characters of the k-mer columns unless given.  In a
+    code space beyond 2^27 the matrix is keyed by column: the file's k-mers (those of the alphabet) in file order."""
     d = sidecar.read_counts_csr(path)
     kmers = d["kmers"]
     if not d["rows"] or d["rows"][0] != "Totals":
         raise ValueError(f"{path}: a counts table starts with its Totals row")
     k = len(kmers[0]) if kmers else 1
     symbols = "".join(sorted(set("".join(kmers)))) if symbols is None else "".join(sorted(set(symbols)))
-    S = len(symbols) ** k
     codes, ok = E.encode_kmers(kmers, symbols, k)
     dev = E._require_cuda()
+    columns = None
+    if _wide(symbols, k):
+        columns = E.wide_basis_from_codes(codes[ok], E.alphabet_tables_from_symbols(symbols, dev), k, dev)
+        key_of_col = np.cumsum(ok) - 1                   # file column -> learned column
+        S = columns.K
+    else:
+        key_of_col = codes.astype(np.int64)
+        S = len(symbols) ** k
     rowptr, cols, vals = d["rowptr"], d["cols"].astype(np.int64), d["vals"]
     rows = np.repeat(np.arange(len(d["rows"])), np.diff(rowptr))
     good = ok[cols]
     totals = np.zeros(S, dtype=np.int64)
     t = (rows == 0) & good
-    totals[codes[cols[t]].astype(np.int64)] = vals[t]
+    totals[key_of_col[cols[t]]] = vals[t]
     m = (rows > 0) & good
-    keys = (rows[m] - 1).astype(np.int64) * S + codes[cols[m]].astype(np.int64)
+    keys = (rows[m] - 1).astype(np.int64) * S + key_of_col[cols[m]]
     order = np.argsort(keys, kind="stable")
     return SparseCounts(list(d["rows"][1:]), d["seq_count"][1:].astype(np.int64), symbols, k,
                         torch.from_numpy(keys[order]).to(dev), torch.from_numpy(vals[m][order].astype(np.int64)).to(dev),
-                        torch.from_numpy(totals).to(dev), int(d["seq_count"][0]))
+                        torch.from_numpy(totals).to(dev), int(d["seq_count"][0]), columns)
 
 
 def merge_counts_sparse(parts: Sequence[SparseCounts]) -> SparseCounts:
     """Merge.merge_dataframes (learn.smk:467-494): outer join on the annotation rows (first appearance), element-wise sum."""
     assert parts and all(p.symbols == parts[0].symbols and p.k == parts[0].k for p in parts), "same reduced alphabet and k"
-    S = parts[0].S
     index: Dict[str, int] = {}
     for p in parts:
         for a in p.annotations:
             index.setdefault(a, len(index))
+    if parts[0].columns is not None:
+        return _merge_wide(parts, index)
+    S = parts[0].S
     seq_count = np.zeros(len(index), dtype=np.int64)
     ks, vs = [], []
     totals = torch.zeros_like(parts[0].totals)
@@ -164,6 +210,36 @@ def merge_counts_sparse(parts: Sequence[SparseCounts]) -> SparseCounts:
         total_seqs += p.total_seqs
     keys, vals = E.coo_merge(torch.cat(ks), torch.cat(vs), key_bound=len(index) * S)
     return SparseCounts(list(index), seq_count, parts[0].symbols, parts[0].k, keys, vals, totals, total_seqs)
+
+
+def _merge_wide(parts: Sequence[SparseCounts], index: Dict[str, int]) -> SparseCounts:
+    """merge_counts_sparse of matrices keyed by column: the union of the columns in first-appearance order (the first
+    part's columns, then each later part's new ones: learn.smk:467-494), every part re-keyed onto it, summed."""
+    assert all(p.columns is not None for p in parts), "all parts keyed by column"
+    tab = E.alphabet_tables_from_symbols(parts[0].symbols)
+    codes = torch.cat([p.columns.codes for p in parts])
+    n = codes.numel()
+    dev = codes.device
+    union = E.basis_table_finalize(tab, parts[0].k, codes, torch.ones(n, dtype=torch.int64, device=dev),
+                                   torch.arange(n, dtype=torch.int64, device=dev), merged=False, min_filter=0, first_bound=n)
+    KU = union.K
+    seq_count = np.zeros(len(index), dtype=np.int64)
+    ks, vs = [], []
+    totals = torch.zeros(KU, dtype=torch.int64, device=dev)
+    total_seqs = 0
+    for p in parts:
+        Kp = p.columns.K
+        col = E.codes_to_columns(p.columns.codes, union).to(torch.int64)
+        remap = torch.tensor([index[a] for a in p.annotations] + [0], dtype=torch.int64, device=dev)
+        if Kp:
+            ks.append(remap[p.keys // Kp] * KU + col[p.keys % Kp])
+            vs.append(p.vals)
+            totals.index_add_(0, col, p.totals)
+        np.add.at(seq_count, [index[a] for a in p.annotations], p.seq_count)
+        total_seqs += p.total_seqs
+    keys, vals = (E.coo_merge(torch.cat(ks), torch.cat(vs), key_bound=len(index) * KU) if ks
+                  else (torch.zeros(0, dtype=torch.int64, device=dev),) * 2)
+    return SparseCounts(list(index), seq_count, parts[0].symbols, parts[0].k, keys, vals, totals, total_seqs, union)
 
 
 def restrict_csr_to_kmers(rowptr: torch.Tensor, cols: torch.Tensor, vals: torch.Tensor, symbols: str, k: int,
@@ -194,11 +270,19 @@ def apply_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], sc: Spa
     seqs = [str(reduced_seqs[int(i)]) for i in pick]
     tab = E.alphabet_tables_from_symbols(sc.symbols)
     batch = E.SequenceBatch.from_strings(seqs)
-    rowptr, cols, cvals = E.count_csr(batch, tab, sc.k, None)
-    if query_kmers is not None:
-        rowptr, cols, cvals = restrict_csr_to_kmers(rowptr, cols, cvals, tab.symbols, sc.k, query_kmers)
     A = len(sc.annotations)
-    r = E.apply_sparse_tiled(rowptr, cols, cvals, sc.keys, sc.vals, sc.S, A, tile)
+    if sc.columns is not None:
+        restrict = None
+        if query_kmers is not None:
+            qcodes, ok = E.encode_kmers([str(x) for x in query_kmers], tab.symbols, sc.k)
+            restrict = E.wide_basis_from_codes(np.unique(qcodes[ok]), tab, sc.k, batch.device)
+        rowptr, cols, cvals = E.query_csr_wide(batch, tab, sc.k, sc.columns, restrict)
+        r = E.apply_wide(rowptr, cols, cvals, sc.keys, sc.vals, sc.columns.K, A, tile)
+    else:
+        rowptr, cols, cvals = E.count_csr(batch, tab, sc.k, None)
+        if query_kmers is not None:
+            rowptr, cols, cvals = restrict_csr_to_kmers(rowptr, cols, cvals, tab.symbols, sc.k, query_kmers)
+        r = E.apply_sparse_tiled(rowptr, cols, cvals, sc.keys, sc.vals, sc.S, A, tile)
     top1, top2 = r.top1.cpu().numpy(), r.top2.cpu().numpy()
     s1, s2 = r.score1.cpu().numpy(), r.score2.cpu().numpy()
     if out_summary:
