@@ -490,6 +490,16 @@ SKM_API int skm_top2_rows_f64(const double *d_scores, int64_t nq, int64_t n_ann,
 SKM_API int skm_confidence_hist(const int32_t *d_top1, const double *d_score1, const double *d_score2,
                         const uint8_t *d_class, int64_t nq, int64_t n_ann, int64_t *d_hist_true,
                         int64_t *d_hist_false, uint8_t *d_bin_out, skm_stream_t stream);
+/* The d_class input of skm_confidence_hist for the rows of eval_apply (learn.smk:712-732), decided as
+ * learn.smk:997-1008 decides it on the row label, without building the labels.  Row q is labelled
+ * name[truth[q]] + "_known_" + decimal(row_base + q), or `<accession>_unknown_<n>` when truth[q] < 0.
+ * Name table: UTF-8 bytes d_names, offsets int64 [n_names + 1]; entries 0 .. A-1 are the matrix's annotations
+ * (the indices of d_top1), the rest any further names truth refers to.  d_class uint8 [nq]: 0 when the label
+ * contains "unknown", else 1 when top1 >= 0 and name[top1] is a byte substring of the label, else 2.  An
+ * index outside [0, n_names) names nothing.  row_base >= 0, row_base + nq <= 2^63 - 1. */
+SKM_API int skm_confidence_classify(const int32_t *d_top1, const int32_t *d_truth, int64_t nq, int64_t row_base,
+                            const uint8_t *d_names, const int64_t *d_name_offsets, int64_t n_names,
+                            uint8_t *d_class, skm_stream_t stream);
 
 /* ---- FASTA ingest (host cores, no device work): Bio.SeqIO.parse(f, "fasta") as kmerize.smk:90-129 uses it ----
  * text = the (decompressed) file in host memory.  A record starts at a '>' in column 0; id = the title up to its

@@ -87,6 +87,7 @@ SIGNATURES = {
     "skm_top2_merge": (_int, [_p, _p, _i64, _i64, _p, _p, _p, _p, _p]),
     "skm_top2_rows_f64": (_int, [_p, _i64, _i64, _p, _p, _p, _p, _p]),
     "skm_confidence_hist": (_int, [_p, _p, _p, _p, _i64, _i64, _p, _p, _p, _p]),
+    "skm_confidence_classify": (_int, [_p, _p, _i64, _i64, _p, _p, _i64, _p, _p]),
     "skm_fasta_scan": (_int, [_p, _i64, _int, C.POINTER(_i64), C.POINTER(_i64), C.POINTER(_i64)]),
     "skm_fasta_pack": (_int, [_p, _i64, _int, _p, _p, _p, _p]),
     "skm_row_norm2_i32": (_int, [_p, _i64, _i64, _p, _p]),

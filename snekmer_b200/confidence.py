@@ -7,10 +7,12 @@ the apply rule looks up (apply.smk:301-335).
 
 Here the per-row work (top-2 of a score matrix, Difference bins, the two histograms) runs on the device
 (``skm_top2_rows_f64``, ``skm_confidence_hist``); when the scores come straight from ``engine.apply_*`` the
-Q x A matrix never exists.  What stays on the host is what the reference decides with string tests on the row
-label (T iff the predicted name is a substring of the label, Known iff the label lacks "unknown",
-learn.smk:997-1008) and the 101-point curve arithmetic (float64, same operation order as the reference).
-Multi-GPU: histograms are summed with one all_reduce.
+Q x A matrix never exists.  The reference decides a row's class with string tests on its label (T iff the predicted
+name is a substring of the label, Known iff the label lacks "unknown", learn.smk:997-1008): ``classify_rows`` does
+that on the host for labels read from a file; for the rows of eval_apply, whose labels are built from the annotation
+name and the row number, ``skm_confidence_classify`` does it on the device from a name table (``add_device``).  The
+101-point curve arithmetic stays on the host (float64, same operation order as the reference).
+Multi-GPU: histograms are summed with one all_reduce (dist.allreduce_confidence_tables).
 """
 from __future__ import annotations
 
@@ -20,7 +22,9 @@ from typing import Dict, List, Optional, Sequence
 import numpy as np
 import torch
 
+from . import dist as D
 from . import engine as E
+from .sidecar import _strings_to_arrays
 from ._native import check, lib
 
 NBINS = 101
@@ -79,6 +83,47 @@ def classify_rows(pred: np.ndarray, labels: Sequence[str], annotations: Sequence
     return cls
 
 
+def joint_name_table(annotations: Sequence[str], names: Sequence[Optional[str]]):
+    """(table, index int32 [len(names)]): the name table of ``skm_confidence_classify`` — the matrix's annotations
+    in matrix order, then every other name of `names` once, in order of first appearance — and the entry of each of
+    `names` in it (-1 for None: an ``_unknown_`` row)."""
+    table = [str(a) for a in annotations]
+    index: Dict[str, int] = {}
+    for i, a in enumerate(table):
+        index.setdefault(a, i)
+    idx = np.full(len(names), -1, dtype=np.int32)
+    for j, n in enumerate(names):
+        if n is None:
+            continue
+        n = str(n)
+        i = index.get(n)
+        if i is None:
+            i = index[n] = len(table)
+            table.append(n)
+        idx[j] = i
+    return table, idx
+
+
+def classify_device(top1: torch.Tensor, truth: torch.Tensor, row_base: int, names: Sequence[str]) -> torch.Tensor:
+    """uint8 [Q], the classes of ``classify_rows`` for the eval_apply labels ``names[truth[q]]_known_<row_base + q>``
+    (``<accession>_unknown_<n>`` where truth[q] < 0), without the labels.  top1 indexes the first A entries of
+    `names` (joint_name_table)."""
+    dev = E._require_cuda(top1.device)
+    nq = top1.numel()
+    assert truth.numel() == nq
+    buf, off = _strings_to_arrays(names)
+    d_buf = torch.from_numpy(buf.copy()).to(dev) if buf.size else None
+    d_off = torch.from_numpy(off).to(dev)
+    cls = torch.empty(nq, dtype=torch.uint8, device=dev)
+    check(lib().skm_confidence_classify(E._ptr(top1.to(dev, torch.int32).contiguous()), E._ptr(truth.to(dev, torch.int32).contiguous()),
+                                        nq, int(row_base), E._ptr(d_buf), E._ptr(d_off), len(names), E._ptr(cls), E._stream()))
+    return cls
+
+
+# zero-bin key of a rank with no qualifying row (dist.allreduce_confidence_tables takes the minimum)
+NO_ZERO_ROW = np.iinfo(np.int64).max
+
+
 @dataclass
 class EvalResult:
     rows: List[str]                 # sorted names of the predictions that occur among Known rows
@@ -129,6 +174,35 @@ class ConfidenceAccumulator:
             if z.size:
                 i = int(z[0])
                 self.zero_negative = bool(result.score1[i].item() == result.score2[i].item())
+        self._files += 1
+        self.add_histograms(ht.cpu().numpy(), hf.cpu().numpy(), annotations)
+
+    def add_device(self, result: E.ApplyResult, truth: torch.Tensor, row_base: int, names: Sequence[str],
+                   annotations: Sequence[str]) -> None:
+        """One eval_apply file (or one rank's contiguous rows of it) with the classes decided on the device
+        (classify_device): row q is global row ``row_base + q``, labelled from ``names[truth[q]]``; `names` starts with
+        the A `annotations` that result.top1 indexes.  With several ranks every rank calls this for every file: the
+        histograms are summed over ranks and the zero-bin label comes from the lowest global row that qualifies."""
+        dev = E._require_cuda(result.top1.device)
+        a, nq = len(annotations), result.top1.numel()
+        top1 = result.top1.contiguous()
+        cls = classify_device(top1, truth, row_base, names)
+        ht = torch.zeros((max(a, 1), NBINS), dtype=torch.int64, device=dev)
+        hf = torch.zeros((max(a, 1), NBINS), dtype=torch.int64, device=dev)
+        bins = torch.empty(max(nq, 1), dtype=torch.uint8, device=dev)
+        s1, s2 = result.score1.contiguous(), result.score2.contiguous()
+        check(lib().skm_confidence_hist(E._ptr(top1), E._ptr(s1), E._ptr(s2), E._ptr(cls), nq, a, E._ptr(ht), E._ptr(hf),
+                                        E._ptr(bins), E._stream()))
+        # zero-bin label (see add): key 2 * row + (exact tie) of the first Known & True row in bin 0
+        zero = torch.full((1,), NO_ZERO_ROW, dtype=torch.int64, device=dev)
+        if self._files == 0 and nq:
+            key = (torch.arange(nq, dtype=torch.int64, device=dev) + int(row_base)) * 2 + (s1 == s2)
+            zero = torch.where((cls == 1) & (bins[:nq] == 0), key, zero).min().reshape(1)
+        D.allreduce_confidence_tables(ht, hf, zero)
+        if self._files == 0:
+            z = int(zero.item())
+            if z != NO_ZERO_ROW:
+                self.zero_negative = bool(z & 1)
         self._files += 1
         self.add_histograms(ht.cpu().numpy(), hf.cpu().numpy(), annotations)
 

@@ -13,6 +13,8 @@ has exactly three exchange steps, each a plain collective on integer / top-2 buf
   apply   (apply.smk:312-335)    when the annotation matrix is row-(annotation-)sharded:
                                  all_gather of per-shard (top1, top2, score1, score2) and a
                                  2-way merge — top-2, not top-1: delta needs the runner-up
+  evaluate (learn.smk:1052-1110) training rows sharded, matrix replicated: all_reduce(SUM) of
+                                 the True / False crosstabs, all_reduce(MIN) of the zero-bin key
 
 encode / count / apply-with-replicated-M need no collective (weak scaling).
 Every function works on whatever device the tensors live on, so the collective
@@ -106,6 +108,16 @@ def allreduce_sum_(*tensors: torch.Tensor) -> None:
         return
     for t in tensors:
         dist.all_reduce(t, op=dist.ReduceOp.SUM)
+
+
+def allreduce_confidence_tables(hist_true: torch.Tensor, hist_false: torch.Tensor, zero_key: torch.Tensor) -> None:
+    """Evaluate fan-in over ranks that scored disjoint rows of one file, in place: the int64 [A, 101] crosstabs are
+    summed; zero_key (int64 [1], 2 * global row + exact-tie flag of a rank's first Known & True row in the zero bin,
+    INT64_MAX for none) becomes the minimum, i.e. the lowest such row of the file."""
+    if world()[1] == 1:
+        return
+    allreduce_sum_(hist_true, hist_false)
+    dist.all_reduce(zero_key, op=dist.ReduceOp.MIN)
 
 
 def exclusive_prefix(value: int, device=None) -> Tuple[int, int]:

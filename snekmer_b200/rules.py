@@ -520,6 +520,14 @@ def evaluate_results(results: Sequence[ScoreResult], out_conf: Optional[str] = N
                             torch.from_numpy(np.ascontiguousarray(r.score1, dtype=np.float64)).to(dev),
                             torch.from_numpy(np.ascontiguousarray(r.score2, dtype=np.float64)).to(dev))
         acc.add(res, r.rows, r.annotations)
+    return _write_evaluation(acc, out_conf, out_glob, base_confidence, modifier)
+
+
+def _write_evaluation(acc, out_conf: Optional[str], out_glob: Optional[str], base_confidence: Sequence[str], modifier: float):
+    """The end of Evaluator.execute_all: the curve of the accumulated crosstabs, merged with ONE prior
+    global-confidence file when given, and the two files."""
+    from . import confidence as CF
+
     prior = CF.read_global_confidence(str(base_confidence[0])) if len(base_confidence) == 1 else None
     out = acc.finalize(prior, modifier)
     if out_glob:

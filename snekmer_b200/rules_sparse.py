@@ -7,6 +7,9 @@ binary ``.skmc`` side-car (sidecar.py) as the file between them:
 
   learn_counts_sparse   Library (learn.smk:306-408)      -> COO matrix + Totals on the device
   merge_counts_sparse   Merge (learn.smk:467-494)        -> outer join on annotations, sum (skm_coo_merge)
+  eval_counts_sparse    KmerCompare of learn (learn.smk:628-887) -> SpMM cosine, top-2 + each row's annotation
+                        (EvalScores; the ``.skme`` side-car in place of seq-annotation-scores-*.csv)
+  evaluate_sparse       Evaluator (learn.smk:923-1348)   -> row classes and crosstabs on the device, the confidence files
   apply_counts_sparse   KmerCompare (apply.smk:224-342)  -> SpMM cosine, top-2, delta, Confidence
 
 Row / column conventions are the reference's: annotation rows in order of first appearance, ``Totals`` over ALL
@@ -25,9 +28,12 @@ from typing import Dict, List, Optional, Sequence
 import numpy as np
 import torch
 
+from . import confidence as CF
+from . import dist as D
 from . import engine as E
 from . import sidecar
-from .rules import _ACCESSION, ScoreResult, _unique_last, _write_arrow_csv, delta_and_confidence, read_confidence_csv
+from .rules import (_ACCESSION, ScoreResult, _unique_last, _write_arrow_csv, _write_evaluation, delta_and_confidence,
+                    read_confidence_csv)
 
 
 @dataclass
@@ -257,6 +263,25 @@ def restrict_csr_to_kmers(rowptr: torch.Tensor, cols: torch.Tensor, vals: torch.
     return csum[rowptr], cols[keep].contiguous(), vals[keep].contiguous()
 
 
+def _score_sparse(seqs: Sequence[str], sc: SparseCounts, tile: Optional[int], query_kmers: Optional[Sequence[str]]) -> E.ApplyResult:
+    """Cosine of every sequence against every annotation row of `sc` as SpMM, top-2 on the device (see
+    apply_counts_sparse for `query_kmers` and `tile`)."""
+    tab = E.alphabet_tables_from_symbols(sc.symbols)
+    batch = E.SequenceBatch.from_strings(list(seqs))
+    A = len(sc.annotations)
+    if sc.columns is not None:
+        restrict = None
+        if query_kmers is not None:
+            qcodes, ok = E.encode_kmers([str(x) for x in query_kmers], tab.symbols, sc.k)
+            restrict = E.wide_basis_from_codes(np.unique(qcodes[ok]), tab, sc.k, batch.device)
+        rowptr, cols, cvals = E.query_csr_wide(batch, tab, sc.k, sc.columns, restrict)
+        return E.apply_wide(rowptr, cols, cvals, sc.keys, sc.vals, sc.columns.K, A, tile)
+    rowptr, cols, cvals = E.count_csr(batch, tab, sc.k, None)
+    if query_kmers is not None:
+        rowptr, cols, cvals = restrict_csr_to_kmers(rowptr, cols, cvals, tab.symbols, sc.k, query_kmers)
+    return E.apply_sparse_tiled(rowptr, cols, cvals, sc.keys, sc.vals, sc.S, A, tile)
+
+
 def apply_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], sc: SparseCounts, confidence_csv: Optional[str] = None,
                         out_summary: Optional[str] = None, tile: Optional[int] = None,
                         query_kmers: Optional[Sequence[str]] = None) -> ScoreResult:
@@ -268,21 +293,8 @@ def apply_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], sc: Spa
     accumulator width the data needs (engine.apply_sparse_tiled)."""
     uniq, pick = _unique_last(list(ids))
     seqs = [str(reduced_seqs[int(i)]) for i in pick]
-    tab = E.alphabet_tables_from_symbols(sc.symbols)
-    batch = E.SequenceBatch.from_strings(seqs)
     A = len(sc.annotations)
-    if sc.columns is not None:
-        restrict = None
-        if query_kmers is not None:
-            qcodes, ok = E.encode_kmers([str(x) for x in query_kmers], tab.symbols, sc.k)
-            restrict = E.wide_basis_from_codes(np.unique(qcodes[ok]), tab, sc.k, batch.device)
-        rowptr, cols, cvals = E.query_csr_wide(batch, tab, sc.k, sc.columns, restrict)
-        r = E.apply_wide(rowptr, cols, cvals, sc.keys, sc.vals, sc.columns.K, A, tile)
-    else:
-        rowptr, cols, cvals = E.count_csr(batch, tab, sc.k, None)
-        if query_kmers is not None:
-            rowptr, cols, cvals = restrict_csr_to_kmers(rowptr, cols, cvals, tab.symbols, sc.k, query_kmers)
-        r = E.apply_sparse_tiled(rowptr, cols, cvals, sc.keys, sc.vals, sc.S, A, tile)
+    r = _score_sparse(seqs, sc, tile, query_kmers)
     top1, top2 = r.top1.cpu().numpy(), r.top2.cpu().numpy()
     s1, s2 = r.score1.cpu().numpy(), r.score2.cpu().numpy()
     if out_summary:
@@ -293,3 +305,73 @@ def apply_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], sc: Spa
         _write_arrow_csv(out_summary, {"index": uniq, "Prediction": [str(sc.annotations[i]) for i in top1], "Score": s1,
                                        "delta": delta, "Confidence": pa.array(confidence, from_pandas=True)})
     return ScoreResult(uniq, list(sc.annotations), top1, top2, s1, s2, None)
+
+
+@dataclass
+class EvalScores:
+    """eval_apply of one training file on the sparse path: top-2 of every row on the device and, in place of the row
+    label ``<annotation>_known_<n>`` / ``<accession>_unknown_<n>`` (learn.smk:712-732), its parts — the entry of
+    `names` it was built from (`truth`, -1 for an unknown row) and n = row_base + row.  `names` starts with the
+    matrix's `annotations` (the columns top1 / top2 index), then the file's other annotation names."""
+    annotations: List[str]
+    names: List[str]
+    top1: torch.Tensor              # int32 [Q]
+    top2: torch.Tensor              # int32 [Q]
+    score1: torch.Tensor            # float64 [Q]
+    score2: torch.Tensor            # float64 [Q]
+    truth: torch.Tensor             # int32 [Q]
+    row_base: int
+
+    def result(self) -> E.ApplyResult:
+        return E.ApplyResult(self.top1, self.top2, self.score1, self.score2)
+
+
+def eval_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], sc: SparseCounts, seq_annot: Dict[str, str],
+                       out_sidecar: Optional[str] = None, tile: Optional[int] = None,
+                       query_kmers: Optional[Sequence[str]] = None) -> EvalScores:
+    """KmerCompare of the learn workflow (learn.smk:628-887) as SpMM: the training sequences of one file against the
+    merged matrix.  Rows as eval_apply_rule: the distinct ids (a repeated id keeps its first position and last record),
+    numbered in that order; a row is known when its accession is in `seq_annot` — the caller passes the FIRST
+    annotation file only, as the rule reads only that one.  Top-2 stay on the device; `out_sidecar` writes the
+    ``.skme`` that evaluate_sparse reads.  With several ranks (matrix replicated), each passes a contiguous share of the
+    file's distinct ids, in order; row numbers continue across ranks."""
+    uniq, pick = _unique_last(list(ids))
+    dev = E._require_cuda()
+    if uniq:
+        r = _score_sparse([str(reduced_seqs[int(i)]) for i in pick], sc, tile, query_kmers)
+    else:
+        e32, e64 = torch.zeros(0, dtype=torch.int32, device=dev), torch.zeros(0, dtype=torch.float64, device=dev)
+        r = E.ApplyResult(e32, e32.clone(), e64, e64.clone())
+    accs = [_ACCESSION.findall(sid)[0] for sid in uniq]         # IndexError without two pipes, like learn.smk:714
+    names, truth = CF.joint_name_table(sc.annotations, [seq_annot[a] if a in seq_annot else None for a in accs])
+    row_base, _ = D.exclusive_prefix(len(uniq), r.top1.device)
+    ev = EvalScores(list(sc.annotations), names, r.top1, r.top2, r.score1, r.score2, torch.from_numpy(truth).to(r.top1.device),
+                    row_base)
+    if out_sidecar:
+        write_eval_sidecar(out_sidecar, ev)
+    return ev
+
+
+def write_eval_sidecar(path: str, ev: EvalScores) -> None:
+    sidecar.write_evalscores(path, ev.annotations, ev.names, ev.top1.cpu().numpy(), ev.top2.cpu().numpy(),
+                             ev.score1.cpu().numpy(), ev.score2.cpu().numpy(), ev.truth.cpu().numpy(), ev.row_base)
+
+
+def read_eval_sidecar(path: str) -> EvalScores:
+    d = sidecar.read_evalscores(path)
+    dev = E._require_cuda()
+    t = {k: torch.from_numpy(d[k]).to(dev) for k in ("top1", "top2", "score1", "score2", "truth")}
+    return EvalScores(d["annotations"], d["names"], t["top1"], t["top2"], t["score1"], t["score2"], t["truth"], d["row_base"])
+
+
+def evaluate_sparse(evals: Sequence, out_conf: Optional[str] = None, out_glob: Optional[str] = None,
+                    base_confidence: Sequence[str] = (), modifier: float = 1.0) -> CF.EvalResult:
+    """Evaluator.execute_all (learn.smk:923-1348) over eval_counts_sparse results or their ``.skme`` side-cars, in file
+    order: row classes (skm_confidence_classify) and crosstabs (skm_confidence_hist) on the device, then the same
+    curve, prior-confidence merge (ONE base file, weight `modifier`) and files as evaluate_rule."""
+    acc = CF.ConfidenceAccumulator()
+    for ev in evals:
+        if not isinstance(ev, EvalScores):
+            ev = read_eval_sidecar(str(ev))
+        acc.add_device(ev.result(), ev.truth, ev.row_base, ev.names, ev.annotations)
+    return _write_evaluation(acc, out_conf, out_glob, base_confidence, modifier)

@@ -10,6 +10,9 @@ every kernel, so the GPU path keeps
            counts as CSR (rowptr int64, cols int32, vals int32)
   *.skmc   a learned count matrix: row labels (annotations, ``Totals`` first), sequence counts, k-mer list and the
            matrix as CSR (int64 values)
+  *.skme   eval_apply scores of one training file for the evaluate rule (in place of seq-annotation-scores-*.csv):
+           the matrix's annotations, the name table of the row labels, top-2 columns and scores and the label's
+           annotation (truth) of every row, and the global number of the first row
 
 in one flat container (below), whose arrays can be memory-mapped and uploaded without parsing.  ``export_npz`` /
 ``export_counts_csv`` / ``export_totals_csv`` write exactly what the reference's rules write; ``import_counts_csv``
@@ -178,6 +181,31 @@ def read_counts_csr(path: str, mmap: bool = True) -> Dict:
     return dict(rows=_arrays_to_strings(a["rows"], a["row_offsets"]), kmers=_arrays_to_strings(a["kmers"], a["kmer_offsets"]),
                 seq_count=np.array(a["seq_count"]), kmer_count=np.array(a["kmer_count"]), rowptr=np.array(a["rowptr"]),
                 cols=np.array(a["cols"]), vals=np.array(a["vals"]))
+
+
+# ---------------------------------------------------------------------------
+# eval_apply scores (.skme)
+# ---------------------------------------------------------------------------
+def write_evalscores(path: str, annotations: Sequence[str], names: Sequence[str], top1: np.ndarray, top2: np.ndarray,
+                     score1: np.ndarray, score2: np.ndarray, truth: np.ndarray, row_base: int) -> None:
+    """names: the label name table (the annotations first); truth int32 [Q]: entry of names the row's label was built
+    from, -1 for an ``_unknown_`` row; row q is row ``row_base + q`` of the file."""
+    ab, ao = _strings_to_arrays(annotations)
+    nb, no = _strings_to_arrays(names)
+    write_container(path, "evalscores", {"n_ann": len(annotations), "nrows": int(len(top1)), "row_base": int(row_base)},
+                    {"annotations": ab, "annotation_offsets": ao, "names": nb, "name_offsets": no,
+                     "top1": np.asarray(top1, dtype=np.int32), "top2": np.asarray(top2, dtype=np.int32),
+                     "score1": np.asarray(score1, dtype=np.float64), "score2": np.asarray(score2, dtype=np.float64),
+                     "truth": np.asarray(truth, dtype=np.int32)})
+
+
+def read_evalscores(path: str, mmap: bool = True) -> Dict:
+    kind, attrs, a = read_container(path, mmap)
+    if kind != "evalscores":
+        raise ValueError(f"{path}: holds '{kind}', not evalscores")
+    return dict(annotations=_arrays_to_strings(a["annotations"], a["annotation_offsets"]),
+                names=_arrays_to_strings(a["names"], a["name_offsets"]), row_base=int(attrs["row_base"]),
+                **{k: np.array(a[k]) for k in ("top1", "top2", "score1", "score2", "truth")})
 
 
 def read_counts(path: str, mmap: bool = True):
