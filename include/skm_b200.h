@@ -327,6 +327,19 @@ SKM_API int skm_apply_sparse(const int64_t *d_rowptr, const uint32_t *d_cols, co
                      const float *d_inv_m32, int64_t n_ann, int acc_bits, int32_t *d_top1, int32_t *d_top2,
                      double *d_score1, double *d_score2, double *d_qnorm2,
                      skm_stream_t stream);
+/* skm_apply_sparse that also writes every query's full cosine row, the association matrix of
+ * apply.smk:282-299 (save_apply_associations) and learn.smk:821-849 (seq-annotation-scores-*.csv):
+ * d_out_rows[q * ld_rows + a] for every q < nq and a < n_ann (float64, ld_rows >= n_ann, d_out_rows
+ * non-NULL), each the exact score of skm_apply_sparse — exactly 0.0 when the integer dot is 0, so the
+ * entries at d_top1 / d_top2 are bit-equal to d_score1 / d_score2.  Top-2 outputs as skm_apply_sparse,
+ * bit for bit.  The rows are written with streaming stores; [q, a0, a0 + n_ann) slices of a wider
+ * row-major buffer are what an annotation-sharded caller passes (d_out_rows offset by a0). */
+SKM_API int skm_apply_sparse_rows(const int64_t *d_rowptr, const uint32_t *d_cols, const int32_t *d_vals,
+                     int64_t nq, const int64_t *d_colptr, const int32_t *d_rows,
+                     const int32_t *d_mvals, const uint32_t *d_packed, const double *d_mnorm2,
+                     const float *d_inv_m32, int64_t n_ann, int acc_bits, int32_t *d_top1, int32_t *d_top2,
+                     double *d_score1, double *d_score2, double *d_qnorm2, double *d_out_rows,
+                     int64_t ld_rows, skm_stream_t stream);
 
 /* (a16/a17) apply: cosine_similarity + top-2, apply.smk:278-335 and
  * learn.smk:811-849.  Queries are int32 count rows [nq, K] over the same

@@ -80,6 +80,7 @@ SIGNATURES = {
     "skm_csc_build": (_int, [_p, _p, _i64, _i64, _i64, _p, _p, _p, _p, _p, _p, _p, _sz, _p]),
     "skm_csc_pack": (_int, [_p, _p, _i64, _p, _p]),
     "skm_apply_sparse": (_int, [_p, _p, _p, _i64, _p, _p, _p, _p, _p, _p, _i64, _int, _p, _p, _p, _p, _p, _p]),
+    "skm_apply_sparse_rows": (_int, [_p, _p, _p, _i64, _p, _p, _p, _p, _p, _p, _i64, _int, _p, _p, _p, _p, _p, _p, _i64, _p]),
     "skm_apply_tc_planes_bytes": (_sz, [_i64, _i64]),
     "skm_apply_tc_prepare": (_int, [_p, _i64, _i64, _p, _sz, C.POINTER(_int), _p]),
     "skm_apply_tc_workspace": (_sz, [_i64, _i64, _i64]),

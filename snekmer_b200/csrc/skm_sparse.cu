@@ -20,6 +20,8 @@
 //                     with shared-memory integer atomics (order-independent, hence reproducible),
 //                     then scan the accumulators for the top-2 (float32 screening, exact float64
 //                     scores for the survivors; apply.smk:278-335).
+//  skm_apply_sparse_rows  the same kernel that also streams every query's full cosine row out of the scan (the
+//                     association matrix, apply.smk:295-299 / learn.smk:821-849).
 //  window_keys_kernel is also the key generator of skm_count_csr (skm_count.cu).
 #include <vector>
 
@@ -239,14 +241,17 @@ constexpr int SPA_DUMMY = 32;      // dummy accumulators behind the padded real 
 //   scan   every thread owns the same accumulators for every query (4 adjacent ones per step): float32 screening
 //          score acc * inv_m32 against the thread's running runner-up, survivors inserted into a Top2x; the
 //          accumulators are zeroed on the way.  The threads' top-2 lists are then merged with exact float64 scores.
-template <typename AccT, bool PACKED>
+// ROWS: the scan also writes rows_out[q * ld + a] for every a < n_ann — sp_exact's value, exactly 0.0 for a zero dot
+// (which covers a zero-norm annotation and a query without a valid window) — so the row's entries at top1 / top2 are
+// bit-equal to score1 / score2.  Streaming stores: the CSC is what should stay in L2.
+template <typename AccT, bool PACKED, bool ROWS>
 __global__ void __launch_bounds__(SPA_THREADS, 1)
 apply_sparse_kernel(const int64_t *__restrict__ rowptr, const uint32_t *__restrict__ qcols, const int32_t *__restrict__ qvals,
                     int64_t nq, const int64_t *__restrict__ colptr, const int32_t *__restrict__ rows,
                     const int32_t *__restrict__ mvals, const uint32_t *__restrict__ packed,
                     const double *__restrict__ mnorm2, const float *__restrict__ inv_m32,
                     int n_ann, int32_t *__restrict__ top1, int32_t *__restrict__ top2, double *__restrict__ sc1,
-                    double *__restrict__ sc2, double *__restrict__ qnorm2_out) {
+                    double *__restrict__ sc2, double *__restrict__ qnorm2_out, double *__restrict__ rows_out, int64_t ld) {
     extern __shared__ __align__(16) uint8_t s_raw[];
     __shared__ unsigned long long s_n2;
     __shared__ Top2d s_top[SPA_THREADS / 32];
@@ -396,6 +401,12 @@ apply_sparse_kernel(const int64_t *__restrict__ rowptr, const uint32_t *__restri
                 for (int i = 0; i < PER; ++i) inv[i] = (a0 + i < n_ann) ? __ldg(inv_m32 + a0 + i) : 0.f;
             }
             *reinterpret_cast<uint4 *>(v) = *reinterpret_cast<const uint4 *>(&acc[a0]);
+            if constexpr (ROWS) {
+                double *dst = rows_out + q * ld + a0;
+#pragma unroll
+                for (int i = 0; i < PER; ++i)
+                    if (a0 + i < n_ann) __stcs(dst + i, v[i] != 0 ? sp_exact((unsigned long long)v[i], inv_qn, mnorm2, a0 + i) : 0.0);
+            }
             bool any = false;
 #pragma unroll
             for (int i = 0; i < PER; ++i) any |= (v[i] != 0);
@@ -1123,33 +1134,62 @@ int skm_csc_pack(const int32_t *d_rows, const int32_t *d_mvals, int64_t nnz, uin
     return SKM_OK;
 }
 
-int skm_apply_sparse(const int64_t *d_rowptr, const uint32_t *d_cols, const int32_t *d_vals, int64_t nq,
-                     const int64_t *d_colptr, const int32_t *d_rows, const int32_t *d_mvals, const uint32_t *d_packed, const double *d_mnorm2,
-                     const float *d_inv_m32, int64_t n_ann, int acc_bits, int32_t *d_top1, int32_t *d_top2,
-                     double *d_score1, double *d_score2, double *d_qnorm2, skm_stream_t stream) {
-    using namespace skm;
-    if (acc_bits != 32 && acc_bits != 64) { set_error("skm_apply_sparse: acc_bits must be 32 or 64"); return SKM_ERR_INVALID; }
+}  // extern "C"
+
+namespace skm {
+// the argument checks and the launch of skm_apply_sparse / skm_apply_sparse_rows
+template <bool ROWS>
+static int apply_sparse_launch(const char *fn, const int64_t *d_rowptr, const uint32_t *d_cols, const int32_t *d_vals, int64_t nq,
+                               const int64_t *d_colptr, const int32_t *d_rows, const int32_t *d_mvals, const uint32_t *d_packed,
+                               const double *d_mnorm2, const float *d_inv_m32, int64_t n_ann, int acc_bits, int32_t *d_top1,
+                               int32_t *d_top2, double *d_score1, double *d_score2, double *d_qnorm2, double *d_out_rows,
+                               int64_t ld_rows, skm_stream_t stream) {
+    if (acc_bits != 32 && acc_bits != 64) { set_error("%s: acc_bits must be 32 or 64", fn); return SKM_ERR_INVALID; }
     const int64_t cap = (200 * 1024) / (acc_bits / 8);
-    if (nq < 0 || n_ann <= 0 || n_ann > cap) { set_error("skm_apply_sparse: n_ann=%lld outside [1, %lld] for %d-bit accumulators (shard the annotations)", (long long)n_ann, (long long)cap, acc_bits); return n_ann > cap ? SKM_ERR_UNSUPPORTED : SKM_ERR_INVALID; }
+    if (nq < 0 || n_ann <= 0 || n_ann > cap) { set_error("%s: n_ann=%lld outside [1, %lld] for %d-bit accumulators (shard the annotations)", fn, (long long)n_ann, (long long)cap, acc_bits); return n_ann > cap ? SKM_ERR_UNSUPPORTED : SKM_ERR_INVALID; }
+    if (ROWS && ld_rows < n_ann) { set_error("%s: ld_rows=%lld < n_ann=%lld", fn, (long long)ld_rows, (long long)n_ann); return SKM_ERR_INVALID; }
     if (nq == 0) return SKM_OK;
-    if (!d_rowptr || !d_colptr || !d_mnorm2 || !d_inv_m32 || !d_top1 || !d_top2 || !d_score1 || !d_score2) { set_error("skm_apply_sparse: NULL argument"); return SKM_ERR_INVALID; }
-    if (d_packed && n_ann > 65536 - 4 - SPA_DUMMY) { set_error("skm_apply_sparse: the packed CSC holds 16-bit annotation indices (n_ann <= 65500)"); return SKM_ERR_INVALID; }
-    if ((reinterpret_cast<uintptr_t>(d_inv_m32) & 15u) != 0) { set_error("skm_apply_sparse: d_inv_m32 must be 16-byte aligned (vector loads)"); return SKM_ERR_INVALID; }
+    if (!d_rowptr || !d_colptr || !d_mnorm2 || !d_inv_m32 || !d_top1 || !d_top2 || !d_score1 || !d_score2 || (ROWS && !d_out_rows)) { set_error("%s: NULL argument", fn); return SKM_ERR_INVALID; }
+    if (d_packed && n_ann > 65536 - 4 - SPA_DUMMY) { set_error("%s: the packed CSC holds 16-bit annotation indices (n_ann <= 65500)", fn); return SKM_ERR_INVALID; }
+    if ((reinterpret_cast<uintptr_t>(d_inv_m32) & 15u) != 0) { set_error("%s: d_inv_m32 must be 16-byte aligned (vector loads)", fn); return SKM_ERR_INVALID; }
     const size_t smem = std::max<size_t>(size_t(n_ann + 4 + SPA_DUMMY) * (acc_bits / 8), 116 * 1024);   // > half an SM: one CTA per SM by construction
     const int grid = (int)std::min<int64_t>(nq, int64_t(sm_count()));
     cudaStream_t st = (cudaStream_t)stream;
 #define SKM_LAUNCH_SPA(ACC, PK)                                                                                              \
     {                                                                                                                        \
-        auto kern = apply_sparse_kernel<ACC, PK>;                                                                            \
+        auto kern = apply_sparse_kernel<ACC, PK, ROWS>;                                                                      \
         SKM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                    \
         kern<<<grid, SPA_THREADS, smem, st>>>(d_rowptr, d_cols, d_vals, nq, d_colptr, d_rows, d_mvals, d_packed, d_mnorm2,   \
-                                              d_inv_m32, (int)n_ann, d_top1, d_top2, d_score1, d_score2, d_qnorm2);          \
+                                              d_inv_m32, (int)n_ann, d_top1, d_top2, d_score1, d_score2, d_qnorm2,           \
+                                              d_out_rows, ld_rows);                                                          \
     }
     if (acc_bits == 32) { if (d_packed) SKM_LAUNCH_SPA(uint32_t, true) else SKM_LAUNCH_SPA(uint32_t, false) }
     else { if (d_packed) SKM_LAUNCH_SPA(unsigned long long, true) else SKM_LAUNCH_SPA(unsigned long long, false) }
 #undef SKM_LAUNCH_SPA
     SKM_LAUNCH_CHECK("apply_sparse_kernel");
     return SKM_OK;
+}
+}  // namespace skm
+
+extern "C" {
+
+int skm_apply_sparse(const int64_t *d_rowptr, const uint32_t *d_cols, const int32_t *d_vals, int64_t nq,
+                     const int64_t *d_colptr, const int32_t *d_rows, const int32_t *d_mvals, const uint32_t *d_packed, const double *d_mnorm2,
+                     const float *d_inv_m32, int64_t n_ann, int acc_bits, int32_t *d_top1, int32_t *d_top2,
+                     double *d_score1, double *d_score2, double *d_qnorm2, skm_stream_t stream) {
+    return skm::apply_sparse_launch<false>("skm_apply_sparse", d_rowptr, d_cols, d_vals, nq, d_colptr, d_rows, d_mvals, d_packed,
+                                           d_mnorm2, d_inv_m32, n_ann, acc_bits, d_top1, d_top2, d_score1, d_score2, d_qnorm2,
+                                           nullptr, 0, stream);
+}
+
+int skm_apply_sparse_rows(const int64_t *d_rowptr, const uint32_t *d_cols, const int32_t *d_vals, int64_t nq,
+                          const int64_t *d_colptr, const int32_t *d_rows, const int32_t *d_mvals, const uint32_t *d_packed,
+                          const double *d_mnorm2, const float *d_inv_m32, int64_t n_ann, int acc_bits, int32_t *d_top1,
+                          int32_t *d_top2, double *d_score1, double *d_score2, double *d_qnorm2, double *d_out_rows,
+                          int64_t ld_rows, skm_stream_t stream) {
+    return skm::apply_sparse_launch<true>("skm_apply_sparse_rows", d_rowptr, d_cols, d_vals, nq, d_colptr, d_rows, d_mvals, d_packed,
+                                          d_mnorm2, d_inv_m32, n_ann, acc_bits, d_top1, d_top2, d_score1, d_score2, d_qnorm2,
+                                          d_out_rows, ld_rows, stream);
 }
 
 }  // extern "C"

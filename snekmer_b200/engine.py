@@ -18,7 +18,7 @@ from __future__ import annotations
 
 import os
 from dataclasses import dataclass
-from typing import Optional, Sequence, Tuple, Union
+from typing import Callable, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -1211,10 +1211,13 @@ SPARSE_MAX_ANN = 50 * 1024          # annotations per apply_sparse call with 32-
 
 
 def apply_sparse(rowptr: torch.Tensor, cols: torch.Tensor, vals: torch.Tensor, csc: AnnotationCSC,
-                 max_row_total: Optional[int] = None, use_packed: bool = True) -> ApplyResult:
+                 max_row_total: Optional[int] = None, use_packed: bool = True,
+                 rows_out: Optional[torch.Tensor] = None) -> ApplyResult:
     """SpMM scoring of CSR queries (codes + counts, count_csr with basis=None) against one annotation slice.
     max_row_total bounds the sum of a query's counts (default: the largest row total, one reduction); it decides
-    whether the exact integer dots fit 32-bit accumulators."""
+    whether the exact integer dots fit 32-bit accumulators.  rows_out: a float64 device view [nq, >= n_ann] with unit
+    column stride (any row stride) that receives every query's full cosine row, entry for entry the value the top-2
+    scores are taken from (skm_apply_sparse_rows)."""
     dev = _require_cuda(rowptr.device)
     nq = rowptr.numel() - 1
     if nq == 0 or csc.n_ann == 0:               # no candidates: -1 / NaN, like apply_dense
@@ -1231,9 +1234,16 @@ def apply_sparse(rowptr: torch.Tensor, cols: torch.Tensor, vals: torch.Tensor, c
     if csc.n_ann > sparse_max_ann(acc_bits):
         raise SkmError(-3, f"apply_sparse: {csc.n_ann} annotations with {acc_bits}-bit accumulators exceed one pass "
                            f"({sparse_max_ann(acc_bits)}); use apply_sparse_tiled")
-    check(lib().skm_apply_sparse(_ptr(rowptr), _ptr(cols), _ptr(vals), nq, _ptr(csc.colptr), _ptr(csc.rows), _ptr(csc.mvals),
-                                 _ptr(csc.packed) if use_packed else None, _ptr(csc.mnorm2), _ptr(csc.inv_m32), csc.n_ann, acc_bits, _ptr(top1), _ptr(top2), _ptr(s1), _ptr(s2),
-                                 None, _stream()))
+    args = (_ptr(rowptr), _ptr(cols), _ptr(vals), nq, _ptr(csc.colptr), _ptr(csc.rows), _ptr(csc.mvals),
+            _ptr(csc.packed) if use_packed else None, _ptr(csc.mnorm2), _ptr(csc.inv_m32), csc.n_ann, acc_bits, _ptr(top1), _ptr(top2),
+            _ptr(s1), _ptr(s2), None)
+    if rows_out is None:
+        check(lib().skm_apply_sparse(*args, _stream()))
+    else:
+        if (rows_out.dtype != torch.float64 or rows_out.device != dev or rows_out.dim() != 2 or rows_out.shape[0] != nq
+                or rows_out.shape[1] < csc.n_ann or rows_out.stride(1) != 1):
+            raise SkmError(-2, f"apply_sparse: rows_out must be a float64 [{nq}, >= {csc.n_ann}] view with unit column stride on {dev}")
+        check(lib().skm_apply_sparse_rows(*args, _ptr(rows_out), rows_out.stride(0), _stream()))
     return ApplyResult(top1, top2, s1, s2, None)
 
 
@@ -1256,12 +1266,24 @@ def sparse_max_ann(acc_bits: int) -> int:
     return SPARSE_MAX_ANN if acc_bits == 32 else SPARSE_MAX_ANN // 2
 
 
-def apply_sparse_tiled(rowptr, cols, vals, keys, mvals, S: int, n_ann: int, tile: Optional[int] = None) -> ApplyResult:
+ROWS_CHUNK_BYTES = 1 << 30         # device buffer of one query chunk of association rows (two are in flight)
+
+
+def apply_sparse_tiled(rowptr, cols, vals, keys, mvals, S: int, n_ann: int, tile: Optional[int] = None,
+                       rows_sink: Optional[Callable[[int, np.ndarray], None]] = None,
+                       chunk_rows: Optional[int] = None) -> ApplyResult:
     """All annotations of a sorted COO matrix, `tile` at a time, merged with the top-2 merge (the same fan-in as the
     multi-GPU annotation sharding).  The tile defaults to what one pass can hold, which depends on the accumulator
-    width: 51,200 annotations with 32-bit accumulators, 25,600 when max(M) * (largest query total) needs 64 bits."""
+    width: 51,200 annotations with 32-bit accumulators, 25,600 when max(M) * (largest query total) needs 64 bits.
+
+    rows_sink(q0, block): also stream the full cosine rows (the association matrix) to the host, `chunk_rows` queries
+    at a time (default: a ~1 GiB float64 block), in query order: block is float64 [rows, n_ann] for queries
+    [q0, q0 + rows), a view of pinned memory that is reused once the call returns.  The result is bit-identical to the
+    call without a sink."""
     dev = rowptr.device
     nq = rowptr.numel() - 1
+    if rows_sink is not None and nq > 0:
+        return _apply_sparse_rows_tiled(rowptr, cols, vals, keys, mvals, S, n_ann, tile, rows_sink, chunk_rows)
     if n_ann <= 0 or nq <= 0:
         return ApplyResult(torch.full((nq,), -1, dtype=torch.int32, device=dev), torch.full((nq,), -1, dtype=torch.int32, device=dev),
                            torch.full((nq,), float("nan"), dtype=torch.float64, device=dev),
@@ -1280,6 +1302,65 @@ def apply_sparse_tiled(rowptr, cols, vals, keys, mvals, S: int, n_ann: int, tile
         idxs.append(torch.where(i >= 0, i + a0, i))
         scs.append(torch.stack([r.score1, r.score2]))
     return merge_top2(torch.stack(idxs), torch.stack(scs))
+
+
+def _apply_sparse_rows_tiled(rowptr, cols, vals, keys, mvals, S: int, n_ann: int, tile: Optional[int], rows_sink,
+                             chunk_rows: Optional[int]) -> ApplyResult:
+    """apply_sparse_tiled with a rows sink (nq > 0).  The annotation-tile CSCs are built once; every query chunk runs
+    each tile into its column slice of a [chunk, n_ann] device block (the kernel reads absolute CSR offsets, so a chunk
+    is rowptr[q0:q1 + 1] without a copy).  Two device and two pinned host blocks: the copy of chunk i (side stream,
+    events) and the sink's work on it overlap the kernels of chunk i + 1."""
+    dev = rowptr.device
+    nq = rowptr.numel() - 1
+    n_ann = max(int(n_ann), 0)
+    chunk = int(chunk_rows) if chunk_rows is not None else ROWS_CHUNK_BYTES // (8 * max(n_ann, 1))
+    chunk = max(1, min(chunk, nq))
+    tiles = []
+    row_total = 0
+    if n_ann > 0:
+        row_total = query_row_total_max(rowptr, vals)
+        max_m = int(mvals.max().item()) if mvals.numel() else 0
+        cap = sparse_max_ann(sparse_acc_bits(max_m, row_total))
+        tile = cap if tile is None else max(1, min(int(tile), cap))
+        tiles = [(a0, csc_build(keys, mvals, S, min(tile, n_ann - a0), a0)) for a0 in range(0, n_ann, tile)]
+    main = torch.cuda.current_stream(dev)
+    side = torch.cuda.Stream(dev)
+    dbuf = [torch.empty((chunk, n_ann), dtype=torch.float64, device=dev) for _ in range(2)]
+    hbuf = [torch.empty((chunk, n_ann), dtype=torch.float64, pin_memory=True) for _ in range(2)]
+    copied = [torch.cuda.Event() for _ in range(2)]
+    outs = [[] for _ in tiles]                      # per tile: the chunks' ApplyResults
+    pending = None                                  # (slot, q0, rows) whose copy is in flight
+    for i, q0 in enumerate(range(0, nq, chunk)):
+        s, n = i % 2, min(chunk, nq - q0)
+        main.wait_event(copied[s])                  # the copy of chunk i - 2 has left dbuf[s]
+        rp = rowptr[q0:q0 + n + 1]
+        for t, (a0, csc) in enumerate(tiles):
+            outs[t].append(apply_sparse(rp, cols, vals, csc, row_total, rows_out=dbuf[s][:n, a0:a0 + csc.n_ann]))
+        side.wait_stream(main)
+        with torch.cuda.stream(side):
+            hbuf[s][:n].copy_(dbuf[s][:n], non_blocking=True)
+            copied[s].record(side)
+        if pending is not None:
+            _rows_flush(pending, hbuf, copied, rows_sink)
+        pending = (s, q0, n)
+    _rows_flush(pending, hbuf, copied, rows_sink)
+    if not tiles:
+        return apply_sparse_tiled(rowptr, cols, vals, keys, mvals, S, 0)
+    res = [ApplyResult(*(torch.cat([getattr(r, f) for r in o]) for f in ("top1", "top2", "score1", "score2"))) for o in outs]
+    if len(res) == 1:
+        return res[0]
+    idxs, scs = [], []
+    for (a0, _), r in zip(tiles, res):
+        i = torch.stack([r.top1.to(torch.int64), r.top2.to(torch.int64)])
+        idxs.append(torch.where(i >= 0, i + a0, i))
+        scs.append(torch.stack([r.score1, r.score2]))
+    return merge_top2(torch.stack(idxs), torch.stack(scs))
+
+
+def _rows_flush(pending, hbuf, copied, rows_sink) -> None:
+    s, q0, n = pending
+    copied[s].synchronize()
+    rows_sink(q0, hbuf[s][:n].numpy())
 
 
 # ---------------------------------------------------------------------------
@@ -1505,10 +1586,11 @@ def query_csr_wide(batch: SequenceBatch, alphabet: AlphabetT, k: int, basis: Wid
 
 
 def apply_wide(rowptr: torch.Tensor, cols: torch.Tensor, vals: torch.Tensor, keys: torch.Tensor, mvals: torch.Tensor, K: int,
-               n_ann: int, tile: Optional[int] = None) -> ApplyResult:
+               n_ann: int, tile: Optional[int] = None, rows_sink: Optional[Callable[[int, np.ndarray], None]] = None,
+               chunk_rows: Optional[int] = None) -> ApplyResult:
     """apply_sparse_tiled for a matrix keyed by basis column (learn_wide, key = ann * K + col) and queries from
     query_csr_wide: the matrix is re-keyed to the stride K + 1, whose last column is the empty one."""
-    return apply_sparse_tiled(rowptr, cols, vals, keys + keys // K if K else keys, mvals, K + 1, n_ann, tile)
+    return apply_sparse_tiled(rowptr, cols, vals, keys + keys // K if K else keys, mvals, K + 1, n_ann, tile, rows_sink, chunk_rows)
 
 
 def build_basis_wide_distributed(batch: SequenceBatch, alphabet, k: int, min_filter: int = 0,

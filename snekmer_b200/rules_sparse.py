@@ -8,7 +8,7 @@ binary ``.skmc`` side-car (sidecar.py) as the file between them:
   learn_counts_sparse   Library (learn.smk:306-408)      -> COO matrix + Totals on the device
   merge_counts_sparse   Merge (learn.smk:467-494)        -> outer join on annotations, sum (skm_coo_merge)
   eval_counts_sparse    KmerCompare of learn (learn.smk:628-887) -> SpMM cosine, top-2 + each row's annotation
-                        (EvalScores; the ``.skme`` side-car in place of seq-annotation-scores-*.csv)
+                        (EvalScores; the ``.skme`` side-car, and seq-annotation-scores-*.csv or its ``.skma`` when asked)
   evaluate_sparse       Evaluator (learn.smk:923-1348)   -> row classes and crosstabs on the device, the confidence files
   apply_counts_sparse   KmerCompare (apply.smk:224-342)  -> SpMM cosine, top-2, delta, Confidence
 
@@ -263,9 +263,11 @@ def restrict_csr_to_kmers(rowptr: torch.Tensor, cols: torch.Tensor, vals: torch.
     return csum[rowptr], cols[keep].contiguous(), vals[keep].contiguous()
 
 
-def _score_sparse(seqs: Sequence[str], sc: SparseCounts, tile: Optional[int], query_kmers: Optional[Sequence[str]]) -> E.ApplyResult:
+def _score_sparse(seqs: Sequence[str], sc: SparseCounts, tile: Optional[int], query_kmers: Optional[Sequence[str]],
+                  rows_sink=None, chunk_rows: Optional[int] = None) -> E.ApplyResult:
     """Cosine of every sequence against every annotation row of `sc` as SpMM, top-2 on the device (see
-    apply_counts_sparse for `query_kmers` and `tile`)."""
+    apply_counts_sparse for `query_kmers` and `tile`); rows_sink / chunk_rows: the full rows as well
+    (engine.apply_sparse_tiled)."""
     tab = E.alphabet_tables_from_symbols(sc.symbols)
     batch = E.SequenceBatch.from_strings(list(seqs))
     A = len(sc.annotations)
@@ -275,26 +277,54 @@ def _score_sparse(seqs: Sequence[str], sc: SparseCounts, tile: Optional[int], qu
             qcodes, ok = E.encode_kmers([str(x) for x in query_kmers], tab.symbols, sc.k)
             restrict = E.wide_basis_from_codes(np.unique(qcodes[ok]), tab, sc.k, batch.device)
         rowptr, cols, cvals = E.query_csr_wide(batch, tab, sc.k, sc.columns, restrict)
-        return E.apply_wide(rowptr, cols, cvals, sc.keys, sc.vals, sc.columns.K, A, tile)
+        return E.apply_wide(rowptr, cols, cvals, sc.keys, sc.vals, sc.columns.K, A, tile, rows_sink, chunk_rows)
     rowptr, cols, cvals = E.count_csr(batch, tab, sc.k, None)
     if query_kmers is not None:
         rowptr, cols, cvals = restrict_csr_to_kmers(rowptr, cols, cvals, tab.symbols, sc.k, query_kmers)
-    return E.apply_sparse_tiled(rowptr, cols, cvals, sc.keys, sc.vals, sc.S, A, tile)
+    return E.apply_sparse_tiled(rowptr, cols, cvals, sc.keys, sc.vals, sc.S, A, tile, rows_sink, chunk_rows)
+
+
+MASK_BLOCK_ROWS = 65536     # rows per record batch of a top-2-only association file
+
+
+def _write_top2_rows(w, r: E.ApplyResult, A: int) -> None:
+    """The masked association rows of eval_apply without save_associations (learn.smk:831-849): each row keeps its
+    top-2 scores, every other entry NaN — built from the top-2, block by block."""
+    top1, top2 = r.top1.cpu().numpy(), r.top2.cpu().numpy()
+    s1, s2 = r.score1.cpu().numpy(), r.score2.cpu().numpy()
+    for q0 in range(0, len(top1), MASK_BLOCK_ROWS):
+        q1 = min(q0 + MASK_BLOCK_ROWS, len(top1))
+        block = np.full((q1 - q0, A), np.nan)
+        rows = np.arange(q1 - q0)
+        t1, t2 = top1[q0:q1], top2[q0:q1]
+        k1, k2 = t1 >= 0, t2 >= 0
+        block[rows[k1], t1[k1]] = s1[q0:q1][k1]
+        block[rows[k2], t2[k2]] = s2[q0:q1][k2]
+        w.write(q0, block)
 
 
 def apply_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], sc: SparseCounts, confidence_csv: Optional[str] = None,
                         out_summary: Optional[str] = None, tile: Optional[int] = None,
-                        query_kmers: Optional[Sequence[str]] = None) -> ScoreResult:
+                        query_kmers: Optional[Sequence[str]] = None, out_scores: Optional[str] = None,
+                        save_associations: bool = False, chunk_rows: Optional[int] = None) -> ScoreResult:
     """KmerCompare of the apply workflow (apply.smk:224-342) as SpMM: cosine of every query against every annotation
     row, top-2, delta, Confidence; writes kmer-summary CSV when asked.  A repeated id keeps its last record.
     query_kmers: the query file's kmerlist (from its .npz / side-car).  The reference's query norm and dot run over that
     list; without it every valid window of the query counts — the same thing when the vectorize step ran with
     min_filter = 0 and no basis file, which is the only case the two differ in.  The annotation tile follows the
-    accumulator width the data needs (engine.apply_sparse_tiled)."""
+    accumulator width the data needs (engine.apply_sparse_tiled).
+    out_scores with save_associations (learnapp: save_apply_associations, apply.smk:295-299): the association file,
+    every query's cosine against every annotation (columns = the annotations, ``__index_level_0__`` = the distinct
+    query ids last), streamed from the device `chunk_rows` queries at a time; a path ending in ``.skma`` writes the
+    side-car (sidecar.export_associations_csv turns it into the CSV)."""
     uniq, pick = _unique_last(list(ids))
     seqs = [str(reduced_seqs[int(i)]) for i in pick]
     A = len(sc.annotations)
-    r = _score_sparse(seqs, sc, tile, query_kmers)
+    if out_scores and save_associations:
+        with sidecar.associations_writer(out_scores, sc.annotations, uniq) as w:
+            r = _score_sparse(seqs, sc, tile, query_kmers, w.write, chunk_rows)
+    else:
+        r = _score_sparse(seqs, sc, tile, query_kmers)
     top1, top2 = r.top1.cpu().numpy(), r.top2.cpu().numpy()
     s1, s2 = r.score1.cpu().numpy(), r.score2.cpu().numpy()
     if out_summary:
@@ -328,23 +358,40 @@ class EvalScores:
 
 def eval_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], sc: SparseCounts, seq_annot: Dict[str, str],
                        out_sidecar: Optional[str] = None, tile: Optional[int] = None,
-                       query_kmers: Optional[Sequence[str]] = None) -> EvalScores:
+                       query_kmers: Optional[Sequence[str]] = None, out_scores: Optional[str] = None,
+                       save_associations: bool = False, chunk_rows: Optional[int] = None) -> EvalScores:
     """KmerCompare of the learn workflow (learn.smk:628-887) as SpMM: the training sequences of one file against the
     merged matrix.  Rows as eval_apply_rule: the distinct ids (a repeated id keeps its first position and last record),
     numbered in that order; a row is known when its accession is in `seq_annot` — the caller passes the FIRST
     annotation file only, as the rule reads only that one.  Top-2 stay on the device; `out_sidecar` writes the
     ``.skme`` that evaluate_sparse reads.  With several ranks (matrix replicated), each passes a contiguous share of the
-    file's distinct ids, in order; row numbers continue across ranks."""
+    file's distinct ids, in order; row numbers continue across ranks.
+    out_scores: the rule's seq-annotation-scores file (``.skma`` side-car for a path ending in .skma), rows labelled
+    ``<annotation>_known_<n>`` / ``<accession>_unknown_<n>`` (learn.smk:712-732): with save_associations every score,
+    streamed from the device `chunk_rows` rows at a time; without, each row's top-2 and NaN elsewhere
+    (learn.smk:831-849).  Each rank writes its own rows."""
     uniq, pick = _unique_last(list(ids))
     dev = E._require_cuda()
-    if uniq:
-        r = _score_sparse([str(reduced_seqs[int(i)]) for i in pick], sc, tile, query_kmers)
-    else:
-        e32, e64 = torch.zeros(0, dtype=torch.int32, device=dev), torch.zeros(0, dtype=torch.float64, device=dev)
-        r = E.ApplyResult(e32, e32.clone(), e64, e64.clone())
     accs = [_ACCESSION.findall(sid)[0] for sid in uniq]         # IndexError without two pipes, like learn.smk:714
+    row_base, _ = D.exclusive_prefix(len(uniq), dev)
+    w = None
+    if out_scores:
+        labels = [f"{seq_annot[a]}_known_{row_base + n}" if a in seq_annot else f"{a}_unknown_{row_base + n}"
+                  for n, a in enumerate(accs)]
+        w = sidecar.associations_writer(out_scores, sc.annotations, labels)
+    try:
+        if uniq:
+            sink = w.write if (w is not None and save_associations) else None
+            r = _score_sparse([str(reduced_seqs[int(i)]) for i in pick], sc, tile, query_kmers, sink, chunk_rows)
+        else:
+            e32, e64 = torch.zeros(0, dtype=torch.int32, device=dev), torch.zeros(0, dtype=torch.float64, device=dev)
+            r = E.ApplyResult(e32, e32.clone(), e64, e64.clone())
+        if w is not None and not save_associations:
+            _write_top2_rows(w, r, len(sc.annotations))
+    finally:
+        if w is not None:
+            w.close()
     names, truth = CF.joint_name_table(sc.annotations, [seq_annot[a] if a in seq_annot else None for a in accs])
-    row_base, _ = D.exclusive_prefix(len(uniq), r.top1.device)
     ev = EvalScores(list(sc.annotations), names, r.top1, r.top2, r.score1, r.score2, torch.from_numpy(truth).to(r.top1.device),
                     row_base)
     if out_sidecar:

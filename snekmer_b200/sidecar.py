@@ -13,6 +13,9 @@ every kernel, so the GPU path keeps
   *.skme   eval_apply scores of one training file for the evaluate rule (in place of seq-annotation-scores-*.csv):
            the matrix's annotations, the name table of the row labels, top-2 columns and scores and the label's
            annotation (truth) of every row, and the global number of the first row
+  *.skma   an association matrix (apply.smk:295-299, learn.smk:821-849): the annotation names, the row labels and
+           the float64 [Q, A] cosine table, written block by block while the rows stream off the device;
+           ``export_associations_csv`` writes the reference's seq-annotation-scores CSV from it
 
 in one flat container (below), whose arrays can be memory-mapped and uploaded without parsing.  ``export_npz`` /
 ``export_counts_csv`` / ``export_totals_csv`` write exactly what the reference's rules write; ``import_counts_csv``
@@ -52,9 +55,10 @@ def _arrays_to_strings(buf: np.ndarray, off: np.ndarray) -> List[str]:
     return [raw[off[i]:off[i + 1]].decode("utf-8") for i in range(len(off) - 1)]
 
 
-def write_container(path: str, kind: str, attrs: Dict, arrays: Dict[str, np.ndarray]) -> None:
-    arrs = {k: np.ascontiguousarray(v) for k, v in arrays.items()}
-    entries = [{"name": k, "dtype": v.dtype.str, "shape": list(v.shape), "offset": 0, "nbytes": int(v.nbytes)} for k, v in arrs.items()]
+def _layout(kind: str, attrs: Dict, specs: Sequence[Tuple[str, np.dtype, Tuple[int, ...]]]) -> Tuple[bytes, List[Dict]]:
+    """(file header with its meta, array entries with their offsets) of a container holding arrays (name, dtype, shape)."""
+    entries = [{"name": k, "dtype": np.dtype(dt).str, "shape": list(shape), "offset": 0,
+                "nbytes": int(np.prod(shape, dtype=np.int64)) * np.dtype(dt).itemsize} for k, dt, shape in specs]
     # offsets depend on the meta length, which depends on the offsets' digits: reserve, then fix
     meta_len = _pad(len(json.dumps({"kind": kind, "attrs": attrs, "arrays": entries}).encode()) + 24 * len(entries) + 64)
     pos = _pad(len(MAGIC) + 16 + meta_len)
@@ -63,9 +67,14 @@ def write_container(path: str, kind: str, attrs: Dict, arrays: Dict[str, np.ndar
         pos = _pad(pos + e["nbytes"])
     meta = json.dumps({"kind": kind, "attrs": attrs, "arrays": entries}).encode()
     assert len(meta) <= meta_len
+    return MAGIC + struct.pack("<IIQ", VERSION, 0, meta_len) + meta + b" " * (meta_len - len(meta)), entries
+
+
+def write_container(path: str, kind: str, attrs: Dict, arrays: Dict[str, np.ndarray]) -> None:
+    arrs = {k: np.ascontiguousarray(v) for k, v in arrays.items()}
+    head, entries = _layout(kind, attrs, [(k, v.dtype, v.shape) for k, v in arrs.items()])
     with open(path, "wb") as f:
-        f.write(MAGIC + struct.pack("<IIQ", VERSION, 0, meta_len))
-        f.write(meta + b" " * (meta_len - len(meta)))
+        f.write(head)
         for e in entries:
             f.write(b"\0" * (e["offset"] - f.tell()))
             f.write(arrs[e["name"]].tobytes())
@@ -246,3 +255,102 @@ def export_counts_csv(skmc_path: str, csv_path: str, total_seqs: Optional[int] =
     assert t.rows and t.rows[0] == "Totals", "a per-file counts table starts with its Totals row"
     r = LearnResult(t.rows[1:], t.seq_count[1:], t.M[1:], t.M[0], int(t.seq_count[0]) if total_seqs is None else total_seqs, t.kmers)
     write_counts_csv(csv_path, r)
+
+
+# ---------------------------------------------------------------------------
+# association matrices (.skma)  ->  seq-annotation-scores-*.csv
+# ---------------------------------------------------------------------------
+INDEX_COL = "__index_level_0__"
+
+
+class AssociationsWriter:
+    """``.skma`` written block by block: the names and labels go first and the [Q, A] float64 array is laid out behind
+    them up front, so write(q0, block) puts rows [q0, q0 + len(block)) straight at their place."""
+
+    def __init__(self, path: str, annotations: Sequence[str], labels: Sequence[str]):
+        ab, ao = _strings_to_arrays(annotations)
+        lb, lo = _strings_to_arrays(labels)
+        small = {"annotations": ab, "annotation_offsets": ao, "rows": lb, "row_offsets": lo}
+        self.Q, self.A = len(labels), len(annotations)
+        head, entries = _layout("associations", {"n_ann": self.A, "nrows": self.Q},
+                                [(k, v.dtype, v.shape) for k, v in small.items()] + [("scores", np.dtype(np.float64), (self.Q, self.A))])
+        self._f = open(path, "wb")
+        self._f.write(head)
+        for e in entries[:-1]:
+            self._f.write(b"\0" * (e["offset"] - self._f.tell()))
+            self._f.write(small[e["name"]].tobytes())
+        self._base = entries[-1]["offset"]
+        self._f.truncate(self._base + entries[-1]["nbytes"])
+
+    def write(self, q0: int, block: np.ndarray) -> None:
+        block = np.ascontiguousarray(block, dtype=np.float64)
+        assert block.ndim == 2 and block.shape[1] == self.A and 0 <= q0 and q0 + block.shape[0] <= self.Q
+        self._f.seek(self._base + q0 * self.A * 8)
+        self._f.write(block.tobytes())
+
+    def close(self) -> None:
+        self._f.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class AssociationsCSVWriter:
+    """The seq-annotation-scores CSV (annotations as float64 columns, the row labels last under ``__index_level_0__``)
+    streamed through pyarrow's CSVWriter, one record batch per block: the bytes of one ``pyarrow.csv.write_csv`` of the
+    whole table, which is how the reference and rules.apply_rule / eval_apply_rule write it.  Blocks come in row order."""
+
+    def __init__(self, path: str, annotations: Sequence[str], labels: Sequence[str]):
+        import pyarrow as pa
+        from pyarrow import csv as pacsv
+
+        self._pa = pa
+        self._labels = [str(x) for x in labels]
+        self.A = len(annotations)
+        self._schema = pa.schema([(str(a), pa.float64()) for a in annotations] + [(INDEX_COL, pa.string())])
+        self._w = pacsv.CSVWriter(path, self._schema)
+        self._next = 0
+
+    def write(self, q0: int, block: np.ndarray) -> None:
+        assert q0 == self._next and block.ndim == 2 and block.shape[1] == self.A, "blocks in row order"
+        n = block.shape[0]
+        pa = self._pa
+        arrays = [pa.array(np.ascontiguousarray(block[:, j], dtype=np.float64)) for j in range(self.A)]
+        self._w.write_batch(pa.record_batch(arrays + [pa.array(self._labels[q0:q0 + n], type=pa.string())], schema=self._schema))
+        self._next = q0 + n
+
+    def close(self) -> None:
+        self._w.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+def associations_writer(path: str, annotations: Sequence[str], labels: Sequence[str]):
+    """``.skma`` side-car for a path ending in .skma, the CSV otherwise."""
+    cls = AssociationsWriter if str(path).endswith(".skma") else AssociationsCSVWriter
+    return cls(path, annotations, labels)
+
+
+def read_associations(path: str, mmap: bool = True) -> Dict:
+    """annotations, rows (labels) and scores float64 [Q, A] (memory-mapped)."""
+    kind, attrs, a = read_container(path, mmap)
+    if kind != "associations":
+        raise ValueError(f"{path}: holds '{kind}', not associations")
+    return dict(annotations=_arrays_to_strings(a["annotations"], a["annotation_offsets"]),
+                rows=_arrays_to_strings(a["rows"], a["row_offsets"]), scores=a["scores"])
+
+
+def export_associations_csv(skma_path: str, csv_path: str, block_rows: int = 65536) -> None:
+    """The seq-annotation-scores CSV of a ``.skma``, byte for byte what the direct writer gives."""
+    d = read_associations(skma_path)
+    S = d["scores"]
+    with AssociationsCSVWriter(csv_path, d["annotations"], d["rows"]) as w:
+        for q0 in range(0, S.shape[0], block_rows):
+            w.write(q0, S[q0:q0 + block_rows])
