@@ -524,6 +524,69 @@ SKM_API int skm_fasta_scan(const uint8_t *text, int64_t nbytes, int threads, int
 SKM_API int skm_fasta_pack(const uint8_t *text, int64_t nbytes, int threads, uint8_t *residues_out,
                    int64_t *offsets_out, uint8_t *ids_out, int64_t *id_offsets_out);
 
+/* ---- CSV interchange files formatted on the device (skm_csv.cu) -----------------------------------------------
+ * The text of the reference's seq-annotation-scores files (apply.smk:295-299, learn.smk:821-849: pyarrow.csv.write_csv
+ * of float64 columns and the string index column) and kmer-counts files (learn.smk:328-357 pandas layout,
+ * :583-594 pyarrow layout).  Two passes: *_measure writes d_row_offsets int64 [rows + 1] (0, then the running byte
+ * count after each row); *_write puts row r at d_text + d_row_offsets[r] - d_row_offsets[0], so a call over rows
+ * [r0, r1) can pass d_row_offsets + r0 of a measure over more rows.  Workspace of a measure call:
+ * skm_csv_rows_workspace(rows).  Row labels: UTF-8 bytes d_labels, absolute offsets int64 [rows + 1]
+ * (d_label_offsets + r0 for a sub-range).
+ *
+ * float64 cells as pyarrow prints them: the shortest decimal that round-trips (closest of the shortest, ties to
+ * even), decimal notation when the value is d.ddd x 10^x with -6 <= x <= 9 (no trailing ".0"), else d[.ddd]e+x /
+ * d[.ddd]e-x; "nan" for any NaN, "inf", "-inf", "-0"; at most 25 bytes.  skm_csv_f64_host: the same function on the
+ * host (out >= 25 bytes, no terminator), returns the length. */
+SKM_API int skm_csv_f64_host(double v, char *out);
+SKM_API size_t skm_csv_rows_workspace(int64_t rows);
+/* Association rows: cells d_scores[r * ld + j] (j < A), each followed by ',', then the label in '"' with inner '"'
+ * doubled, then '\n'. */
+SKM_API int skm_csv_assoc_measure(const double *d_scores, int64_t rows, int64_t A, int64_t ld, const uint8_t *d_labels,
+                          const int64_t *d_label_offsets, int64_t *d_row_offsets, void *workspace, size_t workspace_bytes,
+                          skm_stream_t stream);
+SKM_API int skm_csv_assoc_write(const double *d_scores, int64_t rows, int64_t A, int64_t ld, const uint8_t *d_labels,
+                        const int64_t *d_label_offsets, const int64_t *d_row_offsets, uint8_t *d_text, skm_stream_t stream);
+/* The top-2-masked association rows of eval_apply without save_associations (learn.smk:831-849): cell j of row r is
+ * d_score2[r] when j == d_top2[r], else d_score1[r] when j == d_top1[r], else NaN ("nan"); no [rows, A] block. */
+SKM_API int skm_csv_top2_measure(const int32_t *d_top1, const int32_t *d_top2, const double *d_score1, const double *d_score2,
+                         int64_t rows, int64_t A, const uint8_t *d_labels, const int64_t *d_label_offsets,
+                         int64_t *d_row_offsets, void *workspace, size_t workspace_bytes, skm_stream_t stream);
+SKM_API int skm_csv_top2_write(const int32_t *d_top1, const int32_t *d_top2, const double *d_score1, const double *d_score2,
+                       int64_t rows, int64_t A, const uint8_t *d_labels, const int64_t *d_label_offsets,
+                       const int64_t *d_row_offsets, uint8_t *d_text, skm_stream_t stream);
+/* Count rows from CSR over the file's K k-mer columns (d_rowptr int64 [rows + 1] absolute, d_cols int32 strictly
+ * ascending in [0, K) within a row, d_vals int64; zero values count as absent) with the Sequence count / Kmer Count
+ * fields d_seq_count / d_kmer_count int64 [rows].  layout 0 (learn.smk:328-357): label bytes verbatim (the caller
+ * escapes them), then the two fields and the K cells, zeros blank.  layout 1 (learn.smk:583-594): the two fields and
+ * the K cells with zeros as "0", then the label in '"' with inner '"' doubled.  Cells joined by ',', rows end in '\n'. */
+SKM_API int skm_csv_counts_measure(const int64_t *d_rowptr, const int64_t *d_vals, int64_t rows, int64_t K,
+                           const int64_t *d_seq_count, const int64_t *d_kmer_count, const uint8_t *d_labels,
+                           const int64_t *d_label_offsets, int layout, int64_t *d_row_offsets, void *workspace,
+                           size_t workspace_bytes, skm_stream_t stream);
+SKM_API int skm_csv_counts_write(const int64_t *d_rowptr, const int32_t *d_cols, const int64_t *d_vals, int64_t rows, int64_t K,
+                         const int64_t *d_seq_count, const int64_t *d_kmer_count, const uint8_t *d_labels,
+                         const int64_t *d_label_offsets, int layout, const int64_t *d_row_offsets, uint8_t *d_text,
+                         skm_stream_t stream);
+
+/* Count-CSV parser (either layout; learn.smk:496-579 reads these files).  skm_csv_parse_rows: d_parity uint8 [nbytes]
+ * = inclusive XOR scan of the '"' bytes (1 inside quotes); d_row_ends int64 [nbytes] receives the positions of the
+ * '\n' bytes outside quotes in order, *d_nrows (device) their number.  Workspace: skm_csv_parse_workspace(nbytes).
+ * skm_csv_parse_cells: row r is [d_row_start[r], d_row_end[r]] (its '\n' included), split into fields at ',' outside
+ * quotes; d_role int32 [nfields] names each field: -1 the label (its byte range [d_label_start, d_label_end) is
+ * written, quotes included), -2 Sequence count, -3 Kmer Count, j >= 0 k-mer column j.  A cell is empty (0), [0-9]+,
+ * [0-9]+\.0* or d[.ddd]e[+-]x of an integer below 2^63.  With d_entry_offsets NULL: the count pass (d_row_nnz, the
+ * two fields, the label ranges); else the write pass: the nonzero cells of row r as (d_cols, d_vals) from
+ * d_entry_offsets[r], in column order.  *d_error (set to ~0 by the caller) takes the least (row << 32 | field) of a
+ * malformed cell, field 0xFFFFFFFF for a row with a field count other than nfields.  rows < 2^31. */
+SKM_API size_t skm_csv_parse_workspace(int64_t nbytes);
+SKM_API int skm_csv_parse_rows(const uint8_t *d_text, int64_t nbytes, uint8_t *d_parity, int64_t *d_row_ends, int64_t *d_nrows,
+                       void *workspace, size_t workspace_bytes, skm_stream_t stream);
+SKM_API int skm_csv_parse_cells(const uint8_t *d_text, const uint8_t *d_parity, const int64_t *d_row_start,
+                        const int64_t *d_row_end, int64_t rows, const int32_t *d_role, int nfields,
+                        const int64_t *d_entry_offsets, int64_t *d_row_nnz, int64_t *d_seq_count, int64_t *d_kmer_count,
+                        int64_t *d_label_start, int64_t *d_label_end, int32_t *d_cols, int64_t *d_vals,
+                        unsigned long long *d_error, skm_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

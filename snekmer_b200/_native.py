@@ -112,6 +112,17 @@ SIGNATURES = {
     "skm_rows_emit": (_int, [_p, _i64, _i64, _p, _p, _p, _p, _p, _i64, _p]),
     "skm_rows_colsum": (_int, [_p, _i64, _i64, _p, _p]),
     "skm_scatter_add_i64": (_int, [_p, _i64, _i64, _p, _p, _p, _i64, _i64, _p]),
+    "skm_csv_f64_host": (_int, [C.c_double, C.c_char_p]),
+    "skm_csv_rows_workspace": (_sz, [_i64]),
+    "skm_csv_assoc_measure": (_int, [_p, _i64, _i64, _i64, _p, _p, _p, _p, _sz, _p]),
+    "skm_csv_assoc_write": (_int, [_p, _i64, _i64, _i64, _p, _p, _p, _p, _p]),
+    "skm_csv_top2_measure": (_int, [_p, _p, _p, _p, _i64, _i64, _p, _p, _p, _p, _sz, _p]),
+    "skm_csv_top2_write": (_int, [_p, _p, _p, _p, _i64, _i64, _p, _p, _p, _p, _p]),
+    "skm_csv_counts_measure": (_int, [_p, _p, _i64, _i64, _p, _p, _p, _p, _int, _p, _p, _sz, _p]),
+    "skm_csv_counts_write": (_int, [_p, _p, _p, _i64, _i64, _p, _p, _p, _p, _int, _p, _p, _p]),
+    "skm_csv_parse_workspace": (_sz, [_i64]),
+    "skm_csv_parse_rows": (_int, [_p, _i64, _p, _p, _p, _p, _sz, _p]),
+    "skm_csv_parse_cells": (_int, [_p, _p, _p, _p, _i64, _p, _int, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
 }
 
 

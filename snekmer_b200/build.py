@@ -20,7 +20,7 @@ LIBDIR = os.path.join(PKG, "lib")
 LIB = os.path.join(LIBDIR, "libskm_b200.so")
 INCLUDE = os.path.join(os.path.dirname(PKG), "include")
 
-SOURCES = ["skm_api.cu", "skm_encode.cu", "skm_basis.cu", "skm_count.cu", "skm_learn.cu", "skm_apply.cu", "skm_apply_tc.cu", "skm_util.cu", "skm_sparse.cu", "skm_wide.cu", "skm_confidence.cu", "skm_fasta.cu", "skm_csrsort.cu", "skm_bench.cu", "skm_rows.cu", "skm_peer.cu"]
+SOURCES = ["skm_api.cu", "skm_encode.cu", "skm_basis.cu", "skm_count.cu", "skm_learn.cu", "skm_apply.cu", "skm_apply_tc.cu", "skm_util.cu", "skm_sparse.cu", "skm_wide.cu", "skm_confidence.cu", "skm_fasta.cu", "skm_csrsort.cu", "skm_bench.cu", "skm_rows.cu", "skm_peer.cu", "skm_csv.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -52,7 +52,7 @@ int check_common(const void *d_residues, int64_t nres, const void *d_offsets, in
 
 extern "C" {
 
-int skm_version(void) { return 20300; /* 2.3.0 */ }
+int skm_version(void) { return 20400; /* 2.4.0 */ }
 
 const char *skm_last_error(void) { return skm::g_err; }
 

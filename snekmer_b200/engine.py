@@ -1278,8 +1278,9 @@ def apply_sparse_tiled(rowptr, cols, vals, keys, mvals, S: int, n_ann: int, tile
 
     rows_sink(q0, block): also stream the full cosine rows (the association matrix) to the host, `chunk_rows` queries
     at a time (default: a ~1 GiB float64 block), in query order: block is float64 [rows, n_ann] for queries
-    [q0, q0 + rows), a view of pinned memory that is reused once the call returns.  The result is bit-identical to the
-    call without a sink."""
+    [q0, q0 + rows), a view of pinned memory that is reused once the call returns.  An AssociationsCSVText sink
+    instead gets every chunk as CSV text formatted on the device (chunks of ~1 GiB of worst-case text), and only the
+    text is copied to the host.  The result is bit-identical to the call without a sink."""
     dev = rowptr.device
     nq = rowptr.numel() - 1
     if rows_sink is not None and nq > 0:
@@ -1313,7 +1314,9 @@ def _apply_sparse_rows_tiled(rowptr, cols, vals, keys, mvals, S: int, n_ann: int
     dev = rowptr.device
     nq = rowptr.numel() - 1
     n_ann = max(int(n_ann), 0)
-    chunk = int(chunk_rows) if chunk_rows is not None else ROWS_CHUNK_BYTES // (8 * max(n_ann, 1))
+    csv = rows_sink if isinstance(rows_sink, AssociationsCSVText) else None
+    row_bytes = csv.row_bound() if csv is not None else 8 * max(n_ann, 1)
+    chunk = int(chunk_rows) if chunk_rows is not None else ROWS_CHUNK_BYTES // row_bytes
     chunk = max(1, min(chunk, nq))
     tiles = []
     row_total = 0
@@ -1325,25 +1328,37 @@ def _apply_sparse_rows_tiled(rowptr, cols, vals, keys, mvals, S: int, n_ann: int
         tiles = [(a0, csc_build(keys, mvals, S, min(tile, n_ann - a0), a0)) for a0 in range(0, n_ann, tile)]
     main = torch.cuda.current_stream(dev)
     side = torch.cuda.Stream(dev)
-    dbuf = [torch.empty((chunk, n_ann), dtype=torch.float64, device=dev) for _ in range(2)]
-    hbuf = [torch.empty((chunk, n_ann), dtype=torch.float64, pin_memory=True) for _ in range(2)]
-    copied = [torch.cuda.Event() for _ in range(2)]
+    dbuf = [torch.empty((chunk, n_ann), dtype=torch.float64, device=dev) for _ in range(2 if csv is None else 1)]
     outs = [[] for _ in tiles]                      # per tile: the chunks' ApplyResults
-    pending = None                                  # (slot, q0, rows) whose copy is in flight
-    for i, q0 in enumerate(range(0, nq, chunk)):
-        s, n = i % 2, min(chunk, nq - q0)
-        main.wait_event(copied[s])                  # the copy of chunk i - 2 has left dbuf[s]
-        rp = rowptr[q0:q0 + n + 1]
-        for t, (a0, csc) in enumerate(tiles):
-            outs[t].append(apply_sparse(rp, cols, vals, csc, row_total, rows_out=dbuf[s][:n, a0:a0 + csc.n_ann]))
-        side.wait_stream(main)
-        with torch.cuda.stream(side):
-            hbuf[s][:n].copy_(dbuf[s][:n], non_blocking=True)
-            copied[s].record(side)
-        if pending is not None:
-            _rows_flush(pending, hbuf, copied, rows_sink)
-        pending = (s, q0, n)
-    _rows_flush(pending, hbuf, copied, rows_sink)
+    if csv is not None:
+        # the block is formatted on the device right behind its kernels; only the text is copied (TextPipe)
+        pipe = csv.pipe(chunk)
+        for q0 in range(0, nq, chunk):
+            n = min(chunk, nq - q0)
+            rp = rowptr[q0:q0 + n + 1]
+            for t, (a0, csc) in enumerate(tiles):
+                outs[t].append(apply_sparse(rp, cols, vals, csc, row_total, rows_out=dbuf[0][:n, a0:a0 + csc.n_ann]))
+            s = pipe.slot()
+            pipe.push(s, csv.format_rows(q0, dbuf[0][:n], pipe.text[s]))
+        pipe.close()
+    else:
+        hbuf = [torch.empty((chunk, n_ann), dtype=torch.float64, pin_memory=True) for _ in range(2)]
+        copied = [torch.cuda.Event() for _ in range(2)]
+        pending = None                              # (slot, q0, rows) whose copy is in flight
+        for i, q0 in enumerate(range(0, nq, chunk)):
+            s, n = i % 2, min(chunk, nq - q0)
+            main.wait_event(copied[s])              # the copy of chunk i - 2 has left dbuf[s]
+            rp = rowptr[q0:q0 + n + 1]
+            for t, (a0, csc) in enumerate(tiles):
+                outs[t].append(apply_sparse(rp, cols, vals, csc, row_total, rows_out=dbuf[s][:n, a0:a0 + csc.n_ann]))
+            side.wait_stream(main)
+            with torch.cuda.stream(side):
+                hbuf[s][:n].copy_(dbuf[s][:n], non_blocking=True)
+                copied[s].record(side)
+            if pending is not None:
+                _rows_flush(pending, hbuf, copied, rows_sink)
+            pending = (s, q0, n)
+        _rows_flush(pending, hbuf, copied, rows_sink)
     if not tiles:
         return apply_sparse_tiled(rowptr, cols, vals, keys, mvals, S, 0)
     res = [ApplyResult(*(torch.cat([getattr(r, f) for r in o]) for f in ("top1", "top2", "score1", "score2"))) for o in outs]
@@ -1361,6 +1376,323 @@ def _rows_flush(pending, hbuf, copied, rows_sink) -> None:
     s, q0, n = pending
     copied[s].synchronize()
     rows_sink(q0, hbuf[s][:n].numpy())
+
+
+# ---------------------------------------------------------------------------
+# CSV text on the device (skm_csv.cu): the reference's interchange files, formatted where the data is
+# ---------------------------------------------------------------------------
+CSV_CELL_MAX = 26                  # a float64 cell as pyarrow prints it (<= 25 bytes) and its separator
+CSV_INDEX_COL = "__index_level_0__"
+
+
+def pyarrow_quote(text: str) -> str:
+    """A string cell or header name as pyarrow's CSV writer quotes it."""
+    return '"' + str(text).replace('"', '""') + '"'
+
+
+def labels_device(labels: Sequence[str], device=None) -> Tuple[torch.Tensor, torch.Tensor, np.ndarray]:
+    """(UTF-8 bytes uint8, offsets int64 [n + 1]) on the device, and the offsets on the host."""
+    dev = _require_cuda(device)
+    enc = [str(x).encode("utf-8") for x in labels]
+    off = np.zeros(len(enc) + 1, dtype=np.int64)
+    if enc:
+        np.cumsum([len(b) for b in enc], out=off[1:])
+    raw = np.frombuffer(b"".join(enc), dtype=np.uint8)
+    return torch.from_numpy(raw.copy()).to(dev), torch.from_numpy(off).to(dev), off
+
+
+def _csv_measure(fn, rows: int, *args) -> torch.Tensor:
+    """Row offsets int64 [rows + 1] of a *_measure entry point (args: everything before d_row_offsets)."""
+    dev = _require_cuda()
+    row_off = torch.empty(rows + 1, dtype=torch.int64, device=dev)
+    ws_bytes = lib().skm_csv_rows_workspace(rows)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    check(fn(*args, _ptr(row_off), _ptr(ws), ws_bytes, _stream()))
+    return row_off
+
+
+class TextPipe:
+    """Chunks of text written on the device into two device buffers, copied to two pinned host buffers and appended to
+    a file: the copy and the file write of one chunk run while the next chunk is computed and formatted."""
+
+    def __init__(self, f, capacity: int, device=None):
+        dev = _require_cuda(device)
+        self.f = f
+        self.main = torch.cuda.current_stream(dev)
+        self.side = torch.cuda.Stream(dev)
+        self.text = [torch.empty(max(int(capacity), 1), dtype=torch.uint8, device=dev) for _ in range(2)]
+        self.host = [torch.empty(max(int(capacity), 1), dtype=torch.uint8, pin_memory=True) for _ in range(2)]
+        self.nbytes = [torch.zeros(1, dtype=torch.int64, pin_memory=True) for _ in range(2)]
+        self.ready = [torch.cuda.Event() for _ in range(2)]
+        self.copied = [torch.cuda.Event() for _ in range(2)]
+        self.i = 0
+        self.pending = None
+
+    def slot(self) -> int:
+        """The buffer for the next chunk; its previous text has left the device before the main stream writes it."""
+        s = self.i % 2
+        self.main.wait_event(self.copied[s])
+        return s
+
+    def push(self, s: int, row_off: torch.Tensor) -> None:
+        """text[s][:row_off[-1]] holds the chunk (written on the main stream).  Flushes the previous chunk first, so
+        its copy is not queued behind this chunk's kernels."""
+        if self.pending is not None:
+            self._flush(self.pending)
+        self.side.wait_stream(self.main)
+        with torch.cuda.stream(self.side):
+            self.nbytes[s].copy_(row_off[-1:], non_blocking=True)
+            self.ready[s].record(self.side)
+        row_off.record_stream(self.side)        # the allocator keeps it until the side stream's copy has read it
+        self.pending = s
+        self.i += 1
+
+    def _flush(self, s: int) -> None:
+        self.ready[s].synchronize()
+        n = int(self.nbytes[s][0])
+        with torch.cuda.stream(self.side):
+            self.host[s][:n].copy_(self.text[s][:n], non_blocking=True)
+            self.copied[s].record(self.side)
+        self.copied[s].synchronize()
+        self.f.write(memoryview(self.host[s][:n].numpy()))
+
+    def close(self) -> None:
+        if self.pending is not None:
+            self._flush(self.pending)
+            self.pending = None
+
+
+class AssociationsCSVText:
+    """The seq-annotation-scores CSV (apply.smk:295-299, learn.smk:821-849) with its rows formatted on the device
+    (skm_csv_assoc_*): byte for byte what sidecar.AssociationsCSVWriter writes through pyarrow.  Passed as the
+    rows_sink of apply_sparse_tiled, or filled by write_top2_csv."""
+
+    def __init__(self, path: str, annotations: Sequence[str], labels: Sequence[str], device=None):
+        self.A = len(annotations)
+        self.Q = len(labels)
+        self.labels, self.label_off, off = labels_device(labels, device)
+        self.max_label = int(np.diff(off).max()) if len(labels) else 0
+        self.f = open(path, "wb")
+        self.f.write((",".join(pyarrow_quote(x) for x in list(annotations) + [CSV_INDEX_COL]) + "\n").encode("utf-8"))
+        self._pipe = None
+
+    def row_bound(self) -> int:
+        """Most bytes a row can take: every cell at its longest, every label byte a quote."""
+        return CSV_CELL_MAX * self.A + 2 * self.max_label + 3
+
+    def pipe(self, rows: int) -> TextPipe:
+        self._pipe = TextPipe(self.f, rows * self.row_bound(), self.label_off.device)
+        return self._pipe
+
+    def format_rows(self, q0: int, block: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
+        """Rows q0 .. q0 + len(block) of a float64 device block [n, A] (unit column stride) into out; -> row offsets."""
+        n = block.shape[0]
+        assert block.dtype == torch.float64 and block.shape[1] == self.A and (n == 0 or block.stride(1) == 1 or self.A <= 1)
+        assert out.numel() >= n * self.row_bound() and 0 <= q0 and q0 + n <= self.Q
+        lo = self.label_off[q0:q0 + n + 1]
+        ld = block.stride(0) if self.A else 0
+        row_off = _csv_measure(lib().skm_csv_assoc_measure, n, _ptr(block), n, self.A, ld, _ptr(self.labels), _ptr(lo))
+        check(lib().skm_csv_assoc_write(_ptr(block), n, self.A, ld, _ptr(self.labels), _ptr(lo), _ptr(row_off), _ptr(out), _stream()))
+        return row_off
+
+    def close(self) -> None:
+        if self._pipe is not None:
+            self._pipe.close()
+            self._pipe = None
+        self.f.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+def write_top2_csv(w: AssociationsCSVText, r: ApplyResult, chunk_rows: Optional[int] = None) -> None:
+    """The top-2-masked association rows of eval_apply without save_associations (learn.smk:831-849) into w: each
+    row's two best scores and "nan" elsewhere, formatted on the device straight from the top-2 (skm_csv_top2_*)."""
+    nq = r.top1.numel()
+    assert nq == w.Q
+    if nq == 0:
+        return
+    chunk = max(1, min(int(chunk_rows) if chunk_rows is not None else ROWS_CHUNK_BYTES // w.row_bound(), nq))
+    pipe = w.pipe(chunk)
+    t1, t2, s1, s2 = (x.contiguous() for x in (r.top1, r.top2, r.score1, r.score2))
+    for q0 in range(0, nq, chunk):
+        n = min(chunk, nq - q0)
+        lo = w.label_off[q0:q0 + n + 1]
+        ptrs = [_ptr(x) + q0 * x.element_size() for x in (t1, t2, s1, s2)]
+        row_off = _csv_measure(lib().skm_csv_top2_measure, n, *ptrs, n, w.A, _ptr(w.labels), _ptr(lo))
+        s = pipe.slot()
+        check(lib().skm_csv_top2_write(*ptrs, n, w.A, _ptr(w.labels), _ptr(lo), _ptr(row_off), _ptr(pipe.text[s]), _stream()))
+        pipe.push(s, row_off)
+    pipe.close()
+
+
+CSV_PARSE_BLOCK = 1 << 30          # bytes of a count CSV on the device at a time
+
+
+def _csv_header(f) -> Tuple[bytes, int]:
+    """(the header line's bytes without its '\n', bytes consumed): the first newline outside quotes."""
+    head, parity = b"", 0
+    while True:
+        piece = f.read(1 << 20)
+        if not piece:
+            return head, len(head)
+        a = np.frombuffer(piece, dtype=np.uint8)
+        par = (np.cumsum(a == ord('"')) + parity) & 1
+        hit = np.flatnonzero((a == ord("\n")) & (par == 0))
+        if hit.size:
+            cut = int(hit[0])
+            f.seek(len(head) + cut + 1)
+            return head + piece[:cut], len(head) + cut + 1
+        head += piece
+        parity = int(par[-1])
+
+
+def _csv_label(raw: bytes) -> str:
+    if len(raw) >= 2 and raw[:1] == b'"' and raw[-1:] == b'"':
+        raw = raw[1:-1].replace(b'""', b'"')
+    return raw.decode("utf-8")
+
+
+def parse_counts_csv(path: str, block_bytes: int = CSV_PARSE_BLOCK, device=None):
+    """A kmer-counts CSV of either layout (learn.smk:328-357 / :583-594) parsed on the device (skm_csv_parse_*), read
+    in blocks of `block_bytes`, each cut at its last row end with the rest carried into the next block.  Header and
+    labels are decoded on the host.  -> (labels, kmers, seq_count int64 [R], kmer_count int64 [R], rowptr int64 [R + 1],
+    cols int32 (file columns, ascending in a row), vals int64) with the CSR on the device; zeros are left out.
+    A cell outside the grammar (empty, [0-9]+, [0-9]+.0*, pyarrow's exponent form of an integer below 2^63) raises
+    SkmError naming the line and the column."""
+    import csv as _csv
+    import io as _io
+
+    dev = _require_cuda(device)
+    with open(path, "rb") as f:
+        head, consumed = _csv_header(f)
+        header = next(_csv.reader(_io.StringIO(head.decode("utf-8")))) if head else []
+        if CSV_INDEX_COL not in header:
+            raise SkmError(-1, f"{path}: no {CSV_INDEX_COL} column in the header")
+        role = np.empty(len(header), dtype=np.int32)
+        kmers = []
+        for j, name in enumerate(header):
+            if name == CSV_INDEX_COL:
+                role[j] = -1
+            elif name == "Sequence count":
+                role[j] = -2
+            elif name == "Kmer Count":
+                role[j] = -3
+            else:
+                role[j] = len(kmers)
+                kmers.append(name)
+        if (role == -2).sum() != 1 or (role == -3).sum() != 1 or (role == -1).sum() != 1:
+            raise SkmError(-1, f"{path}: the header needs one each of {CSV_INDEX_COL}, Sequence count and Kmer Count")
+        d_role = torch.from_numpy(role).to(dev)
+        labels, seqs, kcs, nnzs, colss, valss = [], [], [], [], [], []
+        line = 2                                    # line number of the next row
+        carry, block, eof = b"", max(int(block_bytes), 1), False
+        while not eof or carry:
+            piece = f.read(max(block - len(carry), 1)) if not eof else b""
+            eof = eof or not piece
+            buf = carry + piece
+            if eof and buf and not buf.endswith(b"\n"):
+                buf += b"\n"
+            if not buf:
+                break
+            n = len(buf)
+            text = torch.from_numpy(np.frombuffer(buf, dtype=np.uint8).copy()).to(dev)
+            parity = torch.empty(n, dtype=torch.uint8, device=dev)
+            ends = torch.empty(n, dtype=torch.int64, device=dev)
+            d_n = torch.zeros(1, dtype=torch.int64, device=dev)
+            ws_bytes = lib().skm_csv_parse_workspace(n)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            check(lib().skm_csv_parse_rows(_ptr(text), n, _ptr(parity), _ptr(ends), _ptr(d_n), _ptr(ws), ws_bytes, _stream()))
+            m = int(d_n.item())
+            if m == 0:                              # a row longer than the block: read on with a larger one
+                carry, block = buf, 2 * block
+                if eof:
+                    raise SkmError(-1, f"{path}: line {line}: a quoted field is not closed")
+                continue
+            ends = ends[:m]
+            last_nl = int(ends[-1].item())          # the block is cut after its last row end
+            starts = torch.cat([torch.zeros(1, dtype=torch.int64, device=dev), ends[:-1] + 1])
+            keep = ends > starts                    # blank lines are skipped, like csv.reader
+            starts, ends = starts[keep].contiguous(), ends[keep].contiguous()
+            R = starts.numel()
+            if R:
+                nnz = torch.empty(R, dtype=torch.int64, device=dev)
+                sq = torch.zeros(R, dtype=torch.int64, device=dev)
+                kc = torch.zeros(R, dtype=torch.int64, device=dev)
+                ls = torch.zeros(R, dtype=torch.int64, device=dev)
+                le = torch.zeros(R, dtype=torch.int64, device=dev)
+                err = torch.full((1,), -1, dtype=torch.int64, device=dev)
+                check(lib().skm_csv_parse_cells(_ptr(text), _ptr(parity), _ptr(starts), _ptr(ends), R, _ptr(d_role), len(header), None,
+                                                _ptr(nnz), _ptr(sq), _ptr(kc), _ptr(ls), _ptr(le), None, None, _ptr(err), _stream()))
+                e = int(err.item()) & 0xFFFFFFFFFFFFFFFF
+                if e != 0xFFFFFFFFFFFFFFFF:
+                    r, fld = e >> 32, e & 0xFFFFFFFF
+                    at = line + buf.count(b"\n", 0, int(starts[r].item()))
+                    if fld == 0xFFFFFFFF:
+                        raise SkmError(-1, f"{path}: line {at}: the row does not have the header's {len(header)} fields")
+                    raise SkmError(-1, f"{path}: line {at}, column {header[fld]!r}: the cell is not an integer count")
+                off = torch.zeros(R + 1, dtype=torch.int64, device=dev)
+                torch.cumsum(nnz, 0, out=off[1:])
+                tot = int(off[-1].item())
+                cols = torch.empty(max(tot, 1), dtype=torch.int32, device=dev)
+                vals = torch.empty(max(tot, 1), dtype=torch.int64, device=dev)
+                check(lib().skm_csv_parse_cells(_ptr(text), _ptr(parity), _ptr(starts), _ptr(ends), R, _ptr(d_role), len(header),
+                                                _ptr(off), None, None, None, None, None, _ptr(cols), _ptr(vals), _ptr(err), _stream()))
+                lsh, leh = ls.cpu().numpy(), le.cpu().numpy()
+                labels += [_csv_label(buf[a:b]) for a, b in zip(lsh.tolist(), leh.tolist())]
+                seqs.append(sq.cpu().numpy())
+                kcs.append(kc.cpu().numpy())
+                nnzs.append(nnz)
+                colss.append(cols[:tot])
+                valss.append(vals[:tot])
+            line += buf.count(b"\n", 0, last_nl + 1)
+            carry = buf[last_nl + 1:]
+            if eof and carry:
+                raise SkmError(-1, f"{path}: line {line}: a quoted field is not closed")
+    R = len(labels)
+    rowptr = torch.zeros(R + 1, dtype=torch.int64, device=dev)
+    if R:
+        torch.cumsum(torch.cat(nnzs), 0, out=rowptr[1:])
+    cols = torch.cat(colss) if colss else torch.zeros(0, dtype=torch.int32, device=dev)
+    vals = torch.cat(valss) if valss else torch.zeros(0, dtype=torch.int64, device=dev)
+    cat = lambda xs: np.concatenate(xs) if xs else np.zeros(0, dtype=np.int64)
+    return labels, kmers, cat(seqs), cat(kcs), rowptr, cols, vals
+
+
+CSV_LEARN, CSV_TOTAL = 0, 1        # count-file layouts: learn.smk:328-357 (pandas) and :583-594 (pyarrow)
+
+
+def write_counts_csv_rows(f, rowptr: torch.Tensor, cols: torch.Tensor, vals: torch.Tensor, K: int, seq_count: torch.Tensor,
+                          kmer_count: torch.Tensor, labels: Sequence[str], layout: int) -> None:
+    """Rows of a kmer-counts CSV from device CSR over the file's K k-mer columns (skm_csv_counts_*), appended to the
+    open binary file f.  labels: written verbatim with CSV_LEARN (escape them first), quoted with CSV_TOTAL."""
+    dev = rowptr.device
+    R = rowptr.numel() - 1
+    if R == 0:
+        return
+    lab, lab_off, _ = labels_device(labels, dev)
+    row_off = _csv_measure(lib().skm_csv_counts_measure, R, _ptr(rowptr), _ptr(vals), R, int(K), _ptr(seq_count), _ptr(kmer_count),
+                           _ptr(lab), _ptr(lab_off), int(layout))
+    off = row_off.cpu().numpy()
+    # chunks of whole rows of about ROWS_CHUNK_BYTES of text (a longer row is a chunk of its own)
+    cuts = [0]
+    while cuts[-1] < R:
+        r0 = cuts[-1]
+        r1 = int(np.searchsorted(off, off[r0] + ROWS_CHUNK_BYTES, side="right")) - 1
+        cuts.append(min(max(r1, r0 + 1), R))
+    cap = max(int(off[b] - off[a]) for a, b in zip(cuts[:-1], cuts[1:]))
+    pipe = TextPipe(f, cap, dev)
+    for r0, r1 in zip(cuts[:-1], cuts[1:]):
+        n = r1 - r0
+        s = pipe.slot()
+        check(lib().skm_csv_counts_write(_ptr(rowptr) + 8 * r0, _ptr(cols), _ptr(vals), n, int(K), _ptr(seq_count) + 8 * r0,
+                                         _ptr(kmer_count) + 8 * r0, _ptr(lab), _ptr(lab_off) + 8 * r0, int(layout),
+                                         _ptr(row_off) + 8 * r0, _ptr(pipe.text[s]), _stream()))
+        pipe.push(s, row_off[r0:r1 + 1] - row_off[r0])
+    pipe.close()
 
 
 # ---------------------------------------------------------------------------

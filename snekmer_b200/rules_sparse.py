@@ -103,17 +103,21 @@ def learn_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], symbols
     return SparseCounts(annotations, seq_count, tab.symbols, int(k), keys, vals, totals, total)
 
 
-def write_counts_sidecar(path: str, sc: SparseCounts, kmers: Optional[Sequence[str]] = None) -> None:
-    """``.skmc`` of a learned matrix: rows ``Totals`` + annotations, columns = `kmers` (default: the k-mers that occur, in
-    code order; pass the vectorize rule's kmerlist to get the reference's column order), CSR values."""
+def _file_csr(sc: SparseCounts, kmers: Optional[Sequence[str]] = None):
+    """A learned matrix as CSR over the columns of a counts file: (kmers, rowptr int64 [A + 2], cols int32, vals int64,
+    seq_count int64 [A + 1] on the host, kmer_count int64 [A + 1]), rows ``Totals`` + annotations, columns ascending in
+    a row, zeros left out; device tensors.  kmers: the file's columns (default: the k-mers that occur, in code order;
+    the vectorize rule's kmerlist gives the reference's column order).  The key -> file-column remap and the row sort
+    (skm_coo_merge over annotation * K + column) run on the device."""
     S = sc.stride
-    totals = sc.totals.cpu().numpy()
+    dev = sc.keys.device
+    totals = sc.totals
     # col_of_code: file column of every key % S (a code, or a learned column when the matrix has a column table)
     if sc.columns is not None:
         learned = sc.columns.codes_host()
         col_of_code = np.full(S, -1, dtype=np.int64)
         if kmers is None:
-            occ = np.flatnonzero(totals)
+            occ = np.flatnonzero(totals.cpu().numpy())
             kmers = list(E.decode_kmers(learned[occ], sc.symbols, sc.k))
             col_of_code[occ] = np.arange(len(occ))
         else:
@@ -126,7 +130,7 @@ def write_counts_sidecar(path: str, sc: SparseCounts, kmers: Optional[Sequence[s
             hit = (fcodes[j] == learned) if len(fcodes) else np.zeros(len(learned), dtype=bool)
             col_of_code[hit] = fcol[order][j[hit]]
     elif kmers is None:
-        codes = np.flatnonzero(totals).astype(np.uint64)
+        codes = np.flatnonzero(totals.cpu().numpy()).astype(np.uint64)
         kmers = list(E.decode_kmers(codes, sc.symbols, sc.k))
         col_of_code = np.full(S, -1, dtype=np.int64)
         col_of_code[codes.astype(np.int64)] = np.arange(len(codes))
@@ -135,42 +139,89 @@ def write_counts_sidecar(path: str, sc: SparseCounts, kmers: Optional[Sequence[s
         codes, ok = E.encode_kmers(kmers, sc.symbols, sc.k)
         col_of_code = np.full(S, -1, dtype=np.int64)
         col_of_code[codes[ok].astype(np.int64)] = np.flatnonzero(ok)
-    keys = sc.keys.cpu().numpy()
-    vals = sc.vals.cpu().numpy()
-    ann, code = keys // S, keys % S
-    col = col_of_code[code]
+    K, A = len(kmers), len(sc.annotations)
+    cmap = torch.from_numpy(col_of_code).to(dev)
+    z = torch.zeros(0, dtype=torch.int64, device=dev)
+    col = cmap[sc.keys % S] if sc.keys.numel() else z
     keep = col >= 0
-    ann, col, vals = ann[keep], col[keep], vals[keep]
-    order = np.lexsort((col, ann))                                   # rows by annotation, columns ascending inside a row
-    ann, col, vals = ann[order], col[order], vals[order]
-    t_cols = np.flatnonzero(col_of_code >= 0)
-    t_col = col_of_code[t_cols]
-    t_order = np.argsort(t_col, kind="stable")
-    t_vals = totals[t_cols][t_order]
-    nzt = t_vals != 0
-    A = len(sc.annotations)
-    rowptr = np.zeros(A + 2, dtype=np.int64)
-    rowptr[1] = int(nzt.sum())
-    np.cumsum(np.bincount(ann, minlength=A), out=rowptr[2:])
-    rowptr[2:] += rowptr[1]
-    row_sum = np.zeros(A, dtype=np.int64)
-    np.add.at(row_sum, ann, vals)
-    sidecar.write_counts_csr(path, ["Totals"] + list(sc.annotations), kmers,
-                             np.concatenate([[sc.total_seqs], sc.seq_count]), np.concatenate([[int(t_vals.sum())], row_sum]),
-                             rowptr, np.concatenate([t_col[t_order][nzt], col]).astype(np.int32), np.concatenate([t_vals[nzt], vals]))
+    fkeys, fvals = (sc.keys // S)[keep] * K + col[keep], sc.vals[keep]
+    if fkeys.numel():
+        fkeys, fvals = E.coo_merge(fkeys, fvals, key_bound=A * K)    # rows by annotation, columns ascending in a row
+    tkeep = (cmap >= 0) & (totals != 0) if S else torch.zeros(0, dtype=torch.bool, device=dev)
+    tcols, tvals = cmap[tkeep], totals[tkeep]
+    if tcols.numel():
+        tcols, tvals = E.coo_merge(tcols, tvals, key_bound=K)
+    rowptr = torch.zeros(A + 2, dtype=torch.int64, device=dev)
+    rowptr[1:] = tcols.numel()
+    if A:
+        rowptr[2:] += torch.searchsorted(fkeys, torch.arange(1, A + 1, dtype=torch.int64, device=dev) * K)
+    vals = torch.cat([tvals, fvals])
+    csum = torch.zeros(vals.numel() + 1, dtype=torch.int64, device=dev)
+    torch.cumsum(vals, 0, out=csum[1:])
+    kmer_count = csum[rowptr[1:]] - csum[rowptr[:-1]]
+    cols = torch.cat([tcols, fkeys % K if K else fkeys]).to(torch.int32)
+    seq_count = np.concatenate([[sc.total_seqs], sc.seq_count]).astype(np.int64)
+    return kmers, rowptr, cols, vals, seq_count, kmer_count
+
+
+def write_counts_sidecar(path: str, sc: SparseCounts, kmers: Optional[Sequence[str]] = None) -> None:
+    """``.skmc`` of a learned matrix: rows ``Totals`` + annotations, columns = `kmers` (default: the k-mers that occur, in
+    code order; pass the vectorize rule's kmerlist to get the reference's column order), CSR values."""
+    kmers, rowptr, cols, vals, seq_count, kmer_count = _file_csr(sc, kmers)
+    sidecar.write_counts_csr(path, ["Totals"] + list(sc.annotations), kmers, seq_count, kmer_count.cpu().numpy(),
+                             rowptr.cpu().numpy(), cols.cpu().numpy(), vals.cpu().numpy())
+
+
+def write_counts_csv(path: str, sc: SparseCounts, kmers: Optional[Sequence[str]] = None, layout: str = "learn") -> None:
+    """The reference's count file of a learned matrix, its rows formatted on the device from the file-column CSR —
+    no dense matrix: ``layout="learn"`` kmer-counts-{nb}.csv as the learn rule writes it (learn.smk:328-357: index
+    first, zeros blank), ``"total"`` kmer-counts-total.csv as the merge rule writes it (learn.smk:583-594: quoted header,
+    zeros as 0, index last).  Byte for byte write_counts_sidecar followed by sidecar.export_counts_csv /
+    export_totals_csv; `kmers` as in write_counts_sidecar."""
+    from .rules import INDEX_COL, _csv_field
+
+    if layout not in ("learn", "total"):
+        raise ValueError(f"layout must be 'learn' or 'total', not {layout!r}")
+    kmers, rowptr, cols, vals, seq_count, kmer_count = _file_csr(sc, kmers)
+    rows = ["Totals"] + [str(a) for a in sc.annotations]
+    d_seq = torch.from_numpy(seq_count).to(rowptr.device)
+    with open(path, "wb") as f:
+        if layout == "learn":
+            f.write((",".join([INDEX_COL, "Sequence count", "Kmer Count"] + [_csv_field(km) for km in kmers]) + "\n").encode("utf-8"))
+            E.write_counts_csv_rows(f, rowptr, cols, vals, len(kmers), d_seq, kmer_count, [_csv_field(r) for r in rows], E.CSV_LEARN)
+        else:
+            f.write((",".join(E.pyarrow_quote(x) for x in ["Sequence count", "Kmer Count"] + list(kmers) + [INDEX_COL]) + "\n").encode("utf-8"))
+            E.write_counts_csv_rows(f, rowptr, cols, vals, len(kmers), d_seq, kmer_count, rows, E.CSV_TOTAL)
 
 
 def read_counts_sidecar(path: str, symbols: Optional[str] = None) -> SparseCounts:
     """``.skmc`` -> device COO.  The reduced alphabet is the set of characters of the k-mer columns unless given.  In a
     code space beyond 2^27 the matrix is keyed by column: the file's k-mers (those of the alphabet) in file order."""
     d = sidecar.read_counts_csr(path)
-    kmers = d["kmers"]
-    if not d["rows"] or d["rows"][0] != "Totals":
+    dev = E._require_cuda()
+    return _counts_from_file_csr(path, d["rows"], d["kmers"], d["seq_count"], torch.from_numpy(d["rowptr"]).to(dev),
+                                 torch.from_numpy(d["cols"]).to(dev), torch.from_numpy(d["vals"]).to(dev), symbols)
+
+
+def read_counts_csv(path: str, symbols: Optional[str] = None, block_bytes: int = E.CSV_PARSE_BLOCK) -> SparseCounts:
+    """A kmer-counts CSV of either layout (a stock ``kmer-counts-total.csv`` or ``base/counts`` file, learn.smk:496-579)
+    parsed on the device (engine.parse_counts_csv) straight into the device COO: what
+    ``read_counts_sidecar(import_counts_csv(path))`` returns, without a dense matrix.  Cells follow a stated grammar —
+    empty, [0-9]+, [0-9]+.0*, pyarrow's exponent form of an integer — and anything else raises SkmError."""
+    labels, kmers, seq_count, _, rowptr, cols, vals = E.parse_counts_csv(path, block_bytes)
+    return _counts_from_file_csr(path, labels, kmers, seq_count, rowptr, cols, vals, symbols)
+
+
+def _counts_from_file_csr(path: str, rows: Sequence[str], kmers: Sequence[str], seq_count: np.ndarray, rowptr: torch.Tensor,
+                          cols: torch.Tensor, vals: torch.Tensor, symbols: Optional[str]) -> SparseCounts:
+    """A counts file's rows (``Totals`` first) as device CSR over its k-mer columns -> device COO: the file column -> key
+    conversion of read_counts_sidecar and read_counts_csv."""
+    if not rows or rows[0] != "Totals":
         raise ValueError(f"{path}: a counts table starts with its Totals row")
     k = len(kmers[0]) if kmers else 1
     symbols = "".join(sorted(set("".join(kmers)))) if symbols is None else "".join(sorted(set(symbols)))
     codes, ok = E.encode_kmers(kmers, symbols, k)
-    dev = E._require_cuda()
+    dev = rowptr.device
     columns = None
     if _wide(symbols, k):
         columns = E.wide_basis_from_codes(codes[ok], E.alphabet_tables_from_symbols(symbols, dev), k, dev)
@@ -179,18 +230,19 @@ def read_counts_sidecar(path: str, symbols: Optional[str] = None) -> SparseCount
     else:
         key_of_col = codes.astype(np.int64)
         S = len(symbols) ** k
-    rowptr, cols, vals = d["rowptr"], d["cols"].astype(np.int64), d["vals"]
-    rows = np.repeat(np.arange(len(d["rows"])), np.diff(rowptr))
-    good = ok[cols]
-    totals = np.zeros(S, dtype=np.int64)
-    t = (rows == 0) & good
-    totals[key_of_col[cols[t]]] = vals[t]
-    m = (rows > 0) & good
-    keys = (rows[m] - 1).astype(np.int64) * S + key_of_col[cols[m]]
-    order = np.argsort(keys, kind="stable")
-    return SparseCounts(list(d["rows"][1:]), d["seq_count"][1:].astype(np.int64), symbols, k,
-                        torch.from_numpy(keys[order]).to(dev), torch.from_numpy(vals[m][order].astype(np.int64)).to(dev),
-                        torch.from_numpy(totals).to(dev), int(d["seq_count"][0]), columns)
+    kc = torch.from_numpy(np.ascontiguousarray(key_of_col, dtype=np.int64)).to(dev)
+    okd = torch.from_numpy(np.asarray(ok, dtype=bool)).to(dev)
+    cols = cols.to(torch.int64)
+    rows_of = torch.repeat_interleave(torch.arange(len(rows), dtype=torch.int64, device=dev), rowptr[1:] - rowptr[:-1])
+    good = okd[cols] if cols.numel() else torch.zeros(0, dtype=torch.bool, device=dev)
+    totals = torch.zeros(S, dtype=torch.int64, device=dev)
+    t = (rows_of == 0) & good
+    totals[kc[cols[t]]] = vals[t].to(torch.int64)
+    m = (rows_of > 0) & good
+    keys = (rows_of[m] - 1) * S + kc[cols[m]]
+    keys, order = torch.sort(keys, stable=True)
+    return SparseCounts(list(rows[1:]), np.asarray(seq_count[1:], dtype=np.int64), symbols, k, keys,
+                        vals[m][order].to(torch.int64).contiguous(), totals, int(seq_count[0]), columns)
 
 
 def merge_counts_sparse(parts: Sequence[SparseCounts]) -> SparseCounts:
@@ -284,7 +336,14 @@ def _score_sparse(seqs: Sequence[str], sc: SparseCounts, tile: Optional[int], qu
     return E.apply_sparse_tiled(rowptr, cols, cvals, sc.keys, sc.vals, sc.S, A, tile, rows_sink, chunk_rows)
 
 
-MASK_BLOCK_ROWS = 65536     # rows per record batch of a top-2-only association file
+MASK_BLOCK_ROWS = 65536     # rows per block of a top-2-only association side-car
+
+
+def _associations_file(path: str, annotations: Sequence[str], labels: Sequence[str]):
+    """``.skma`` side-car for a path ending in .skma, else the CSV with its text formatted on the device."""
+    if str(path).endswith(".skma"):
+        return sidecar.AssociationsWriter(path, annotations, labels)
+    return E.AssociationsCSVText(path, annotations, labels)
 
 
 def _write_top2_rows(w, r: E.ApplyResult, A: int) -> None:
@@ -321,8 +380,8 @@ def apply_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], sc: Spa
     seqs = [str(reduced_seqs[int(i)]) for i in pick]
     A = len(sc.annotations)
     if out_scores and save_associations:
-        with sidecar.associations_writer(out_scores, sc.annotations, uniq) as w:
-            r = _score_sparse(seqs, sc, tile, query_kmers, w.write, chunk_rows)
+        with _associations_file(out_scores, sc.annotations, uniq) as w:
+            r = _score_sparse(seqs, sc, tile, query_kmers, w if isinstance(w, E.AssociationsCSVText) else w.write, chunk_rows)
     else:
         r = _score_sparse(seqs, sc, tile, query_kmers)
     top1, top2 = r.top1.cpu().numpy(), r.top2.cpu().numpy()
@@ -378,16 +437,21 @@ def eval_counts_sparse(ids: Sequence[str], reduced_seqs: Sequence[str], sc: Spar
     if out_scores:
         labels = [f"{seq_annot[a]}_known_{row_base + n}" if a in seq_annot else f"{a}_unknown_{row_base + n}"
                   for n, a in enumerate(accs)]
-        w = sidecar.associations_writer(out_scores, sc.annotations, labels)
+        w = _associations_file(out_scores, sc.annotations, labels)
     try:
         if uniq:
-            sink = w.write if (w is not None and save_associations) else None
+            sink = None
+            if w is not None and save_associations:
+                sink = w if isinstance(w, E.AssociationsCSVText) else w.write
             r = _score_sparse([str(reduced_seqs[int(i)]) for i in pick], sc, tile, query_kmers, sink, chunk_rows)
         else:
             e32, e64 = torch.zeros(0, dtype=torch.int32, device=dev), torch.zeros(0, dtype=torch.float64, device=dev)
             r = E.ApplyResult(e32, e32.clone(), e64, e64.clone())
         if w is not None and not save_associations:
-            _write_top2_rows(w, r, len(sc.annotations))
+            if isinstance(w, E.AssociationsCSVText):
+                E.write_top2_csv(w, r, chunk_rows)
+            else:
+                _write_top2_rows(w, r, len(sc.annotations))
     finally:
         if w is not None:
             w.close()
