@@ -17,6 +17,7 @@
 // basis): window keys -> segmented radix sort of each sequence's keys -> run-length encode into CSR.  Both are the
 // cross-checks of skm_count_csr_sorted (skm_csrsort.cu).
 #include <cstring>
+#include <type_traits>
 
 #include <cub/cub.cuh>
 
@@ -149,7 +150,9 @@ constexpr int CW_SYM = ts_sym_bytes(CW_SEG);      // 480
 
 // MAP: 0 = identity basis (column = code), 1 = col_of_code staged in shared memory as uint16 columns (S <= 16384;
 // filtered codes point at a dummy counter behind the row, so the scan needs no validity test), 2 = col_of_code read
-// from global memory (large code spaces).
+// from global memory (large code spaces), 3 = MAP 1's columns in lane-striped words (small S, count_dense_warp_kernel
+// only): word w of lane l sits at byte (w * 32 + l) * 4 and holds entries 2w and 2w + 1, so every lane reads its own
+// bank and a warp's map read is one shared-memory wavefront instead of ~4.3 at random codes.
 // The scan is written out here rather than through ts_scan_chunk: one sequence per warp needs no boundary handling,
 // symbols are used raw (an invalid symbol's garbage digit is added and later subtracted with the same value, and no
 // window containing it is ever emitted), and the column comes from shared memory: 13 SASS instructions per residue
@@ -163,8 +166,9 @@ __device__ __forceinline__ void cw_emit(uint32_t code, uint32_t cnt_addr, uint32
     cnt_ops<OutT>::add(cnt_addr, col);
 }
 
-// Branch-free emission: an invalid window is counted into the dummy counter behind the row (MAP 0: column K; MAP 1:
-// the extra map entry S points at it), so the compiler can issue LDS.U16 + ATOMS without a branch around them.
+// Branch-free emission: an invalid window is counted into the dummy counter behind the row (MAP 0: column K; MAP 1
+// and 3: the extra map entry S points at it), so the compiler can issue LDS + ATOMS without a branch around them.
+// MAP 3: col_addr is the map's shared address plus 4 * lane.
 template <typename OutT, int MAP>
 __device__ __forceinline__ void cw_emit_sel(uint32_t code, bool ok, uint32_t cnt_addr, uint32_t col_addr,
                                             const int32_t *__restrict__ col_of_code, int S, int K) {
@@ -173,43 +177,97 @@ __device__ __forceinline__ void cw_emit_sel(uint32_t code, bool ok, uint32_t cnt
         return;
     }
     uint32_t col;
-    if (MAP == 0) col = ok ? code : uint32_t(K);
-    else asm volatile("ld.shared.u16 %0, [%1];" : "=r"(col) : "r"(col_addr + 2u * (ok ? code : uint32_t(S))));
+    if (MAP == 0) {
+        col = ok ? code : uint32_t(K);
+    } else if (MAP == 1) {
+        asm volatile("ld.shared.u16 %0, [%1];" : "=r"(col) : "r"(col_addr + 2u * (ok ? code : uint32_t(S))));
+    } else {
+        const uint32_t c = ok ? code : uint32_t(S);      // entry c: byte (c >> 1) * 128 + (c & 1) * 2 = c * 2 + (c >> 1) * 124
+        asm volatile("ld.shared.u16 %0, [%1];" : "=r"(col) : "r"(col_addr + 2u * c + 124u * (c >> 1)));
+    }
     cnt_ops<OutT>::add(cnt_addr, col);
 }
 
-// Column map (MAP 1) and this warp's zeroed counter row, before the kernel's one CTA-wide barrier.
-template <int MAP>
-__device__ __forceinline__ void cw_prologue(uint16_t *s_col, const int32_t *__restrict__ col_of_code, int S, int K,
-                                            uint4 *s_cnt4, uint32_t row_bytes, int lane) {
-    if (MAP == 1) {
-        for (int i = threadIdx.x; i < S; i += blockDim.x) {
-            const int32_t c = __ldg(col_of_code + i);
-            s_col[i] = uint16_t(c >= 0 ? c : K);                                // K = the dummy counter
-        }
-        if (threadIdx.x == 0) s_col[S] = uint16_t(K);                           // entry S: where invalid windows go
-    }
-    for (int i = lane; i < int(row_bytes >> 4); i += 32) s_cnt4[i] = make_uint4(0u, 0u, 0u, 0u);
+// Zero `bytes` (a multiple of 8) of shared memory from shared address `addr` with one st.bulk (SASS UMEMSETS) instead
+// of 16-byte stores from every lane.  st.bulk has no completion mechanism of its own: it is a weak store of the generic
+// proxy, ordered against the other lanes' later shared-memory atomics by the __syncwarp / __syncthreads that follows.
+__device__ __forceinline__ void cw_zero_row(uint32_t addr, uint32_t bytes) {
+    asm volatile("st.bulk.weak.shared::cta [%0], %1, 0;" ::"r"(addr), "l"(uint64_t(bytes)) : "memory");
 }
 
-// Flush the finished row to dst (one contiguous K * sizeof(OutT) range of the output) and re-zero it.
+// Column of basis entry i for the shared map: K (the dummy counter) for codes outside the basis and for entry S,
+// where invalid windows go.
+__device__ __forceinline__ uint32_t cw_map_entry(const int32_t *__restrict__ col_of_code, int i, int S, int K) {
+    const int32_t c = i < S ? __ldg(col_of_code + i) : -1;
+    return uint32_t(c >= 0 ? c : K);
+}
+
+// Column map (MAP 1 or 3) and this warp's zeroed counter row, before the kernel's one CTA-wide barrier.
+template <int MAP>
+__device__ __forceinline__ void cw_prologue(uint8_t *s_map, const int32_t *__restrict__ col_of_code, int S, int K,
+                                            uint32_t cnt_addr, uint32_t row_bytes, int lane) {
+    if (MAP == 1) {
+        uint16_t *s_col = reinterpret_cast<uint16_t *>(s_map);
+        for (int i = threadIdx.x; i <= S; i += blockDim.x) s_col[i] = uint16_t(cw_map_entry(col_of_code, i, S, K));
+    } else if (MAP == 3) {
+        uint32_t *s_words = reinterpret_cast<uint32_t *>(s_map);
+        const int nwords = (S + 2) >> 1;                                        // entries 0 .. S
+        for (int i = threadIdx.x; i < nwords * 32; i += blockDim.x) {
+            const int e = (i >> 5) * 2;
+            s_words[i] = cw_map_entry(col_of_code, e, S, K) | (cw_map_entry(col_of_code, e + 1, S, K) << 16);
+        }
+    }
+    if (lane == 0) cw_zero_row(cnt_addr, row_bytes);
+}
+
+// Flush the finished row to dst (one contiguous K * sizeof(OutT) range of the output) and re-zero it.  Lane 0 zeroes
+// the row after the bulk copy has read it (cp.async.bulk.wait_group.read in the same thread).
 template <typename OutT>
-__device__ __forceinline__ void cw_flush_row(OutT *dst, uint8_t *mine, uint32_t cnt_addr, int K, uint32_t row_bytes,
+__device__ __forceinline__ void cw_flush_row(OutT *dst, const uint8_t *mine, uint32_t cnt_addr, int K, uint32_t row_bytes,
                                              int bulk_ok, int lane) {
     if (bulk_ok) {
         ts_bulk_fence();
         __syncwarp();
         if (lane == 0) { ts_bulk_store(dst, cnt_addr, uint32_t(K) * uint32_t(sizeof(OutT))); ts_bulk_wait_read(); }
-        __syncwarp();
     } else {
         __syncwarp();
         const OutT *s_cnt = reinterpret_cast<const OutT *>(mine);
         for (int i = lane; i < K; i += 32) dst[i] = s_cnt[i];
         __syncwarp();
     }
-    uint4 *s_cnt4 = reinterpret_cast<uint4 *>(mine);
-    for (int i = lane; i < int(row_bytes >> 4); i += 32) s_cnt4[i] = make_uint4(0u, 0u, 0u, 0u);
+    if (lane == 0) cw_zero_row(cnt_addr, row_bytes);
     __syncwarp();
+}
+
+// PRMT in its sign mode: byte i of the result is 0xFF where bit 7 of byte i of x is set, else 0.
+__device__ __forceinline__ uint32_t cw_sign_bytes(uint32_t x) {
+    uint32_t r;
+    asm("prmt.b32 %0, %1, 0, 0xBA98;" : "=r"(r) : "r"(x));
+    return r;
+}
+
+// PRMT with a selector whose nibbles are known to be < 8 (__byte_perm masks them with 0x7777 first)
+__device__ __forceinline__ uint32_t cw_prmt(uint32_t a, uint32_t b, uint32_t sel) {
+    uint32_t r;
+    asm("prmt.b32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(sel));
+    return r;
+}
+
+// Four residue bytes -> four symbols (digit or SYM_BAD), for a LUT that maps every byte outside 0x40-0x5F to SYM_BAD
+// (upper-case letters and @[\]^_; every built-in alphabet but ptm).  L holds the LUT entries 0x40-0x5F, four per
+// register.  One PRMT per register pair picks by the low 3 bits of each byte, two byte-mask muxes by bits 3 and 4,
+// and bytes whose top three bits are not 010 become SYM_BAD: ~20 ALU instructions against four LDS.U8.
+__device__ __forceinline__ uint32_t cw_translate_reg(uint32_t raw, const uint32_t (&L)[8]) {
+    const uint32_t s = raw & 0x07070707u;
+    const uint32_t sel = __byte_perm(s | (s >> 4), 0u, 0x0020u);                // nibble i = low 3 bits of byte i
+    const uint32_t q0 = cw_prmt(L[0], L[1], sel), q1 = cw_prmt(L[2], L[3], sel);
+    const uint32_t q2 = cw_prmt(L[4], L[5], sel), q3 = cw_prmt(L[6], L[7], sel);
+    const uint32_t m3 = cw_sign_bytes(raw << 4), m4 = cw_sign_bytes(raw << 3);   // bytes with bit 3 / bit 4 set
+    const uint32_t lo = (q0 & ~m3) | (q1 & m3), hi = (q2 & ~m3) | (q3 & m3);
+    const uint32_t t = (lo & ~m4) | (hi & m4);
+    const uint32_t y = raw ^ 0x40404040u;
+    const uint32_t bad = cw_sign_bytes(y | (y << 1) | (y << 2));                // any of bits 5-7 of byte ^ 0x40 set
+    return (t & ~bad) | (SYM_BAD * 0x01010101u & bad);
 }
 
 // First version of the warp kernel (round 1): translated symbols staged as bytes, two LDS.U8 per residue, a run
@@ -223,13 +281,12 @@ count_dense_warp_bytes_kernel(const uint8_t *__restrict__ res, int64_t nres, con
     extern __shared__ __align__(128) uint8_t s_raw[];
     __shared__ uint8_t s_lut[256];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    uint16_t *s_col = reinterpret_cast<uint16_t *>(s_raw);                       // [S + 1] when MAP == 1
     uint8_t *mine = s_raw + map_bytes + size_t(warp) * (row_bytes + CW_SYM);
     uint8_t *s_sym = mine + row_bytes;
-    uint32_t cnt_addr = smem_addr(mine), sym_addr = smem_addr(s_sym), col_addr = smem_addr(s_col);
+    uint32_t cnt_addr = smem_addr(mine), sym_addr = smem_addr(s_sym), col_addr = smem_addr(s_raw);   // map: [S + 1] uint16 when MAP == 1
     asm volatile("" : "+r"(cnt_addr), "+r"(sym_addr), "+r"(col_addr));      // keep the window addresses in registers
     ts_lut_init(s_lut, lut);
-    cw_prologue<MAP>(s_col, col_of_code, S, K, reinterpret_cast<uint4 *>(mine), row_bytes, lane);
+    cw_prologue<MAP>(s_raw, col_of_code, S, K, cnt_addr, row_bytes, lane);
     __syncthreads();                                        // LUT and column map; the only CTA-wide barrier
     // this warp's sequences: those that start in the w-th 1/W of the residue buffer
     int64_t lo = 0, hi = 0;
@@ -260,31 +317,37 @@ count_dense_warp_bytes_kernel(const uint8_t *__restrict__ res, int64_t nres, con
 //     word, last word, an X somewhere in 192 bytes — and made the first word-based version execute MORE instructions);
 //   * positions are 32-bit offsets from the warp's own (16-byte aligned) base, and the offsets of 31 sequences are
 //     fetched with one coalesced load and handed out by shuffles;
-// Measured and dropped (profiles/R2e_*): re-zeroing the flushed row with the copy engine instead of 8 STS.128 per lane
-// (zeroing is 32 of the 189 LSU wavefronts per sequence and the LSU wavefront pipe is what bounds the kernel: 85 % busy,
-// the SRAM banks 14 %).  cp.async.bulk shared -> shared from a zero row of the CTA on a per-warp mbarrier needs a
-// cluster launch (illegal instruction otherwise) and ran at 1.21 ms against 0.85 ms; global (L2) -> shared 0.92 ms.
+// Round 3 (profiles/count_dense_*, DESIGN 3.2) took the LSU wavefronts that are not the counter atomics off the
+// shared-memory pipe: the flushed row is re-zeroed with one st.bulk from lane 0 (cw_zero_row) instead of 8 STS.128 per
+// lane; for a LUT whose entries outside 0x40-0x5F are all SYM_BAD the residues are translated in registers
+// (cw_translate_reg) instead of four LDS.U8 per word; for small S the column map is lane-striped (MAP 3), which needs
+// one CTA of up to 32 warps per SM for its 4 * 32 bytes per map word.
+// Measured and dropped (profiles/R2e_*): re-zeroing the flushed row with the copy engine (cp.async.bulk shared -> shared
+// from a zero row needs a cluster launch and ran at 1.21 ms against 0.85 ms; global (L2) -> shared 0.92 ms).
 template <typename OutT, int MAP>
-__global__ void __launch_bounds__(32 * CW_WARPS, 6)
+__global__ void __launch_bounds__(MAP == 3 ? 1024 : 32 * CW_WARPS, MAP == 3 ? 1 : 6)
 count_dense_warp_kernel(const uint8_t *__restrict__ res, int64_t nres, const int64_t *__restrict__ off, int64_t nseq,
                         const uint8_t *__restrict__ lut, uint32_t nsym, int k, uint32_t pow_k1,
                         const int32_t *__restrict__ col_of_code, int S, int K, uint32_t row_bytes, uint32_t map_bytes, int bulk_ok,
                         OutT *__restrict__ out) {
     extern __shared__ __align__(128) uint8_t s_raw[];
     __shared__ __align__(16) uint8_t s_lut[256];
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    uint16_t *s_col = reinterpret_cast<uint16_t *>(s_raw);                       // [S + 1] when MAP == 1
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
     uint8_t *mine = s_raw + map_bytes + size_t(warp) * (row_bytes + CW_SYM);
     uint8_t *s_res = mine + row_bytes;                                           // raw residue bytes of the segment
-    uint32_t cnt_addr = smem_addr(mine), raw_addr = smem_addr(s_res), col_addr = smem_addr(s_col), lut_addr = smem_addr(s_lut);
+    uint32_t cnt_addr = smem_addr(mine), raw_addr = smem_addr(s_res), lut_addr = smem_addr(s_lut);
+    uint32_t col_addr = smem_addr(s_raw) + (MAP == 3 ? 4u * uint32_t(lane) : 0u);
     asm volatile("" : "+r"(cnt_addr), "+r"(raw_addr), "+r"(col_addr), "+r"(lut_addr));
     ts_lut_init(s_lut, lut);                                                     // invalid bytes -> SYM_BAD (0x40)
     if (threadIdx.x == 0) s_lut[0] = uint8_t(SYM_BAD);                           // byte 0 pads the staged segment: never a symbol
-    cw_prologue<MAP>(s_col, col_of_code, S, K, reinterpret_cast<uint4 *>(mine), row_bytes, lane);
-    __syncthreads();                                        // LUT and column map; the only CTA-wide barrier
+    bool lut_in_regs = true;                                                     // every entry outside 0x40-0x5F is SYM_BAD
+    for (int i = threadIdx.x; i < 256; i += blockDim.x)
+        if ((i & 0xE0) != 0x40 && i != 0 && lut[i] != SYM_INVALID) lut_in_regs = false;
+    cw_prologue<MAP>(s_raw, col_of_code, S, K, cnt_addr, row_bytes, lane);
+    const bool reg_lut = __syncthreads_and(lut_in_regs);    // LUT and column map; the only CTA-wide barrier
     // this warp's sequences: those that start in the w-th 1/W of the residue buffer
     int64_t lo = 0, hi = 0;
-    if (lane == 0) seq_range(off, nseq, int64_t(blockIdx.x) * CW_WARPS + warp, int64_t(gridDim.x) * CW_WARPS, &lo, &hi);
+    if (lane == 0) seq_range(off, nseq, int64_t(blockIdx.x) * nwarps + warp, int64_t(gridDim.x) * nwarps, &lo, &hi);
     lo = __shfl_sync(FULL, lo, 0);
     hi = __shfl_sync(FULL, hi, 0);
     if (lo >= hi) return;
@@ -297,93 +360,110 @@ count_dense_warp_kernel(const uint8_t *__restrict__ res, int64_t nres, const int
     const uint32_t out_shift = 32u - 8u * km1;              // (previous : current) >> out_shift = the four outgoing symbols
     const uint32_t win0 = ((1u << uk) - 1u) << (4u - km1);  // validity bits a window ending at byte 0 of `current` covers
     const uint32_t npow = 0u - pow_k1;
-    uint32_t tailw = 0;
-    for (int64_t s0 = lo; s0 < hi; s0 += 31) {
-        // one coalesced load of 32 offsets: sequences s0 .. s0+30 (b = rel[i], e = rel[i+1])
-        const int64_t si = min(s0 + lane, hi);
-        const uint32_t rel = uint32_t(__ldg(off + si) - r_base);
-        const int ns = (hi - s0 < 31) ? int(hi - s0) : 31;
-        for (int i = 0; i < ns; ++i) {
-            const uint32_t b = __shfl_sync(FULL, rel, i), e = __shfl_sync(FULL, rel, i + 1);
-            bool first = true;
-            for (uint32_t a = b; a < e;) {
-                const uint32_t a2 = min(e, (a + uint32_t(CW_SEG)) & ~15u);
-                const uint32_t base = a & ~15u;
-                const int lo_i = TS_PAD + int(a - base), hi_i = lo_i + int(a2 - a);
-                const int nvec = int((a2 - base + 15u) >> 4);
-                // stage the raw bytes [base, a2) at s_res[TS_PAD ...): one 16-byte vector per lane (at most 25)
-                if (lane < nvec) {
-                    const uint32_t p = base + 16u * uint32_t(lane);
-                    uint4 x;
-                    if (p + 16u <= lim) {
-                        x = __ldg(reinterpret_cast<const uint4 *>(resw + p));
-                    } else {
-                        uint32_t w4[4] = {0, 0, 0, 0};
-                        for (int j = 0; j < 16; ++j)
-                            if (p + uint32_t(j) < lim) w4[j >> 2] |= uint32_t(resw[p + j]) << (8 * (j & 3));
-                        x = make_uint4(w4[0], w4[1], w4[2], w4[3]);
-                    }
-                    reinterpret_cast<uint4 *>(s_res + TS_PAD)[lane] = x;
-                }
-                if (!first && lane == 0) reinterpret_cast<uint32_t *>(s_res)[TS_PAD / 4 - 1] = tailw;   // the 4 bytes in front of this segment
-                __syncwarp();
-                // byte 0 translates to SYM_BAD: everything in front of the sequence and behind the segment's last word is invalid
-                if (first) { const int f0 = (lo_i & ~3) - 4; if (f0 + lane < lo_i) s_res[f0 + lane] = 0; }   // previous word + front of the first word
-                if (lane < ((4 - (hi_i & 3)) & 3)) s_res[hi_i + lane] = 0;
-                __syncwarp();
-                // lane owns cw words (cw odd -> conflict-free LDS.32) from word index w0
-                const int A = lo_i & ~3;
-                const int n = hi_i - A;
-                const int cw = (((n + 31) >> 5) + 3) >> 2 | 1;
-                const int w0 = (A >> 2) + lane * cw, w1 = min(w0 + cw, (hi_i + 3) >> 2);
-                if (w0 < w1) {
-                    uint32_t pa = raw_addr + 4u * uint32_t(w0);
-                    uint32_t raw;
-                    asm volatile("ld.shared.u32 %0, [%1+-4];" : "=r"(raw) : "r"(pa));
-                    uint32_t t0, t1, t2, t3;
-                    asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t0) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4440u)));
-                    asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t1) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4441u)));
-                    asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t2) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4442u)));
-                    asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t3) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4443u)));
-                    uint32_t prevT = t0 | (t1 << 8) | (t2 << 16) | (t3 << 24);
-                    uint32_t pinv = (((prevT >> 6) & 0x01010101u) * 0x01020408u) >> 24;      // bit i: byte i of prevT is no symbol
-                    uint32_t code = 0;
-                    for (uint32_t t = 0; t < km1; ++t) code = code * nsym + ((prevT >> (out_shift + 8u * t)) & 0xFFu);
-                    for (int w = w0; w < w1; ++w, pa += 4u) {
-                        asm volatile("ld.shared.u32 %0, [%1];" : "=r"(raw) : "r"(pa));
-                        asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t0) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4440u)));
-                        asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t1) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4441u)));
-                        asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t2) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4442u)));
-                        asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t3) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4443u)));
-                        const uint32_t curT = t0 | (t1 << 8) | (t2 << 16) | (t3 << 24);
-                        const uint32_t outw = __funnelshift_rc(prevT, curT, out_shift);
-                        const uint32_t cinv = (((curT >> 6) & 0x01010101u) * 0x01020408u) >> 24;
-                        const uint32_t inv8 = pinv | (cinv << 4);
-                        code = code * nsym + t0;
-                        cw_emit_sel<OutT, MAP>(code, (inv8 & win0) == 0u, cnt_addr, col_addr, col_of_code, S, K);
-                        code = __byte_perm(outw, 0u, 0x4440u) * npow + code;
-                        code = code * nsym + t1;
-                        cw_emit_sel<OutT, MAP>(code, (inv8 & (win0 << 1)) == 0u, cnt_addr, col_addr, col_of_code, S, K);
-                        code = __byte_perm(outw, 0u, 0x4441u) * npow + code;
-                        code = code * nsym + t2;
-                        cw_emit_sel<OutT, MAP>(code, (inv8 & (win0 << 2)) == 0u, cnt_addr, col_addr, col_of_code, S, K);
-                        code = __byte_perm(outw, 0u, 0x4442u) * npow + code;
-                        code = code * nsym + t3;
-                        cw_emit_sel<OutT, MAP>(code, (inv8 & (win0 << 3)) == 0u, cnt_addr, col_addr, col_of_code, S, K);
-                        code = __byte_perm(outw, 0u, 0x4443u) * npow + code;
-                        prevT = curT;
-                        pinv = cinv;
-                    }
-                }
-                __syncwarp();
-                if (a2 < e && lane == 0) tailw = reinterpret_cast<const uint32_t *>(s_res)[(hi_i >> 2) - 1];   // hi_i is 16-aligned here
-                __syncwarp();
-                first = false;
-                a = a2;
-            }
-            cw_flush_row(out + (s0 + i) * K, mine, cnt_addr, K, row_bytes, bulk_ok, lane);
-        }
+    uint32_t L[8];                                          // LUT entries 0x40-0x5F (used when reg_lut)
+    {
+        const uint4 a = reinterpret_cast<const uint4 *>(s_lut + 0x40)[0], b = reinterpret_cast<const uint4 *>(s_lut + 0x40)[1];
+        L[0] = a.x; L[1] = a.y; L[2] = a.z; L[3] = a.w; L[4] = b.x; L[5] = b.y; L[6] = b.z; L[7] = b.w;
     }
+    // the whole walk, once per translation (a uniform branch: every warp of the CTA takes the same one)
+    auto walk = [&](auto use_regs) {
+        constexpr bool REG = decltype(use_regs)::value;
+        // the four symbols of a word, packed and one by one
+        auto translate = [&](uint32_t raw, uint32_t (&t)[4]) -> uint32_t {
+            if (REG) {
+                const uint32_t T = cw_translate_reg(raw, L);
+                t[0] = T & 0xFFu; t[1] = __byte_perm(T, 0u, 0x4441u); t[2] = __byte_perm(T, 0u, 0x4442u); t[3] = T >> 24;
+                return T;
+            }
+            asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t[0]) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4440u)));
+            asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t[1]) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4441u)));
+            asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t[2]) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4442u)));
+            asm volatile("ld.shared.u8 %0, [%1];" : "=r"(t[3]) : "r"(lut_addr + __byte_perm(raw, 0u, 0x4443u)));
+            return t[0] | (t[1] << 8) | (t[2] << 16) | (t[3] << 24);
+        };
+        uint32_t tailw = 0;
+        for (int64_t s0 = lo; s0 < hi; s0 += 31) {
+            // one coalesced load of 32 offsets: sequences s0 .. s0+30 (b = rel[i], e = rel[i+1])
+            const int64_t si = min(s0 + lane, hi);
+            const uint32_t rel = uint32_t(__ldg(off + si) - r_base);
+            const int ns = (hi - s0 < 31) ? int(hi - s0) : 31;
+            for (int i = 0; i < ns; ++i) {
+                const uint32_t b = __shfl_sync(FULL, rel, i), e = __shfl_sync(FULL, rel, i + 1);
+                bool first = true;
+                for (uint32_t a = b; a < e;) {
+                    const uint32_t a2 = min(e, (a + uint32_t(CW_SEG)) & ~15u);
+                    const uint32_t base = a & ~15u;
+                    const int lo_i = TS_PAD + int(a - base), hi_i = lo_i + int(a2 - a);
+                    const int nvec = int((a2 - base + 15u) >> 4);
+                    // stage the raw bytes [base, a2) at s_res[TS_PAD ...): one 16-byte vector per lane (at most 25)
+                    if (lane < nvec) {
+                        const uint32_t p = base + 16u * uint32_t(lane);
+                        uint4 x;
+                        if (p + 16u <= lim) {
+                            x = __ldg(reinterpret_cast<const uint4 *>(resw + p));
+                        } else {
+                            uint32_t w4[4] = {0, 0, 0, 0};
+                            for (int j = 0; j < 16; ++j)
+                                if (p + uint32_t(j) < lim) w4[j >> 2] |= uint32_t(resw[p + j]) << (8 * (j & 3));
+                            x = make_uint4(w4[0], w4[1], w4[2], w4[3]);
+                        }
+                        reinterpret_cast<uint4 *>(s_res + TS_PAD)[lane] = x;
+                    }
+                    if (!first && lane == 0) reinterpret_cast<uint32_t *>(s_res)[TS_PAD / 4 - 1] = tailw;   // the 4 bytes in front of this segment
+                    __syncwarp();
+                    // byte 0 translates to SYM_BAD: everything in front of the sequence and behind the segment's last word is invalid
+                    if (first) { const int f0 = (lo_i & ~3) - 4; if (f0 + lane < lo_i) s_res[f0 + lane] = 0; }   // previous word + front of the first word
+                    if (lane < ((4 - (hi_i & 3)) & 3)) s_res[hi_i + lane] = 0;
+                    __syncwarp();
+                    // lane owns cw words (cw odd -> conflict-free LDS.32) from word index w0
+                    const int A = lo_i & ~3;
+                    const int n = hi_i - A;
+                    const int cw = (((n + 31) >> 5) + 3) >> 2 | 1;
+                    const int w0 = (A >> 2) + lane * cw, w1 = min(w0 + cw, (hi_i + 3) >> 2);
+                    if (w0 < w1) {
+                        uint32_t pa = raw_addr + 4u * uint32_t(w0);
+                        uint32_t raw;
+                        asm volatile("ld.shared.u32 %0, [%1+-4];" : "=r"(raw) : "r"(pa));
+                        uint32_t t[4];
+                        uint32_t prevT = translate(raw, t);
+                        uint32_t pinv = (((prevT >> 6) & 0x01010101u) * 0x01020408u) >> 24;      // bit i: byte i of prevT is no symbol
+                        uint32_t code = 0;
+                        for (uint32_t t = 0; t < km1; ++t) code = code * nsym + ((prevT >> (out_shift + 8u * t)) & 0xFFu);
+                        for (int w = w0; w < w1; ++w, pa += 4u) {
+                            asm volatile("ld.shared.u32 %0, [%1];" : "=r"(raw) : "r"(pa));
+                            const uint32_t curT = translate(raw, t);
+                            const uint32_t outw = __funnelshift_rc(prevT, curT, out_shift);
+                            const uint32_t cinv = (((curT >> 6) & 0x01010101u) * 0x01020408u) >> 24;
+                            const uint32_t inv8 = pinv | (cinv << 4);
+                            code = code * nsym + t[0];
+                            cw_emit_sel<OutT, MAP>(code, (inv8 & win0) == 0u, cnt_addr, col_addr, col_of_code, S, K);
+                            code = __byte_perm(outw, 0u, 0x4440u) * npow + code;
+                            code = code * nsym + t[1];
+                            cw_emit_sel<OutT, MAP>(code, (inv8 & (win0 << 1)) == 0u, cnt_addr, col_addr, col_of_code, S, K);
+                            code = __byte_perm(outw, 0u, 0x4441u) * npow + code;
+                            code = code * nsym + t[2];
+                            cw_emit_sel<OutT, MAP>(code, (inv8 & (win0 << 2)) == 0u, cnt_addr, col_addr, col_of_code, S, K);
+                            code = __byte_perm(outw, 0u, 0x4442u) * npow + code;
+                            code = code * nsym + t[3];
+                            cw_emit_sel<OutT, MAP>(code, (inv8 & (win0 << 3)) == 0u, cnt_addr, col_addr, col_of_code, S, K);
+                            code = __byte_perm(outw, 0u, 0x4443u) * npow + code;
+                            prevT = curT;
+                            pinv = cinv;
+                        }
+                    }
+                    __syncwarp();
+                    if (a2 < e && lane == 0) tailw = reinterpret_cast<const uint32_t *>(s_res)[(hi_i >> 2) - 1];   // hi_i is 16-aligned here
+                    __syncwarp();
+                    first = false;
+                    a = a2;
+                }
+                cw_flush_row(out + (s0 + i) * K, mine, cnt_addr, K, row_bytes, bulk_ok, lane);
+            }
+        }
+    };
+    // the register translation needs the 1024-thread CTA's 64 registers: at 40 the walk spills
+    if (MAP == 3 && reg_lut) walk(std::true_type{});
+    else walk(std::false_type{});
 }
 
 // Everything a dense count launch passes to its kernel besides the launch shape.
@@ -414,17 +494,17 @@ static int launch_dense_tile(const DenseArgs &a, int grid, size_t smem, int T, i
     return SKM_OK;
 }
 
-// words: the round-2 kernel (k - 1 <= 4), else the byte-wise one; map_mode selects MAP
+// words: the round-2 kernel (k - 1 <= 4), else the byte-wise one; map_mode selects MAP (3: words only)
 template <typename OutT>
-static int launch_dense_warp(const DenseArgs &a, bool words, int map_mode, int grid, size_t smem, uint32_t row_bytes,
+static int launch_dense_warp(const DenseArgs &a, bool words, int map_mode, int grid, int warps, size_t smem, uint32_t row_bytes,
                              uint32_t map_bytes, int bulk_ok) {
     using Kern = decltype(&count_dense_warp_kernel<OutT, 0>);
-    const Kern kerns[2][3] = {{count_dense_warp_bytes_kernel<OutT, 0>, count_dense_warp_bytes_kernel<OutT, 1>, count_dense_warp_bytes_kernel<OutT, 2>},
-                              {count_dense_warp_kernel<OutT, 0>, count_dense_warp_kernel<OutT, 1>, count_dense_warp_kernel<OutT, 2>}};
+    const Kern kerns[2][4] = {{count_dense_warp_bytes_kernel<OutT, 0>, count_dense_warp_bytes_kernel<OutT, 1>, count_dense_warp_bytes_kernel<OutT, 2>, nullptr},
+                              {count_dense_warp_kernel<OutT, 0>, count_dense_warp_kernel<OutT, 1>, count_dense_warp_kernel<OutT, 2>, count_dense_warp_kernel<OutT, 3>}};
     const Kern kern = kerns[words][map_mode];
     SKM_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, 32 * CW_WARPS, smem, a.st>>>(a.res, a.nres, a.off, a.nseq, a.lut, a.nsym, a.k, a.pow_k1, a.col_of_code, a.S,
-                                              a.K, row_bytes, map_bytes, bulk_ok, static_cast<OutT *>(a.out));
+    kern<<<grid, 32 * warps, smem, a.st>>>(a.res, a.nres, a.off, a.nseq, a.lut, a.nsym, a.k, a.pow_k1, a.col_of_code, a.S,
+                                           a.K, row_bytes, map_bytes, bulk_ok, static_cast<OutT *>(a.out));
     SKM_LAUNCH_CHECK(words ? "count_dense_warp_kernel" : "count_dense_warp_bytes_kernel");
     return SKM_OK;
 }
@@ -521,17 +601,31 @@ int skm_count_dense(const uint8_t *d_residues, int64_t nres, const int64_t *d_of
     // counter behind the row absorbs the windows whose code is filtered out of the basis.
     const uint32_t row_bytes = uint32_t((size_t(K + 1) * out_bytes + 15) & ~size_t(15));
     if (row_bytes + CW_SYM <= 9 * 1024 + 256 && K < 65535) {
-        const int map_mode = !d_col_of_code ? 0 : (S <= 16384 ? 1 : 2);
-        const uint32_t map_bytes = map_mode == 1 ? uint32_t((size_t(S + 1) * 2 + 127) & ~size_t(127)) : 0u;     // + the entry for invalid windows
+        int map_mode = !d_col_of_code ? 0 : (S <= 16384 ? 1 : 2);
         const bool words = k - 1 <= 4;
-        const size_t smem_w = map_bytes + size_t(CW_WARPS) * (row_bytes + CW_SYM);
+        const int bulk_ok = ((size_t(K) * out_bytes) % 16 == 0) ? 1 : 0;
+        const size_t per_warp = row_bytes + CW_SYM;
+        // MAP 3 (lane-striped map): one CTA per SM with as many warps as fit next to the map, if that is at least 24
+        // (the uint16 map with 5-6 CTAs of 8 warps keeps ~40 warps per SM to hide latency; the striped shape was
+        // measured at 32).  C2 (S = K = 1000, int32): 64 KB of map + 32 warps, 208 KB.
+        const size_t cta_smem = 227 * 1024 - 256;                                   // minus the static LUT
+        const uint32_t striped_bytes = uint32_t(size_t((S + 2) / 2) * 128);
+        if (map_mode == 1 && words && striped_bytes + 24 * per_warp <= cta_smem) {
+            map_mode = 3;
+            const int warps = (int)std::min<size_t>(32, (cta_smem - striped_bytes) / per_warp);
+            const size_t smem = striped_bytes + size_t(warps) * per_warp;
+            const int grid = (int)std::min<int64_t>((nseq + warps - 1) / warps, int64_t(sm_count()));
+            return out_bits == 32 ? launch_dense_warp<int32_t>(args, true, 3, grid, warps, smem, row_bytes, striped_bytes, bulk_ok)
+                                  : launch_dense_warp<uint16_t>(args, true, 3, grid, warps, smem, row_bytes, striped_bytes, bulk_ok);
+        }
+        const uint32_t map_bytes = map_mode == 1 ? uint32_t((size_t(S + 1) * 2 + 127) & ~size_t(127)) : 0u;     // + the entry for invalid windows
+        const size_t smem_w = map_bytes + size_t(CW_WARPS) * per_warp;
         int per_sm_w = int((227 * 1024) / (smem_w + 1024 + 256));
         if (per_sm_w > 6) per_sm_w = 6;
         if (per_sm_w < 1) per_sm_w = 1;
         const int grid_w = (int)std::min<int64_t>((nseq + CW_WARPS - 1) / CW_WARPS, int64_t(sm_count()) * per_sm_w);
-        const int bulk_ok = ((size_t(K) * out_bytes) % 16 == 0) ? 1 : 0;
-        return out_bits == 32 ? launch_dense_warp<int32_t>(args, words, map_mode, grid_w, smem_w, row_bytes, map_bytes, bulk_ok)
-                              : launch_dense_warp<uint16_t>(args, words, map_mode, grid_w, smem_w, row_bytes, map_bytes, bulk_ok);
+        return out_bits == 32 ? launch_dense_warp<int32_t>(args, words, map_mode, grid_w, CW_WARPS, smem_w, row_bytes, map_bytes, bulk_ok)
+                              : launch_dense_warp<uint16_t>(args, words, map_mode, grid_w, CW_WARPS, smem_w, row_bytes, map_bytes, bulk_ok);
     }
     // Tile shape.  Many small CTAs per SM (each with its own tile in flight) hide the staging-load, barrier
     // and bulk-store latencies of one another: 128 threads, ~16 KB of counters, rows a multiple of
